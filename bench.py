@@ -27,6 +27,7 @@ if ROOT not in sys.path:
 
 W, H = 1920, 1080     # config 2 geometry (the CPU arm always decodes config-2 images)
 FALLBACK_HBM_GBS = 6650.0          # /opt/skills/guides/B200_PROFILING.md fallback
+DUMP_PIXELS = 4 << 20              # --dump-outputs: sampled RGB pixels over all images (48 MiB as float32)
 
 
 def parse_args():
@@ -49,6 +50,10 @@ def parse_args():
                          "configs[3] and configs[4], the oracle-checked parity block)")
     ap.add_argument("--extra-steps", type=int, default=5)
     ap.add_argument("--parity-images", type=int, default=8, help="images per rank checked against the oracle after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what rank 0's last timed step returned as DIR/<name>.npy: status.npy "
+                         "(per image), image_hw.npy (height, width per image) and rgb.npy, float32 [images, S, 3] RGB at S "
+                         "pixels per image drawn with a fixed seed (S = %d // images, under 64 MB in all)" % DUMP_PIXELS)
     return ap.parse_args()
 
 
@@ -79,10 +84,12 @@ WORKLOADS = {
 
 def load_images(n: int, rank: int, world: int, config: str = "c2", scaling: str = "weak", with_ids: bool = False):
     """Seeded images of one BASELINE.json workload (tools/gen_jpegs), cached on local disk so that
-    the ranks of one run (and the reference arm) generate them only once."""
+    the ranks of one run (and the reference arm) generate them only once; per user, since other accounts may share
+    the temporary directory."""
+    import tempfile
     from tools import gen_jpegs
     wl = WORKLOADS[config]
-    cache = f"/tmp/hjd_bench_{config}_{wl['w']}x{wl['h']}_{n}.bin"
+    cache = os.path.join(tempfile.gettempdir(), f"hjd_bench_{os.getuid()}_{config}_{wl['w']}x{wl['h']}_{n}.bin")
     idx = cache + ".idx"
     if not os.path.exists(idx):
         if rank == 0:
@@ -354,6 +361,26 @@ def file_to_bmp_record(hjd, files, local_rank, rank, n_images=512, with_referenc
         shutil.rmtree(root, ignore_errors=True)
 
 
+def dump_outputs(dec, out_dir):
+    """What the last decode left for its caller, as float32 .npy files: every image's status and size, and its RGB at
+    a fixed, seeded sample of pixel positions (the same positions for the same batch, whichever build decodes it)."""
+    import numpy as np
+    n = dec.num_images
+    hw = np.array([(dec.info(i).height, dec.info(i).width) for i in range(n)], dtype=np.int64).reshape(n, 2)
+    s = max(DUMP_PIXELS // max(n, 1), 1)
+    u = np.random.default_rng(0).random((n, s))
+    rgb = np.zeros((n, s, 3), dtype=np.float32)
+    for i in range(n):
+        h, w = (int(v) for v in hw[i])
+        if h * w:
+            pos = (u[i] * (h * w)).astype(np.int64)
+            rgb[i] = dec.rgb(i).reshape(h * w, 3)[pos]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "status.npy"), dec.status().astype(np.float32))
+    np.save(os.path.join(out_dir, "image_hw.npy"), hw.astype(np.float32))
+    np.save(os.path.join(out_dir, "rgb.npy"), rgb)
+
+
 def timed_resident(dec, steps, barrier):
     """K resident decodes bracketed by barriers; CUDA events on the launching stream.  Returns ms for the K steps
     and the stage times of the last one."""
@@ -534,6 +561,8 @@ def run_ours(args, rank, local_rank, world):
         stage[k] = t[k]
     launches = t["launches"]
     idct_variant = dec.idct_variant          # which fused kernel(s) the timed decodes went through (read while the batch is alive)
+    if args.dump_outputs and rank == 0:      # before the end-to-end leg decodes through the same handle again
+        dump_outputs(dec, args.dump_outputs)
 
     t_ms = torch.tensor([ms_total], dtype=torch.float64, device="cuda")
     tot = torch.tensor([float(pixels), float(scan_bytes), float(alg_bytes), float(n), float(launches * args.steps)],

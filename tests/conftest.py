@@ -31,5 +31,6 @@ def port():
 def refbind():
     from oracle import refbind as r
     if not r.available("std"):
-        pytest.skip("oracle/_ref not built (needs /root/reference; run oracle/build_ref.sh)")
+        pytest.skip("oracle/_ref not built: needs a checkout of the original project, which is not part of this "
+                    "repository (REF=<checkout> oracle/build_ref.sh)")
     return r

@@ -3,6 +3,7 @@ test_gpu_parity.py).  Full-size where the oracle finishes in seconds, size-indep
 otherwise."""
 import hashlib
 import os
+import tempfile
 
 import numpy as np
 import pytest
@@ -11,7 +12,7 @@ pytestmark = pytest.mark.gpu
 
 
 def _cached(name, make):
-    path = f"/tmp/hjd_test_{name}.jpg"
+    path = os.path.join(tempfile.gettempdir(), f"hjd_test_{os.getuid()}_{name}.jpg")     # per user: shared temp dirs
     if not os.path.exists(path):
         data = make()
         with open(path + ".tmp", "wb") as fh:

@@ -17,7 +17,8 @@ LENNA = os.path.join(ROOT, "oracle", "_ref", "data", "Lenna.jpg")
 
 def test_reference_main_runs_on_the_gpu_decode_core(tmp_path, port, hjd):
     if not (os.path.exists(BIN) and os.path.exists(LENNA)):
-        pytest.skip("oracle/_ref/ref_main_on_gpu not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/ref_main_on_gpu not built: needs a checkout of the original project, which is not part "
+                    "of this repository (REF=<checkout> oracle/build_ref.sh)")
     # main.cpp hard-codes ../../../../data/Lenna.jpg and ../../../../data/out.bmp (main.cpp:30-31)
     (tmp_path / "data").mkdir()
     shutil.copy(LENNA, tmp_path / "data" / "Lenna.jpg")

@@ -292,18 +292,31 @@ def test_pipelined_file_to_bmp_conversion(hjd, port, tmp_path):
             k += 1
 
 
-def test_against_the_reference_itself(hjd, refbind, tmp_path):
-    """VERDICT r1 (weak 2): the GPU path against the REFERENCE's own code (oracle/_ref, compiled from
-    /root/reference/src by oracle/build_ref.sh), not its restatement: unmodified JpegParseHeader + JpegDecodeHW
+def test_against_the_reference_itself(hjd, tmp_path):
+    """VERDICT r1 (weak 2): the GPU path against the REFERENCE's own code (oracle/_ref, built from a checkout of the
+    reference by oracle/build_ref.sh), not its restatement: unmodified JpegParseHeader + JpegDecodeHW
     (mode 0) for restart-free colour files, the reference's block-level code with MCU-counted restarts and
-    grayscale by extension (mode 1) otherwise -- coefficients, planes, RGB and the BMP file, bit for bit."""
+    grayscale by extension (mode 1) otherwise -- coefficients, planes, RGB and the BMP file, bit for bit.
+    Without oracle/_ref, the committed fixtures among these files are checked against the answers the reference gave
+    for them (tests/golden/golden.json: coefficients, planes and RGB); the generated files and the BMP need it live."""
+    import hashlib
+    import json
+    from oracle import refbind
     from tools.gen_jpegs import encode_jpeg, make_c2, synth_rgb
-    base = cases.small_cases()
-    files = {n: base[n] for n in ("444_64x48_q85", "422_64x48_q85", "420_37x53_q75", "420_100x70_ri2", "444_opt_ri5",
-                                  "440_61x35_ri3", "gray_33x9_ri4", "420_noise_q100", "420_gradient_q50", "444_1x1")}
-    files["420_512x384_q90"] = encode_jpeg(synth_rgb(512, 384, 77), 90, "4:2:0")
-    files["c2_1080p_ri8"] = make_c2(5)
-    files["c2_1080p_twin"] = make_c2(5, restart=False)
+    live = refbind.available("std")
+    gdir = os.path.join(os.path.dirname(__file__), "golden")
+    golden = json.load(open(os.path.join(gdir, "golden.json")))["cases"]
+
+    def sha(a):
+        return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+    files = {n: open(os.path.join(gdir, n + ".jpg"), "rb").read()
+             for n in ("444_64x48_q85", "422_64x48_q85", "420_37x53_q75", "420_100x70_ri2", "444_opt_ri5",
+                       "440_61x35_ri3", "gray_33x9_ri4", "420_noise_q100", "420_gradient_q50", "444_1x1")}
+    if live:
+        files["420_512x384_q90"] = encode_jpeg(synth_rgb(512, 384, 77), 90, "4:2:0")
+        files["c2_1080p_ri8"] = make_c2(5)
+        files["c2_1080p_twin"] = make_c2(5, restart=False)
     names = list(files)
     with hjd.BatchDecoder(0, hjd.FLAG_KEEP_PLANES) as d1, hjd.BatchDecoder(0) as d2, hjd.BatchDecoder(0, hjd.FLAG_BMP_OUT) as d3:
         for d in (d1, d2, d3):
@@ -312,6 +325,13 @@ def test_against_the_reference_itself(hjd, refbind, tmp_path):
             assert (d.status() == 0).all(), d.status()
         coef, slab = d1.coefficients(), d1.plane_slab()
         for i, n in enumerate(names):
+            if not live:
+                g = golden[n]
+                assert sha(d1.image_coefficients(i, coef)) == g["coef_sha256"], n
+                planes = [p for p in d1.planes(i, slab) if p is not None]
+                assert sha(np.concatenate([p.ravel() for p in planes])) == g["planes_sha256"], n
+                assert sha(d1.rgb(i)) == g["rgb_sha256"] and sha(d2.rgb(i)) == g["rgb_sha256"], n
+                continue
             r = refbind.decode(files[n], mode=1)
             assert r["rc"] == 0, n
             assert np.array_equal(d1.image_coefficients(i, coef), r["coef"]), n

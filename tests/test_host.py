@@ -75,14 +75,14 @@ def test_idct_constants_match_oracle(hjd, port):
     assert (c[:, 0] == 1.0).all()          # the kernels rely on cos(0) == 1 exactly
 
 
-def test_no_gpu_means_loud_failure(hjd):
+def test_no_gpu_means_loud_failure(hjd, tmp_path):
     if hjd.lib().hjd_device_count() > 0:
         pytest.skip("a GPU is present")
     with pytest.raises(hjd.HjdError, match="no CUDA device"):
         hjd.BatchDecoder(0)
     with pytest.raises(hjd.HjdError):
         hjd.DecodeJpgFileData(cases.small_cases()["444_1x1"])
-    assert hjd.ConvertJpgFile("/nonexistent.jpg", "/tmp/x.bmp") == 0
+    assert hjd.ConvertJpgFile(str(tmp_path / "missing.jpg"), str(tmp_path / "x.bmp")) == 0
 
 
 def test_product_does_not_touch_the_oracle():
