@@ -90,11 +90,19 @@ def _dht_payload(tc, th, bits, vals) -> bytes:
     return bytes([(tc << 4) | th]) + bytes(bits) + bytes(vals)
 
 
+def _dqt_payload(tid: int, q) -> bytes:
+    q = [int(v) for v in q]
+    assert len(q) == 64 and all(1 <= v <= 255 for v in q), "8-bit tables, zig-zag order"
+    return bytes([tid]) + bytes(q)
+
+
 def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = None, restart_interval: int = 0,
-            sof_precision: int | None = None, sos_override: bytes | None = None, trailer: bytes = b"\xff\xd9") -> bytes:
+            sof_precision: int | None = None, sos_override: bytes | None = None, trailer: bytes = b"\xff\xd9",
+            quant: dict | None = None, tq: list | None = None) -> bytes:
     """Re-emit `jpg` (baseline, decoded to `coef` [blocks, 64] zig-zag with absolute DC, scan order) with the
     Huffman tables of `tables` ({(class, id): (bits, vals)} overriding the file's own), a new restart interval,
-    and optional header oddities."""
+    and optional header oddities.  `quant` ({table id: 64 values, zig-zag order}) replaces the file's DQT segments;
+    `tq` sets each component's quantisation table selector in the SOF."""
     segs, _ = segments(jpg)
     tabs = dht_tables(segs)
     if tables:
@@ -133,6 +141,8 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
             diff = int(blk[0]) - pred[comp]
             pred[comp] = int(blk[0])
             cat = abs(diff).bit_length()
+            if cat not in dc_codes:
+                raise ValueError(f"DC difference {diff} (MCU {mcu}, block {bi}) has no code in the DC table")
             c, length = dc_codes[cat]
             bw.put(c, length)
             bw.put(diff if diff >= 0 else diff + (1 << cat) - 1, cat)
@@ -159,11 +169,23 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
     scan += bw.out
 
     out = bytearray(b"\xff\xd8")
+    dqt_done = False
     for m, p in segs:
         if m in (0xC4, 0xDA, 0xDD):
             continue
+        if m == 0xDB and quant is not None:
+            if not dqt_done:                    # all of `quant` where the file's first DQT was
+                for tid, q in sorted(quant.items()):
+                    out += _seg(0xDB, _dqt_payload(tid, q))
+                dqt_done = True
+            continue
         if m in (0xC0, 0xC1) and sof_precision is not None:
             p = bytes([sof_precision]) + p[1:]
+        if m in (0xC0, 0xC1) and tq is not None:
+            p = bytearray(p)
+            for c in range(ncomp):
+                p[6 + 3 * c + 2] = tq[c]
+            p = bytes(p)
         out += _seg(m, p)
     for (tc, th), (bits, vals) in sorted(tabs.items()):
         out += _seg(0xC4, _dht_payload(tc, th, bits, vals))
@@ -172,6 +194,29 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
     out += _seg(0xDA, sos_override if sos_override is not None else sos)
     out += scan + trailer
     return bytes(out)
+
+
+def block_index(geometry: dict, ncomp: int, mcu: int, comp: int, sub: int = 0) -> int:
+    """Row of the [blocks, 64] scan-order coefficient array that holds block `sub` (luma: raster order inside the MCU)
+    of component `comp` in MCU `mcu`."""
+    ny = geometry["hf"] * geometry["vf"] if ncomp == 3 else 1
+    bpm = ny + 2 if ncomp == 3 else 1
+    assert (sub < ny) if comp == 0 else sub == 0
+    return mcu * bpm + (sub if comp == 0 else ny + comp - 1)
+
+
+def blocks_to_jpeg(template: bytes, blocks: np.ndarray, geometry: dict, quant: dict, tq: list | None = None,
+                   tables: dict | None = None, restart_interval: int = 0) -> bytes:
+    """A baseline file that holds exactly `blocks` ([blocks, 64] int, zig-zag order, absolute DC, MCU / scan order).
+    `template` gives size, sampling and Huffman tables: a file written by PIL with its standard tables, which code
+    every DC category 0-11 and every AC run/size; `geometry` is its port.decode(..., entropy_only=True)["geometry"].
+    `quant` ({id: 64 values, zig-zag}) and `tq` (table id per component, default 0, 1, 1 / 0) are the
+    quantisation tables written."""
+    ncomp = geometry["ncomp"]
+    if tq is None:
+        tq = [0, 1, 1][:ncomp]
+    return rewrite(template, np.asarray(blocks), geometry, tables=tables, restart_interval=restart_interval,
+                   quant=quant, tq=tq)
 
 
 def replace_tables(jpg: bytes, tables: dict, sof_precision: int | None = None, sos_override: bytes | None = None) -> bytes:
