@@ -25,7 +25,7 @@ import numpy as np
 
 __all__ = ["probe", "MultiDecoder", "shard_range_c", "ConvertJpgFile", "ConvertJpgFiles", "DecodeJpgFileData", "JpegGetImageSize", "WriteBMP24", "encode_bmp24",
            "BatchDecoder", "HjdError", "lib", "build", "LIB_PATH",
-           "FLAG_KEEP_PLANES", "FLAG_HOST_SCAN", "FLAG_NO_SELFSYNC", "FLAG_FUSED_MCU", "FLAG_BMP_OUT", "FLAG_TENSOR_CORE_IDCT", "FLAG_CUDA_CORE_IDCT", "idct_matrix", "idct_tables"]
+           "FLAG_KEEP_PLANES", "FLAG_HOST_SCAN", "FLAG_NO_SELFSYNC", "FLAG_FUSED_MCU", "FLAG_BMP_OUT", "FLAG_TENSOR_CORE_IDCT", "FLAG_CUDA_CORE_IDCT", "FLAG_MULTI_SCAN", "scans", "idct_matrix", "idct_tables"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HJD_LIB_PATH") or os.path.join(_HERE, "libhjd.so")   # override: tuning builds only
@@ -38,6 +38,7 @@ FLAG_FUSED_MCU = 16
 FLAG_BMP_OUT = 32
 FLAG_TENSOR_CORE_IDCT = 128  # always the fused kernel with the IDCT's fast tier as tcgen05.mma
 FLAG_CUDA_CORE_IDCT = 64     # always the fused kernel with the fast tier as FP32 FMA chains (default: chosen per chunk)
+FLAG_MULTI_SCAN = 256        # also decode progressive and non-interleaved files (each exactly like its baseline twin)
 
 IMG_WARN_BAD_CODE, IMG_WARN_COEF_RANGE, IMG_WARN_OVERRUN, IMG_WARN_RESTART = 1, 2, 4, 8
 
@@ -53,6 +54,12 @@ class ImageInfo(ctypes.Structure):
                 ("block_base", c_uint64), ("n_blocks", c_uint64), ("rgb_offset", c_uint64),
                 ("y_offset", c_uint64), ("cb_offset", c_uint64), ("cr_offset", c_uint64),
                 ("y_pitch", c_uint32), ("c_pitch", c_uint32), ("status", c_int32)]
+
+
+class ScanInfo(ctypes.Structure):
+    _fields_ = [("ncomp", c_uint8), ("comp", c_uint8 * 3), ("ss", c_uint8), ("se", c_uint8), ("ah", c_uint8),
+                ("al", c_uint8), ("level", c_uint8), ("pad", c_uint8 * 3), ("restart_interval", c_uint32),
+                ("bytes", c_uint32)]
 
 
 class Timings(ctypes.Structure):
@@ -136,6 +143,9 @@ _SIGS = {
     "hjd_multi_decode_host": (c_int, [c_void_p, c_void_p, POINTER(c_int64), POINTER(c_int64), c_int, c_void_p, c_uint64,
                                       POINTER(c_uint64), c_void_p]),
     "hjd_probe_jpeg": (c_int, [c_void_p, c_int64, POINTER(ImageInfo)]),
+    "hjd_probe_jpeg_flags": (c_int, [c_void_p, c_int64, c_uint, POINTER(ImageInfo)]),
+    "hjd_probe_jpeg_scans": (c_int, [c_void_p, c_int64, POINTER(ScanInfo), c_int]),
+    "hjd_batch_num_scans": (c_int, [c_void_p, c_int]),
     "hjd_huff_lookup_probe": (c_uint32, [c_void_p, c_void_p, c_int, c_int, c_uint32]),
 }
 
@@ -212,12 +222,26 @@ def JpegGetImageSize(buf: bytes):
     return w.value, h.value
 
 
-def probe(buf: bytes):
-    """Header parse only (no GPU): (status, ImageInfo) -- the per-image status a batch would report."""
+def probe(buf: bytes, flags: int = 0):
+    """Header parse only (no GPU): (status, ImageInfo) -- the per-image status a batch created with `flags` would report."""
     data = np.frombuffer(buf, dtype=np.uint8)
     o = ImageInfo()
-    st = lib().hjd_probe_jpeg(data.ctypes.data if data.size else None, data.size, ctypes.byref(o))
+    st = lib().hjd_probe_jpeg_flags(data.ctypes.data if data.size else None, data.size, flags, ctypes.byref(o))
     return int(st), o
+
+
+def scans(buf: bytes) -> list[dict]:
+    """The scans a FLAG_MULTI_SCAN batch decodes the file from (no GPU): one dict per scan with ncomp, comp (frame
+    component indices), ss, se, ah, al, level, restart_interval, bytes.  Raises HjdError for an undecodable file."""
+    data = np.frombuffer(buf, dtype=np.uint8)
+    ptr = data.ctypes.data if data.size else None
+    n = lib().hjd_probe_jpeg_scans(ptr, data.size, None, 0)
+    if n < 0:
+        raise HjdError(f"not a decodable JPEG (status {n})")
+    out = (ScanInfo * max(n, 1))()
+    lib().hjd_probe_jpeg_scans(ptr, data.size, out, n)
+    return [dict(ncomp=s.ncomp, comp=list(s.comp[:s.ncomp]), ss=s.ss, se=s.se, ah=s.ah, al=s.al, level=s.level,
+                 restart_interval=s.restart_interval, bytes=s.bytes) for s in out[:n]]
 
 
 def WriteBMP24(szBmpFileName: str, Width: int, Height: int, RGB) -> None:
@@ -363,6 +387,13 @@ class BatchDecoder:
     @property
     def num_images(self) -> int:
         return lib().hjd_batch_num_images(self._h)
+
+    def num_scans(self, i: int) -> int:
+        """Scans image i of the last upload is decoded from (1: single-scan baseline, 0: not decodable)."""
+        n = lib().hjd_batch_num_scans(self._h, i)
+        if n < 0:
+            raise HjdError(f"hjd_batch_num_scans failed: {_err()}")
+        return n
 
     def info(self, i: int) -> ImageInfo:
         o = ImageInfo()

@@ -8,6 +8,7 @@
 #include "jpeg_parse.h"
 #include "kernels.cuh"
 #include "selfsync.cuh"
+#include "multiscan.cuh"
 
 #include <cuda_runtime.h>
 #include <math.h>
@@ -17,6 +18,7 @@
 #include <sys/syscall.h>
 #include <unistd.h>
 #include <atomic>
+#include <memory>
 #include <string>
 #include <thread>
 #include <unordered_map>
@@ -26,6 +28,8 @@
 // ------------------------------------------------------------------------------------------
 // errors
 // ------------------------------------------------------------------------------------------
+static_assert(HJD_MAX_SCANS == HJD_MAX_SCANS_PER_IMAGE, "hjd_types.h and include/hjd.h state the same scan cap");
+
 static thread_local std::string g_err;
 
 static int fail(int code, const char* what, const char* detail = nullptr)
@@ -101,6 +105,9 @@ struct Chunk {
     uint32_t ck0 = 0, n_ck = 0;               // 16-byte de-stuffing chunks
     uint32_t sw0 = 0, sw1 = 0, sf0 = 0, sf1 = 0;   // work items: speculative / write kernels, synchronisation kernel
     uint32_t ss_range = 0;                    // sub-sequences per warp in the synchronisation kernel
+    // multi-scan images of this chunk: their slab blocks (zeroed before the first level), their work items per level
+    std::vector<std::pair<uint64_t, uint64_t>> ms_zero;     // (first block, blocks)
+    std::vector<std::pair<uint32_t, uint32_t>> ms_levels;   // work item range of each level present, in level order
 };
 
 #define HJD_NSTREAMS 3
@@ -139,7 +146,16 @@ struct hjd_batch {
     uint64_t ss_dst_bytes = 0;
     bool ss_ran = false;                        // the last decode ran kernel 1b (its round count is in d_flag)
     int max_sync_ctas = 1;                      // grid limit of the cooperative synchronisation kernel on this device
-    std::vector<uint8_t> host_restart_warn;     // HJD_FLAG_HOST_SCAN only
+    std::vector<uint8_t> host_restart_warn;     // HJD_FLAG_HOST_SCAN only (and multi-scan images)
+    // multi-scan images (HJD_FLAG_MULTI_SCAN, csrc/multiscan.cu)
+    std::vector<HjdScanDesc> scans;
+    std::vector<HjdMsWork> mswork;              // one per (scan, restart interval), image order; sorted per chunk
+    std::vector<uint32_t> ms_starts;            // interval starts of every scan (relative to the scan)
+    std::vector<HjdHuffTable> ms_tabs;          // per-scan Huffman tables, de-duplicated by content
+    std::unordered_multimap<uint64_t, uint32_t> ms_tab_of;
+    std::vector<std::vector<uint8_t>> ms_tab_raw;
+    std::vector<uint32_t> ms_items, n_scans;    // per image: work items (multi-scan images), scans (0: not decodable)
+    std::vector<uint32_t> ms_w0;                // per image: its first work item (n + 1 entries)
     std::unordered_multimap<uint64_t, uint32_t> tset_of, qset_of;   // content hash -> candidate sets (verified byte for byte)
     std::vector<HjdRawTables> tset_raw, qset_raw;                    // what each set was built from
     uint64_t total_blocks = 0, rgb_bytes = 0, plane_bytes = 0, scan_bytes = 0, pixels = 0, arena_bytes = 0;
@@ -152,6 +168,7 @@ struct hjd_batch {
     int tc_chunks = 0, cc_chunks = 0;           // chunks of the last decode whose MCUs went through the tensor-core / CUDA-core fused kernel
 
     DevBuf d_arena, d_imgs, d_tsets, d_qsets, d_work, d_segs, d_mcucta, d_slices, d_slicecnt, d_istart, d_coef, d_planes, d_rgb, d_status;
+    DevBuf d_scans, d_mswork, d_msstarts, d_mstabs;
     DevBuf d_ss, d_sswork, d_sssegs, d_destuff, d_dlen, d_counts, d_scantmp, d_ssE0, d_ssX, d_ssnb, d_flag;
     PinBuf h_meta, h_out;                       // h_out: staging of the single-image calls
 };
@@ -244,6 +261,7 @@ extern "C" void hjd_batch_destroy(hjd_batch* b)
     b->d_ss.release(); b->d_sswork.release(); b->d_sssegs.release(); b->d_destuff.release(); b->d_dlen.release(); b->d_counts.release();
     b->d_scantmp.release(); b->d_ssE0.release(); b->d_ssX.release(); b->d_ssnb.release();
     b->d_flag.release();
+    b->d_scans.release(); b->d_mswork.release(); b->d_msstarts.release(); b->d_mstabs.release();
     b->h_meta.release(); b->h_out.release();
     for (int i = 0; i < 5; i++) if (b->ev[i]) cudaEventDestroy(b->ev[i]);
     for (int i = 0; i < HJD_MARK_SLOTS; i++) if (b->mark[i]) cudaEventDestroy(b->mark[i]);
@@ -264,6 +282,73 @@ extern "C" int hjd_batch_set_stream(hjd_batch* b, void* cuda_stream)
     return HJD_OK;
 }
 
+// Index of the per-scan Huffman table built from `raw` (mode 0: DC, 1: sequential AC, 2: progressive AC with the raw
+// run), shared by every scan of the batch with the same contents; -1: the code is over-subscribed.
+static int ms_table(hjd_batch* b, const HjdRawHuff& raw, int mode)
+{
+    std::vector<uint8_t> key(17 + (size_t)raw.nvals);
+    key[0] = (uint8_t)mode;
+    memcpy(&key[1], raw.bits, 16);
+    memcpy(&key[17], raw.vals, (size_t)raw.nvals);
+    uint64_t h = 1469598103934665603ull;
+    for (uint8_t v : key) { h ^= v; h *= 1099511628211ull; }
+    auto range = b->ms_tab_of.equal_range(h);
+    for (auto it = range.first; it != range.second; ++it)
+        if (b->ms_tab_raw[it->second] == key) return (int)it->second;
+    HjdHuffTable t;
+    if (!(mode == 2 ? hjd_build_huff_table_raw(raw, &t) : hjd_build_huff_table(raw, mode == 1, &t))) return -1;
+    b->ms_tabs.push_back(t);
+    b->ms_tab_raw.push_back(std::move(key));
+    b->ms_tab_of.emplace(h, (uint32_t)b->ms_tabs.size() - 1);
+    return (int)b->ms_tabs.size() - 1;
+}
+
+// Scan descriptors, tables, interval starts and work items of multi-scan image i (file at arena offset dev_off).
+// A scan with fewer RSTn markers than its DRI implies (a file cut inside it) gets the intervals it has: the last one
+// runs to the end of the data, and the image is flagged HJD_IMG_WARN_RESTART.  HJD_IMG_OK or HJD_IMG_ERR_BAD_TABLE.
+static int ms_add_image(hjd_batch* b, int i, const HjdMultiParsed& mp, uint64_t dev_off)
+{
+    const size_t scan0 = b->scans.size(), start0 = b->ms_starts.size(), work0 = b->mswork.size();
+    uint32_t items = 0;
+    for (const HjdScanParsed& p : mp.scans) {
+        HjdScanDesc sd;
+        memset(&sd, 0, sizeof sd);
+        sd.image = (uint32_t)i;
+        sd.ncomp = (uint8_t)p.ncomp;
+        for (int k = 0; k < p.ncomp; k++) sd.comp[k] = (uint8_t)p.comp[k];
+        sd.ss = (uint8_t)p.ss; sd.se = (uint8_t)p.se; sd.ah = (uint8_t)p.ah; sd.al = (uint8_t)p.al;
+        sd.kind = (uint8_t)p.kind; sd.level = (uint8_t)(p.level < 255 ? p.level : 255);
+        sd.restart_interval = p.restart_interval;
+        hjd_scan_grid(mp.frame, p, &sd.mcus_x, &sd.mcus_y);
+        const uint64_t total = (uint64_t)sd.mcus_x * sd.mcus_y;
+        const uint64_t want = p.restart_interval ? (total + p.restart_interval - 1) / p.restart_interval : 1;
+        sd.n_intervals = (uint32_t)(want < p.n_starts ? want : p.n_starts);
+        if (p.restart_interval && p.n_starts != want) b->host_restart_warn[i] = 1;
+        sd.start_base = (uint32_t)b->ms_starts.size();
+        sd.scan_len = (uint32_t)p.len;
+        sd.scan_off = dev_off + p.off;
+        for (int k = 0; k < p.ncomp; k++) {
+            const int td = p.dc[k].present ? ms_table(b, p.dc[k], 0) : 0;
+            const int ta = p.ac[k].present ? ms_table(b, p.ac[k], p.kind == HJD_SCAN_SEQ ? 1 : 2) : 0;
+            if (td < 0 || ta < 0) {
+                b->scans.resize(scan0); b->ms_starts.resize(start0); b->mswork.resize(work0);
+                return HJD_IMG_ERR_BAD_TABLE;
+            }
+            sd.dc_tab[k] = (uint32_t)td;
+            sd.ac_tab[k] = (uint32_t)ta;
+        }
+        for (uint32_t j = 0; j < sd.n_intervals; j++) {
+            b->ms_starts.push_back(mp.starts[p.first_start + j]);
+            b->mswork.push_back(HjdMsWork{(uint32_t)b->scans.size(), j});
+        }
+        items += sd.n_intervals;
+        b->scans.push_back(sd);
+    }
+    b->ms_items[i] = items;
+    b->n_scans[i] = (uint32_t)mp.scans.size();
+    return HJD_OK;
+}
+
 // Parse + lay out + upload the metadata.  b->files[i].dev_off must already hold the arena offset of
 // file i.  The files themselves are copied by copy_files(), whole or chunk by chunk.
 static int upload_common(hjd_batch* b, bool chunked)
@@ -279,6 +364,8 @@ static int upload_common(hjd_batch* b, bool chunked)
     b->host_istart.clear();
     b->host_restart_warn.assign(n, 0);
     b->ss.clear(); b->sswork.clear(); b->sssegs.clear();
+    b->scans.clear(); b->mswork.clear(); b->ms_starts.clear(); b->ms_tabs.clear(); b->ms_tab_of.clear(); b->ms_tab_raw.clear();
+    b->ms_items.assign(n, 0); b->n_scans.assign(n, 0); b->ms_w0.assign((size_t)n + 1, 0);
     b->ss_subs = b->ss_chunks = 0;
     b->ss_dst_bytes = 0;
     b->total_blocks = b->rgb_bytes = b->plane_bytes = b->scan_bytes = b->pixels = 0;
@@ -305,6 +392,9 @@ static int upload_common(hjd_batch* b, bool chunked)
         int trep, qrep;            // image whose tables / quantisation tables these are byte-identical to (itself: a representative)
     };
     std::vector<Lite> lite((size_t)n);
+    // HJD_FLAG_MULTI_SCAN: files the single-scan parse rejects as unsupported get the multi-scan walk; these
+    // images keep the result (scans, interval starts, table snapshots) for the serial pass
+    std::vector<std::unique_ptr<HjdMultiParsed>> multi((size_t)n);
     auto parse_range = [&](int lo, int hi) {
         HjdParsed p;
         struct Seen { uint64_t key; int image; HjdRawTables raw; };
@@ -316,6 +406,15 @@ static int upload_common(hjd_batch* b, bool chunked)
             int st = (files[i].ptr && files[i].size > 0) ? hjd_parse_jpeg(files[i].ptr, (size_t)files[i].size, &p)
                                                          : HJD_IMG_ERR_NOT_JPEG;
             if (st == HJD_IMG_OK && p.scan_len > 0xFFFFFF00ull) st = HJD_IMG_ERR_UNSUPPORTED;
+            if (st == HJD_IMG_ERR_UNSUPPORTED && (b->flags & HJD_FLAG_MULTI_SCAN)) {
+                std::unique_ptr<HjdMultiParsed> mp(new HjdMultiParsed());
+                st = hjd_parse_jpeg_multi(files[i].ptr, (size_t)files[i].size, mp.get());
+                if (st == HJD_IMG_OK && mp->frame.scan_len > 0xFFFFFF00ull) st = HJD_IMG_ERR_UNSUPPORTED;
+                if (st == HJD_IMG_OK) {
+                    p = mp->frame;
+                    multi[(size_t)i] = std::move(mp);
+                }
+            }
             l.status = st;
             if (st != HJD_IMG_OK) continue;
             l.width = p.width; l.height = p.height; l.restart_interval = p.restart_interval;
@@ -324,10 +423,11 @@ static int upload_common(hjd_batch* b, bool chunked)
             l.tk = hjd_table_key(p); l.qk = hjd_quant_key(p);
             hjd_raw_tables(p, &raw);
             l.trep = l.qrep = i;
-            bool hit = false;
+            bool hit = multi[(size_t)i] != nullptr;      // multi-scan images carry per-scan tables instead of a table set
             for (const Seen& sn : seen_t)
                 if (sn.key == l.tk && memcmp(sn.raw.huff, raw.huff, sizeof raw.huff) == 0) { l.trep = sn.image; hit = true; break; }
             if (!hit && seen_t.size() < 64) seen_t.push_back(Seen{l.tk, i, raw});
+            if (multi[(size_t)i]) hit = false;
             hit = false;
             for (const Seen& sn : seen_q)
                 if (sn.key == l.qk && memcmp(sn.raw.quant, raw.quant, sizeof raw.quant) == 0) { l.qrep = sn.image; hit = true; break; }
@@ -363,7 +463,13 @@ static int upload_common(hjd_batch* b, bool chunked)
         int st = ps.status;
         uint32_t tset = 0, qset = 0;
         bool have_full = false;
-        if (st == HJD_IMG_OK) {
+        const HjdMultiParsed* mp = multi[(size_t)i].get();
+        if (st == HJD_IMG_OK && mp) {
+            st = ms_add_image(b, i, *mp, files[i].dev_off);
+            full = mp->frame;
+            hjd_raw_tables(full, &full_raw);
+            have_full = true;
+        } else if (st == HJD_IMG_OK) {
             if (ps.trep != i) {                                     // byte-identical to an earlier image of its worker
                 if (b->parse_status[ps.trep] != HJD_IMG_OK) st = b->parse_status[ps.trep];      // e.g. an over-subscribed DHT
                 tset = tset_of_img[(size_t)ps.trep];
@@ -404,7 +510,9 @@ static int upload_common(hjd_batch* b, bool chunked)
         }
         tset_of_img[(size_t)i] = tset; qset_of_img[(size_t)i] = qset;
         b->parse_status[i] = st;
+        b->ms_w0[(size_t)i + 1] = (uint32_t)b->mswork.size();
         if (st != HJD_IMG_OK) { b->any_parse_error = true; continue; }   // n_intervals = n_blocks = 0: skipped
+        if (!mp) b->n_scans[i] = 1;
 
         d.width = ps.width; d.height = ps.height;
         d.ncomp = (uint8_t)ps.ncomp; d.hf = (uint8_t)ps.hf; d.vf = (uint8_t)ps.vf;
@@ -416,7 +524,8 @@ static int upload_common(hjd_batch* b, bool chunked)
         d.n_intervals = ps.restart_interval ? (d.n_mcus + ps.restart_interval - 1) / ps.restart_interval : 1;
         d.scan_len = (uint32_t)ps.scan_len;
         d.scan_off = files[i].dev_off + ps.scan_off;
-        if (!(b->flags & HJD_FLAG_NO_SELFSYNC) && ps.restart_interval == 0 && ps.scan_len >= HJD_SS_MIN_BYTES) {
+        if (mp) d.n_intervals = 0;                   // entropy decode by the multi-scan kernel only (no kernel 0 / 1a / 1b)
+        if (!mp && !(b->flags & HJD_FLAG_NO_SELFSYNC) && ps.restart_interval == 0 && ps.scan_len >= HJD_SS_MIN_BYTES) {
             // restart-free scan: kernel 1b (speculative self-synchronising decode) instead of one thread
             HjdSsImage si;
             memset(&si, 0, sizeof si);
@@ -560,6 +669,39 @@ static int upload_common(hjd_batch* b, bool chunked)
         }
         c.work1 = (uint32_t)b->work.size();
         if (c.arena_lo == ~0ull) c.arena_lo = c.arena_hi = 0;
+        // multi-scan work of the chunk: by level (one launch each), then by kind, so that the lanes of a warp mostly run
+        // the same loop.  A counting sort: a comparison sort of the 30 M items of 1024 1080p files with restart markers
+        // every 8 blocks took seconds of host time.
+        {
+            const uint32_t w0 = b->ms_w0[(size_t)c.img0], w1 = b->ms_w0[(size_t)c.img1];
+            std::vector<uint32_t> at(256 * 5 + 1, 0);
+            for (uint32_t k = w0; k < w1; k++) {
+                const HjdScanDesc& sd = b->scans[b->mswork[k].scan];
+                at[sd.level * 5u + sd.kind + 1]++;
+            }
+            for (size_t q = 1; q < at.size(); q++) at[q] += at[q - 1];
+            std::vector<HjdMsWork> sorted(w1 - w0);
+            for (uint32_t k = w0; k < w1; k++) {
+                const HjdScanDesc& sd = b->scans[b->mswork[k].scan];
+                sorted[at[sd.level * 5u + sd.kind]++] = b->mswork[k];
+            }
+            std::copy(sorted.begin(), sorted.end(), b->mswork.begin() + w0);
+            for (uint32_t k = w0; k < w1;) {
+                const uint8_t lv = b->scans[b->mswork[k].scan].level;
+                uint32_t e = k;
+                while (e < w1 && b->scans[b->mswork[e].scan].level == lv) e++;
+                c.ms_levels.emplace_back(k, e);
+                k = e;
+            }
+            for (int i = c.img0; i < c.img1; i++) {
+                if (b->ms_w0[(size_t)i + 1] == b->ms_w0[(size_t)i] || b->parse_status[i] != HJD_IMG_OK) continue;
+                const HjdImageDesc& d = b->imgs[i];
+                if (!c.ms_zero.empty() && c.ms_zero.back().first + c.ms_zero.back().second == d.block_base)
+                    c.ms_zero.back().second += d.n_blocks;
+                else
+                    c.ms_zero.emplace_back(d.block_base, d.n_blocks);
+            }
+        }
     }
 
     // device slabs
@@ -679,10 +821,22 @@ static int upload_common(hjd_batch* b, bool chunked)
     const size_t sz_is = sizeof(uint32_t) * b->host_istart.size();
     const size_t sz_ss = sizeof(HjdSsImage) * b->ss.size();
     const size_t sz_sw = sizeof(HjdSsWork) * b->sswork.size();
+    const size_t sz_sd = sizeof(HjdScanDesc) * b->scans.size();
+    const size_t sz_mw = sizeof(HjdMsWork) * b->mswork.size();
+    const size_t sz_mst = sizeof(uint32_t) * b->ms_starts.size();
+    const size_t sz_mt = sizeof(HjdHuffTable) * b->ms_tabs.size();
+    if (sz_sd) {
+        CU(b->d_scans.ensure(sz_sd));
+        CU(b->d_mswork.ensure(sz_mw + 16));
+        CU(b->d_msstarts.ensure(sz_mst + 16));
+        CU(b->d_mstabs.ensure(sz_mt + 16));
+    }
     size_t o_imgs = 0, o_ts = align_up(o_imgs + sz_imgs, 256), o_qs = align_up(o_ts + sz_ts, 256),
            o_wk = align_up(o_qs + sz_qs, 256), o_is = align_up(o_wk + sz_wk, 256),
            o_ss = align_up(o_is + sz_is, 256), o_sw = align_up(o_ss + sz_ss, 256),
-           o_sg = align_up(o_sw + sz_sw, 256), o_s2 = align_up(o_sg + sz_sg, 256), o_mc = align_up(o_s2 + sz_s2, 256), o_sl = align_up(o_mc + sz_mc, 256), tot = o_sl + sz_sl;
+           o_sg = align_up(o_sw + sz_sw, 256), o_s2 = align_up(o_sg + sz_sg, 256), o_mc = align_up(o_s2 + sz_s2, 256), o_sl = align_up(o_mc + sz_mc, 256),
+           o_sd = align_up(o_sl + sz_sl, 256), o_mw = align_up(o_sd + sz_sd, 256), o_mst = align_up(o_mw + sz_mw, 256),
+           o_mt = align_up(o_mst + sz_mst, 256), tot = o_mt + sz_mt;
     CU(b->h_meta.ensure(tot + 256));
     uint8_t* hm = (uint8_t*)b->h_meta.p;
     memcpy(hm + o_imgs, b->imgs.data(), sz_imgs);
@@ -696,6 +850,16 @@ static int upload_common(hjd_batch* b, bool chunked)
     if (sz_is) memcpy(hm + o_is, b->host_istart.data(), sz_is);
     if (sz_ss) memcpy(hm + o_ss, b->ss.data(), sz_ss);
     if (sz_sw) memcpy(hm + o_sw, b->sswork.data(), sz_sw);
+    if (sz_sd) {
+        memcpy(hm + o_sd, b->scans.data(), sz_sd);
+        memcpy(hm + o_mw, b->mswork.data(), sz_mw);
+        memcpy(hm + o_mst, b->ms_starts.data(), sz_mst);
+        memcpy(hm + o_mt, b->ms_tabs.data(), sz_mt);
+        CU(cudaMemcpyAsync(b->d_scans.p, hm + o_sd, sz_sd, cudaMemcpyHostToDevice, b->stream));
+        CU(cudaMemcpyAsync(b->d_mswork.p, hm + o_mw, sz_mw, cudaMemcpyHostToDevice, b->stream));
+        CU(cudaMemcpyAsync(b->d_msstarts.p, hm + o_mst, sz_mst, cudaMemcpyHostToDevice, b->stream));
+        CU(cudaMemcpyAsync(b->d_mstabs.p, hm + o_mt, sz_mt, cudaMemcpyHostToDevice, b->stream));
+    }
     if (sz_imgs) CU(cudaMemcpyAsync(b->d_imgs.p, hm + o_imgs, sz_imgs, cudaMemcpyHostToDevice, b->stream));
     if (sz_ts) CU(cudaMemcpyAsync(b->d_tsets.p, hm + o_ts, sz_ts, cudaMemcpyHostToDevice, b->stream));
     if (sz_qs) CU(cudaMemcpyAsync(b->d_qsets.p, hm + o_qs, sz_qs, cudaMemcpyHostToDevice, b->stream));
@@ -878,6 +1042,15 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
                                       b->max_tabs, (int16_t*)b->d_coef.p, status, st));
         b->launches += 1;
     }
+    // multi-scan images: nothing else writes their blocks, and refinement scans read what the levels below left
+    for (const auto& z : c.ms_zero)
+        CU(cudaMemsetAsync((int16_t*)b->d_coef.p + z.first * 64, 0, z.second * 128, st));
+    for (const auto& lv : c.ms_levels) {
+        CU(hjd_launch_multiscan(arena, imgs, (const HjdScanDesc*)b->d_scans.p, (const HjdMsWork*)b->d_mswork.p + lv.first,
+                                (int)(lv.second - lv.first), (const uint32_t*)b->d_msstarts.p,
+                                (const HjdHuffTable*)b->d_mstabs.p, (int16_t*)b->d_coef.p, status, st));
+        b->launches += 1;
+    }
     if (ev) CU(cudaEventRecord(ev[2], st));
     if (!(b->flags & HJD_FLAG_KEEP_PLANES)) {
         // default: kernels 2+3 fused per MCU, planes never reach HBM
@@ -1010,7 +1183,14 @@ extern "C" int hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* o)
     o->block_base = d.block_base; o->n_blocks = d.n_blocks; o->rgb_offset = d.rgb_off;
     o->y_offset = d.y_off; o->cb_offset = d.cb_off; o->cr_offset = d.cr_off;
     o->y_pitch = d.y_pitch; o->c_pitch = d.c_pitch; o->status = b->parse_status[i];
+    if (b->ms_items[i]) o->n_intervals = b->ms_items[i];
     return HJD_OK;
+}
+
+extern "C" int hjd_batch_num_scans(const hjd_batch* b, int i)
+{
+    if (!b || i < 0 || i >= (int)b->imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_num_scans", "bad arguments");
+    return (int)b->n_scans[i];
 }
 
 extern "C" int hjd_batch_get_status(hjd_batch* b, int32_t* status)
@@ -1140,9 +1320,16 @@ extern "C" uint64_t hjd_out_slab_bytes(const uint8_t* arena, const int64_t* offs
     uint64_t total = 0;
     if (!arena || !offsets || !sizes) return 0;
     HjdParsed ps;
-    for (int i = 0; i < n; i++)
-        if (hjd_parse_jpeg(arena + offsets[i], (size_t)sizes[i], &ps) == HJD_IMG_OK)
-            total += align_up(image_out_bytes(flags, ps.width, ps.height), 256);
+    std::unique_ptr<HjdMultiParsed> mp;
+    for (int i = 0; i < n; i++) {
+        int st = hjd_parse_jpeg(arena + offsets[i], (size_t)sizes[i], &ps);
+        if (st == HJD_IMG_ERR_UNSUPPORTED && (flags & HJD_FLAG_MULTI_SCAN)) {
+            if (!mp) mp.reset(new HjdMultiParsed());
+            st = hjd_parse_jpeg_multi(arena + offsets[i], (size_t)sizes[i], mp.get());
+            ps = mp->frame;
+        }
+        if (st == HJD_IMG_OK) total += align_up(image_out_bytes(flags, ps.width, ps.height), 256);
+    }
     return total;
 }
 
@@ -1329,6 +1516,79 @@ extern "C" int hjd_probe_jpeg(const uint8_t* buf, int64_t size, hjd_image_info* 
     } else ps.status = st;
     if (out) fill_info_from_parse(ps, out);
     return ps.status;
+}
+
+// Multi-scan parse plus every table build: the status a batch with HJD_FLAG_MULTI_SCAN reports for the file.
+static int probe_multi(const uint8_t* buf, int64_t size, HjdMultiParsed* mp)
+{
+    int st = hjd_parse_jpeg_multi(buf, (size_t)size, mp);
+    if (st == HJD_IMG_OK && mp->frame.scan_len > 0xFFFFFF00ull) st = HJD_IMG_ERR_UNSUPPORTED;
+    HjdHuffTable t;
+    for (size_t k = 0; st == HJD_IMG_OK && k < mp->scans.size(); k++) {
+        const HjdScanParsed& s = mp->scans[k];
+        for (int c = 0; c < s.ncomp; c++) {
+            if (s.dc[c].present && !hjd_build_huff_table(s.dc[c], false, &t)) st = HJD_IMG_ERR_BAD_TABLE;
+            if (s.ac[c].present && !(s.kind == HJD_SCAN_SEQ ? hjd_build_huff_table(s.ac[c], true, &t) : hjd_build_huff_table_raw(s.ac[c], &t)))
+                st = HJD_IMG_ERR_BAD_TABLE;
+        }
+    }
+    return mp->frame.status = st;
+}
+
+extern "C" int hjd_probe_jpeg_flags(const uint8_t* buf, int64_t size, unsigned flags, hjd_image_info* out)
+{
+    const int st = hjd_probe_jpeg(buf, size, out);
+    if (st != HJD_IMG_ERR_UNSUPPORTED || !(flags & HJD_FLAG_MULTI_SCAN)) return st;
+    std::unique_ptr<HjdMultiParsed> mp(new HjdMultiParsed());
+    probe_multi(buf, size, mp.get());
+    const HjdParsed& f = mp->frame;
+    if (out) {
+        fill_info_from_parse(f, out);
+        if (f.status == HJD_IMG_OK) {
+            out->n_intervals = 0;
+            for (const HjdScanParsed& s : mp->scans) {
+                uint32_t mx, my;
+                hjd_scan_grid(f, s, &mx, &my);
+                const uint64_t want = s.restart_interval ? ((uint64_t)mx * my + s.restart_interval - 1) / s.restart_interval : 1;
+                out->n_intervals += (uint32_t)(want < s.n_starts ? want : s.n_starts);
+            }
+        }
+    }
+    return f.status;
+}
+
+extern "C" int hjd_probe_jpeg_scans(const uint8_t* buf, int64_t size, hjd_scan_info* out, int max)
+{
+    if (max < 0 || (max > 0 && !out)) return fail(HJD_ERR_ARG, "hjd_probe_jpeg_scans", "bad arguments");
+    hjd_image_info info;
+    const int st = hjd_probe_jpeg(buf, size, &info);
+    if (st == HJD_IMG_OK) {                       // one interleaved sequential scan
+        if (max > 0) {
+            memset(out, 0, sizeof *out);
+            out->ncomp = info.ncomp;
+            for (int c = 0; c < info.ncomp; c++) out->comp[c] = (uint8_t)c;
+            out->se = 63;
+            out->restart_interval = info.restart_interval;
+            out->bytes = info.scan_bytes;
+        }
+        return 1;
+    }
+    if (st != HJD_IMG_ERR_UNSUPPORTED) return st;
+    std::unique_ptr<HjdMultiParsed> mp(new HjdMultiParsed());
+    const int ms = probe_multi(buf, size, mp.get());
+    if (ms != HJD_IMG_OK) return ms;
+    for (int k = 0; k < (int)mp->scans.size() && k < max; k++) {
+        const HjdScanParsed& s = mp->scans[(size_t)k];
+        hjd_scan_info& o = out[k];
+        memset(&o, 0, sizeof o);
+        o.ncomp = (uint8_t)s.ncomp;
+        for (int c = 0; c < s.ncomp; c++) o.comp[c] = (uint8_t)s.comp[c];
+        o.ss = (uint8_t)s.ss; o.se = (uint8_t)s.se; o.ah = (uint8_t)s.ah; o.al = (uint8_t)s.al;
+        o.level = (uint8_t)(s.level < 255 ? s.level : 255);
+        o.restart_interval = s.restart_interval;
+        o.bytes = (uint32_t)s.len;
+    }
+    return (int)mp->scans.size();
 }
 
 extern "C" uint32_t hjd_huff_lookup_probe(const uint8_t bits[16], const uint8_t* vals, int nvals, int is_ac, uint32_t peek16)

@@ -150,6 +150,37 @@ struct HjdSsSeg {
     uint32_t n;            // sub-sequences in the segment
 };
 
+// ---- multi-scan path (HJD_FLAG_MULTI_SCAN: progressive and non-interleaved files, csrc/multiscan.cu) ----------
+#define HJD_MAX_SCANS      256   // scans per image; more: HJD_IMG_ERR_UNSUPPORTED (hostile files carry thousands)
+#define HJD_SCAN_SEQ       0     // sequential: the block decode of kernel 1a over the scan's components
+#define HJD_SCAN_DC_FIRST  1
+#define HJD_SCAN_DC_REFINE 2
+#define HJD_SCAN_AC_FIRST  3
+#define HJD_SCAN_AC_REFINE 4
+
+// One scan of one image.  Its MCU is the frame's MCU when it is interleaved (ncomp > 1) and one block of its
+// component otherwise, on the component's own grid ceil(ceil(W h_c / h_max) / 8) x ceil(ceil(H v_c / v_max) / 8).
+// Slab index of (component c, block row by, column bx): block_base + MCU * blocks_per_mcu + (luma:
+// (by % vf) * hf + bx % hf, chroma: hf * vf + c - 1), the layout kernel 1a writes.
+struct HjdScanDesc {
+    uint32_t image;
+    uint8_t  ncomp, comp[3];     // frame component indices, scan order
+    uint8_t  ss, se, ah, al;
+    uint8_t  kind, level, pad[2];
+    uint32_t restart_interval;   // MCUs of this scan, 0 = none
+    uint32_t mcus_x, mcus_y;     // this scan's MCU grid
+    uint32_t n_intervals;
+    uint32_t start_base;         // index of its first interval start in the batch's start table
+    uint32_t scan_len;
+    uint64_t scan_off;           // byte offset of the entropy-coded segment in the file arena
+    uint32_t dc_tab[3], ac_tab[3];   // per scan component: index into the batch's per-scan table pool
+};
+// One work item = one thread of the multi-scan kernel: restart interval `interval` of scan `scan`.
+struct HjdMsWork {
+    uint32_t scan;
+    uint32_t interval;
+};
+
 // Per-image status bits written by kernels (mirrors HJD_IMG_WARN_* in include/hjd.h).
 #define HJD_ST_BAD_CODE     1
 #define HJD_ST_COEF_RANGE   2

@@ -180,16 +180,230 @@ int hjd_parse_jpeg(const uint8_t* buf, size_t size, HjdParsed* o)
     return o->status = HJD_IMG_OK;
 }
 
-static uint32_t sym_fields(uint32_t len, uint32_t sym, bool is_ac)
+// One entropy-coded segment: its length (up to the first marker that is neither FF00 nor RSTn, as
+// hjd_scan_length) and, appended to `starts`, the start of each of its RSTn-delimited intervals (relative to
+// the segment), in the same pass.
+static size_t walk_segment(const uint8_t* scan, size_t avail, std::vector<uint32_t>& starts)
+{
+    starts.push_back(0);
+    const uint8_t* p = scan;
+    const uint8_t* e = scan + avail;
+    while (p + 1 < e) {
+        p = (const uint8_t*)memchr(p, 0xFF, (size_t)(e - 1 - p));
+        if (!p) break;
+        const uint8_t m = p[1];
+        if (m == 0x00) p += 2;
+        else if ((m & 0xF8) == 0xD0) { starts.push_back((uint32_t)(p + 2 - scan)); p += 2; }
+        else if (m == 0xFF) p += 1;                                  // fill byte
+        else return (size_t)(p - scan);
+    }
+    return avail;
+}
+
+int hjd_parse_jpeg_multi(const uint8_t* buf, size_t size, HjdMultiParsed* mp)
+{
+    HjdParsed* o = &mp->frame;
+    memset(o, 0, sizeof *o);
+    mp->scans.clear();
+    mp->starts.clear();
+    o->status = HJD_IMG_ERR_NOT_JPEG;
+    if (!buf || size < 4 || buf[0] != 0xFF || buf[1] != 0xD8) return o->status;
+    Reader r{buf, size, 2};
+    bool have_frame = false, progressive = false;
+    int cid[3] = {0, 0, 0};
+    int chf[3] = {1, 1, 1}, cvf[3] = {1, 1, 1};
+    uint32_t dri = 0;
+    // per (component, coefficient): Al of the last scan that coded it (-1: none yet), level of that scan
+    int al_of[3][64], level_of[3][64];
+    bool seq_done[3] = {false, false, false};
+    for (int c = 0; c < 3; c++)
+        for (int k = 0; k < 64; k++) al_of[c][k] = level_of[c][k] = -1;
+    HjdParsed later;                        // DQT after the first scan: parsed (bounds, errors) but not used
+    // The file ends before EOI: the scans so far are decoded (a missing scan leaves its coefficients 0).
+#define HJD_END_EARLY() do { if (mp->scans.empty()) return o->status = HJD_IMG_ERR_TRUNCATED; goto frame_checks; } while (0)
+
+    for (;;) {
+        if (!r.need(2)) HJD_END_EARLY();
+        if (r.u8() != 0xFF) return o->status = HJD_IMG_ERR_NOT_JPEG;
+        uint8_t m = r.u8();
+        while (m == 0xFF) {
+            if (!r.need(1)) HJD_END_EARLY();
+            m = r.u8();
+        }
+        if (m == 0xD8 || m == 0x01 || (m >= 0xD0 && m <= 0xD7)) continue;
+        if (m == 0xD9) HJD_END_EARLY();
+        if (!r.need(2)) HJD_END_EARLY();
+        const size_t seg = r.i;
+        const uint16_t len = r.u16();
+        if (len < 2 || seg + len > size) HJD_END_EARLY();
+        const size_t end = seg + len;
+
+        if (m == 0xDB) {
+            const int rc = parse_dqt(r, end, mp->scans.empty() ? o : &later);
+            if (rc) return o->status = rc;
+        } else if (m == 0xC4) {
+            const int rc = parse_dht(r, end, o);
+            if (rc) return o->status = rc;
+        } else if (m == 0xC0 || m == 0xC1 || m == 0xC2) {
+            if (have_frame) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            if (len < 8) return o->status = HJD_IMG_ERR_TRUNCATED;
+            const uint8_t prec = r.u8();
+            o->height = r.u16();
+            o->width  = r.u16();
+            o->ncomp  = r.u8();
+            if (prec != 8 || (o->ncomp != 1 && o->ncomp != 3)) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            if (len < 8 + 3 * o->ncomp) return o->status = HJD_IMG_ERR_TRUNCATED;
+            if (o->width == 0 || o->height == 0) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            if ((uint64_t)o->width * o->height > HJD_MAX_PIXELS) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            for (int c = 0; c < o->ncomp; c++) {
+                cid[c] = r.u8();
+                const uint8_t s = r.u8();
+                chf[c] = s >> 4;
+                cvf[c] = s & 15;
+                o->tq[c] = r.u8();
+                if (o->tq[c] > 3) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            }
+            have_frame = true;
+            progressive = (m == 0xC2);
+        } else if (m >= 0xC3 && m <= 0xCF && m != 0xC4 && m != 0xC8 && m != 0xCC) {
+            return o->status = HJD_IMG_ERR_UNSUPPORTED;                           // lossless / arithmetic
+        } else if (m == 0xDD) {
+            if (len < 4) return o->status = HJD_IMG_ERR_TRUNCATED;
+            dri = r.u16();
+        } else if (m == 0xDA) {
+            if (!have_frame) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            if (mp->scans.size() >= HJD_MAX_SCANS) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            if (len < 6) return o->status = HJD_IMG_ERR_TRUNCATED;
+            HjdScanParsed s;
+            memset(&s, 0, sizeof s);
+            s.ncomp = r.u8();
+            if (s.ncomp < 1 || s.ncomp > o->ncomp) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            if (len < 6 + 2 * s.ncomp) return o->status = HJD_IMG_ERR_TRUNCATED;
+            int td[3] = {0, 0, 0}, ta[3] = {0, 0, 0};
+            for (int k = 0; k < s.ncomp; k++) {
+                const int cs = r.u8();
+                const uint8_t t = r.u8();
+                int c = -1;
+                for (int j = 0; j < o->ncomp; j++) if (cid[j] == cs) c = j;
+                // components of a scan come in frame order (T.81 B.2.3), so each at most once
+                if (c < 0 || (k && c <= s.comp[k - 1]) || (t >> 4) > 3 || (t & 15) > 3) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+                s.comp[k] = c;
+                td[k] = t >> 4;
+                ta[k] = t & 15;
+            }
+            s.ss = r.u8();
+            s.se = r.u8();
+            const uint8_t ahal = r.u8();
+            s.ah = ahal >> 4;
+            s.al = ahal & 15;
+            // T.81 G.1.1.1
+            if (!progressive) {
+                if (s.ss != 0 || s.se != 63 || ahal != 0) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+                for (int k = 0; k < s.ncomp; k++) {
+                    if (seq_done[s.comp[k]]) return o->status = HJD_IMG_ERR_UNSUPPORTED;   // every component exactly once
+                    seq_done[s.comp[k]] = true;
+                }
+                s.kind = HJD_SCAN_SEQ;
+            } else {
+                if (s.al > 13 || s.ah > 13) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+                if (s.ss == 0) {
+                    if (s.se != 0) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+                    s.kind = s.ah ? HJD_SCAN_DC_REFINE : HJD_SCAN_DC_FIRST;
+                } else {
+                    if (s.ncomp != 1 || s.se < s.ss || s.se > 63) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+                    s.kind = s.ah ? HJD_SCAN_AC_REFINE : HJD_SCAN_AC_FIRST;
+                }
+                for (int k = 0; k < s.ncomp; k++)
+                    for (int q = s.ss; q <= s.se; q++) {
+                        const int prev = al_of[s.comp[k]][q];
+                        // a first pass codes a coefficient once; a refinement follows it, one bit at a time
+                        if (s.ah == 0 ? prev != -1 : (prev != s.ah || s.al != s.ah - 1)) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+                    }
+            }
+            s.level = 0;
+            for (int k = 0; k < s.ncomp; k++)
+                for (int q = s.ss; q <= s.se; q++)
+                    if (level_of[s.comp[k]][q] + 1 > s.level) s.level = level_of[s.comp[k]][q] + 1;
+            for (int k = 0; k < s.ncomp; k++)
+                for (int q = s.ss; q <= s.se; q++) { level_of[s.comp[k]][q] = s.level; al_of[s.comp[k]][q] = s.al; }
+            // snapshot of the tables this scan decodes with
+            const bool need_dc = s.kind == HJD_SCAN_SEQ || s.kind == HJD_SCAN_DC_FIRST;
+            const bool need_ac = s.kind == HJD_SCAN_SEQ || s.kind == HJD_SCAN_AC_FIRST || s.kind == HJD_SCAN_AC_REFINE;
+            for (int k = 0; k < s.ncomp; k++) {
+                if (need_dc) { if (!o->dc[td[k]].present) return o->status = HJD_IMG_ERR_BAD_TABLE; s.dc[k] = o->dc[td[k]]; }
+                if (need_ac) { if (!o->ac[ta[k]].present) return o->status = HJD_IMG_ERR_BAD_TABLE; s.ac[k] = o->ac[ta[k]]; }
+            }
+            s.restart_interval = dri;
+            s.off = end;
+            s.first_start = (uint32_t)mp->starts.size();
+            s.len = walk_segment(buf + end, size - end, mp->starts);
+            s.n_starts = (uint32_t)mp->starts.size() - s.first_start;
+            if (s.len > 0xFFFFFF00ull) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+            mp->scans.push_back(s);
+            r.i = end + s.len;
+            continue;
+        }
+        r.i = end;
+    }
+#undef HJD_END_EARLY
+
+frame_checks:
+    if (o->ncomp == 3) {
+        if (chf[1] != 1 || cvf[1] != 1 || chf[2] != 1 || cvf[2] != 1) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+        if (chf[0] < 1 || chf[0] > 2 || cvf[0] < 1 || cvf[0] > 2) return o->status = HJD_IMG_ERR_UNSUPPORTED;
+        o->hf = chf[0];
+        o->vf = cvf[0];
+    } else {
+        o->hf = o->vf = 1;
+    }
+    for (int c = 0; c < o->ncomp; c++)
+        if (!o->qt_present[o->tq[c]]) return o->status = HJD_IMG_ERR_BAD_TABLE;
+    o->restart_interval = mp->scans[0].restart_interval;
+    o->scan_off = mp->scans[0].off;
+    o->scan_len = 0;
+    for (const HjdScanParsed& s : mp->scans) o->scan_len += s.len;
+    return o->status = HJD_IMG_OK;
+}
+
+void hjd_scan_grid(const HjdParsed& f, const HjdScanParsed& s, uint32_t* mx, uint32_t* my)
+{
+    const uint32_t hf = (uint32_t)f.hf, vf = (uint32_t)f.vf;
+    if (s.ncomp > 1 || s.comp[0] != 0) {          // interleaved, or a chroma component (1x1: its grid is the MCU grid)
+        *mx = (f.width + 8 * hf - 1) / (8 * hf);
+        *my = (f.height + 8 * vf - 1) / (8 * vf);
+    } else {                                       // luma alone: its own block grid
+        *mx = (f.width + 7) / 8;
+        *my = (f.height + 7) / 8;
+    }
+}
+
+#define HJD_TAB_DC  0
+#define HJD_TAB_AC  1
+#define HJD_TAB_RAW 2      // progressive AC: raw run, see hjd_build_huff_table_raw
+
+static uint32_t sym_fields(uint32_t len, uint32_t sym, int mode)
 {
     // keep in sync with hjd_sym_fields() in device_common.cuh (ProcessHuffmanBlock's run/size logic)
     const uint32_t size = sym & 15u, run = sym >> 4;
-    if (!is_ac) return HJD_SYM_FIELDS(len, size, 1);
+    if (mode == HJD_TAB_RAW) return HJD_SYM_FIELDS(len, size, run);
+    if (mode == HJD_TAB_DC) return HJD_SYM_FIELDS(len, size, 1);
     if (size) return HJD_SYM_FIELDS(len, size, run + 1);
     return HJD_SYM_FIELDS(len, 0, run == 0 ? 63 : (run == 15 ? 16 : 0));
 }
 
+static bool build_table(const HjdRawHuff& raw, int mode, HjdHuffTable* t);
+
 bool hjd_build_huff_table(const HjdRawHuff& raw, bool is_ac, HjdHuffTable* t)
+{
+    return build_table(raw, is_ac ? HJD_TAB_AC : HJD_TAB_DC, t);
+}
+
+bool hjd_build_huff_table_raw(const HjdRawHuff& raw, HjdHuffTable* t)
+{
+    return build_table(raw, HJD_TAB_RAW, t);
+}
+
+static bool build_table(const HjdRawHuff& raw, int mode, HjdHuffTable* t)
 {
     for (int i = 0; i < HJD_LUT_SIZE; i++) t->lut[i] = (uint16_t)HJD_BAD_ENTRY;
     for (int i = 0; i < HJD_LUT2_SIZE; i++) t->lut2[i] = (uint16_t)HJD_BAD_ENTRY;
@@ -210,7 +424,7 @@ bool hjd_build_huff_table(const HjdRawHuff& raw, bool is_ac, HjdHuffTable* t)
     for (int L = 1; L <= HJD_LUT_BITS; L++) {
         for (int k = 0; k < raw.bits[L - 1]; k++) {
             const uint32_t first = (first_code[L] + (uint32_t)k) << (HJD_LUT_BITS - L);
-            const uint16_t e = (uint16_t)sym_fields((uint32_t)L, raw.vals[valptr + k], is_ac);
+            const uint16_t e = (uint16_t)sym_fields((uint32_t)L, raw.vals[valptr + k], mode);
             for (uint32_t j = 0; j < (1u << (HJD_LUT_BITS - L)); j++) t->lut[first + j] = e;
         }
         valptr += raw.bits[L - 1];
@@ -240,7 +454,7 @@ bool hjd_build_huff_table(const HjdRawHuff& raw, bool is_ac, HjdHuffTable* t)
             const uint32_t nb = nb_of[prefix], off = (uint32_t)(t->lut[prefix] >> 8) << 1;
             const uint32_t rest = code & ((1u << (L - HJD_LUT_BITS)) - 1u);   // the bits after the prefix
             const uint32_t rep = nb - (uint32_t)(L - HJD_LUT_BITS);          // bits that follow the code
-            const uint16_t e = (uint16_t)sym_fields((uint32_t)L, raw.vals[valptr + k], is_ac);
+            const uint16_t e = (uint16_t)sym_fields((uint32_t)L, raw.vals[valptr + k], mode);
             for (uint32_t j = 0; j < (1u << rep); j++) t->lut2[off + (rest << rep) + j] = e;
         }
         valptr += raw.bits[L - 1];

@@ -8,6 +8,7 @@
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
+#include <vector>
 #include "hjd_types.h"
 
 struct HjdRawHuff {
@@ -33,6 +34,35 @@ struct HjdParsed {
 
 // Header parse only (no table building).  Returns HJD_IMG_OK or a negative HJD_IMG_ERR_*.
 int hjd_parse_jpeg(const uint8_t* buf, size_t size, HjdParsed* out);
+
+// ---- multi-scan files (HJD_FLAG_MULTI_SCAN): progressive SOF2 and sequential files with several scans ----
+struct HjdScanParsed {
+    int      ncomp, comp[3];     // frame component indices, scan order
+    int      ss, se, ah, al;
+    int      kind, level;        // HJD_SCAN_* ; dependency level (see hjd_parse_jpeg_multi)
+    uint32_t restart_interval;   // the DRI in effect at this scan (MCUs of this scan)
+    size_t   off, len;           // entropy-coded segment in the file
+    uint32_t first_start, n_starts;   // its RSTn-delimited interval starts (relative to off) in HjdMultiParsed::starts
+    HjdRawHuff dc[3], ac[3];     // snapshot of the DHT contents this scan uses, per scan component (present = 0: unused)
+};
+struct HjdMultiParsed {
+    HjdParsed frame;             // geometry and quantisation tables (Huffman fields unused)
+    std::vector<HjdScanParsed> scans;
+    std::vector<uint32_t> starts;
+};
+
+// Walk a whole file that hjd_parse_jpeg rejects as HJD_IMG_ERR_UNSUPPORTED and record every scan (T.81 G.1.1.1
+// checked; scan headers that break it -> HJD_IMG_ERR_UNSUPPORTED).  A file that ends early keeps the scans it has.
+// Each scan's end and RSTn positions are found by a host walk over its bytes.  Levels: 1 + the highest level of
+// an earlier scan that shares a component and overlaps its band (DC = band {0}); 0 if none.  Scans of one level
+// write disjoint (component, coefficient) positions.  Returns HJD_IMG_OK or a negative HJD_IMG_ERR_*.
+int  hjd_parse_jpeg_multi(const uint8_t* buf, size_t size, HjdMultiParsed* out);
+// Block grid of a scan: the frame's MCU grid when it is interleaved, the component's own block grid otherwise.
+void hjd_scan_grid(const HjdParsed& f, const HjdScanParsed& s, uint32_t* mcus_x, uint32_t* mcus_y);
+
+// Progressive AC tables: the same two-level lookup as hjd_build_huff_table, but each entry carries the raw
+// run: len | size << 5 | run << 9 (EOBn keeps its n); HJD_BAD_ENTRY for no such code.
+bool hjd_build_huff_table_raw(const HjdRawHuff& raw, HjdHuffTable* out);
 
 // Length of the entropy-coded segment that starts at `scan` (avail bytes to the end of the file): up to
 // the first marker that is neither FF00 nor RSTn (EOI normally).  Scans of HJD_SCAN_WALK_MAX bytes or

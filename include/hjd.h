@@ -51,10 +51,10 @@ extern "C" {
 #define HJD_IMG_OK                 0
 #define HJD_IMG_ERR_NOT_JPEG      -1   /* openjpg.cpp:481-486 */
 #define HJD_IMG_ERR_TRUNCATED     -2
-#define HJD_IMG_ERR_UNSUPPORTED   -3   /* progressive, 12-bit, 16-bit DQT, CMYK, chroma sampling != 1x1 ... */
+#define HJD_IMG_ERR_UNSUPPORTED   -3   /* 12-bit, 16-bit DQT, CMYK, chroma sampling != 1x1, progressive / multi-scan unless HJD_FLAG_MULTI_SCAN ... */
 #define HJD_IMG_ERR_BAD_TABLE     -4   /* DHT over-subscribed / missing table */
 #define HJD_IMG_WARN_BAD_CODE      1   /* undecodable Huffman code; rest of that restart interval zero-filled */
-#define HJD_IMG_WARN_COEF_RANGE    2   /* run past coefficient 63 (loadjpg.cpp:780-783) */
+#define HJD_IMG_WARN_COEF_RANGE    2   /* run past coefficient 63 (loadjpg.cpp:780-783); multi-scan: run past Se, refinement size != 1 */
 #define HJD_IMG_WARN_OVERRUN       4   /* entropy data ended before the interval did */
 #define HJD_IMG_WARN_RESTART       8   /* RSTn count differs from ceil(MCUs/Ri)-1 */
 
@@ -70,6 +70,15 @@ extern "C" {
 #define HJD_FLAG_CUDA_CORE_IDCT   64u  /* always the fused kernel with the fast tier as FP32 FMA chains on the CUDA cores (csrc/kernels.cu);
                                           default: chosen per chunk -- tensor cores for large colour images, CUDA cores for batches of small ones (same bytes out) */
 #define HJD_FLAG_NO_SELFSYNC   8u   /* restart-free scans: one thread per scan (kernel 1a) instead of kernel 1b */
+#define HJD_FLAG_MULTI_SCAN  256u   /* also decode progressive (SOF2, 8-bit Huffman) files and sequential files whose components come
+                                       in separate scans (csrc/multiscan.cu; one thread per restart interval of each scan).  Such a
+                                       file decodes exactly like its baseline twin, the single interleaved scan with the same quantised
+                                       coefficients: same coefficients, planes, RGB and BMP bytes.  Blocks no scan codes stay 0; a file
+                                       that ends early is decoded from the scans it has.  hjd_image_info of such an image:
+                                       scan_bytes = the sum over its scans, restart_interval = the DRI of its first scan, n_intervals =
+                                       its work items (restart intervals summed over the scans).  Single-scan baseline files take the
+                                       default path unchanged.  At most HJD_MAX_SCANS_PER_IMAGE scans per file. */
+#define HJD_MAX_SCANS_PER_IMAGE 256
 
 typedef struct hjd_batch hjd_batch;
 
@@ -121,11 +130,26 @@ int  hjd_set_default_device(int device);
 int  hjd_get_image_size(const uint8_t* buf, int size, unsigned* width, unsigned* height);
 /* Header parse only (no GPU): the per-image status a batch would report for this file (HJD_IMG_OK or a
  * negative HJD_IMG_ERR_*) and, when it is decodable, its geometry (offsets in *out stay 0).
- * Not decodable, by design: progressive / lossless / arithmetic (SOF2..SOF15), 12-bit samples (SOF1 with
- * P != 8), 16-bit DQT, 4 components, chroma sampling other than 1x1, luma factors other than 1 or 2, and
- * NON-INTERLEAVED baseline files (one scan per component): the reference's decode loop is one interleaved
- * scan of all three components (loadjpg.cpp:945-997), so such files get HJD_IMG_ERR_UNSUPPORTED. */
+ * Not decodable: lossless / arithmetic (SOF3, SOF5..SOF15), 12-bit samples (SOF1 with P != 8), 16-bit DQT,
+ * 4 components, chroma sampling other than 1x1, luma factors other than 1 or 2; and, unless HJD_FLAG_MULTI_SCAN,
+ * progressive files (SOF2) and NON-INTERLEAVED baseline files (one scan per component): the reference's decode
+ * loop is one interleaved scan of all three components (loadjpg.cpp:945-997), so without the flag such files get
+ * HJD_IMG_ERR_UNSUPPORTED. */
 int  hjd_probe_jpeg(const uint8_t* buf, int64_t size, hjd_image_info* out);
+/* The same for a batch created with `flags` (flags 0: identical to hjd_probe_jpeg).  No GPU. */
+int  hjd_probe_jpeg_flags(const uint8_t* buf, int64_t size, unsigned flags, hjd_image_info* out);
+/* The scans of a file as a batch with HJD_FLAG_MULTI_SCAN decodes them (no GPU): up to `max` into out[], in file
+ * order.  comp[] are frame component indices; level: the scan's dependency level (scans of one level write
+ * disjoint coefficients and are decoded by one launch); restart_interval: the DRI in effect at that scan; bytes:
+ * its entropy-coded segment.  Returns the number of scans (a single-scan baseline file: 1), or the negative
+ * per-image status of a file that is not decodable. */
+typedef struct hjd_scan_info {
+    uint8_t  ncomp, comp[3];
+    uint8_t  ss, se, ah, al;
+    uint8_t  level, pad[3];
+    uint32_t restart_interval, bytes;
+} hjd_scan_info;
+int  hjd_probe_jpeg_scans(const uint8_t* buf, int64_t size, hjd_scan_info* out, int max);
 /* openjpg.cpp:504 WriteBMP24. */
 int  hjd_write_bmp24(const char* path, unsigned width, unsigned height, const uint8_t* rgb);
 /* Same bytes as hjd_write_bmp24 into memory; returns the BMP size (call with out = NULL to size it). */
@@ -175,6 +199,8 @@ int  hjd_batch_set_selfsync_range(hjd_batch* b, int range);
  * cores; 0 = none (nothing decoded yet, or HJD_FLAG_KEEP_PLANES). */
 int  hjd_batch_idct_variant(const hjd_batch* b);
 int  hjd_batch_num_images(const hjd_batch* b);
+/* Scans image i of the last upload is decoded from (1: single-scan baseline; 0: not decodable). */
+int  hjd_batch_num_scans(const hjd_batch* b, int i);
 int  hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* out);
 int  hjd_batch_get_status(hjd_batch* b, int32_t* status /* n */);   /* syncs */
 int  hjd_batch_get_timings(hjd_batch* b, hjd_timings* out);          /* syncs */
