@@ -25,7 +25,8 @@ import numpy as np
 
 __all__ = ["probe", "MultiDecoder", "shard_range_c", "ConvertJpgFile", "ConvertJpgFiles", "DecodeJpgFileData", "JpegGetImageSize", "WriteBMP24", "encode_bmp24",
            "BatchDecoder", "HjdError", "lib", "build", "LIB_PATH",
-           "FLAG_KEEP_PLANES", "FLAG_HOST_SCAN", "FLAG_NO_SELFSYNC", "FLAG_FUSED_MCU", "FLAG_BMP_OUT", "FLAG_TENSOR_CORE_IDCT", "FLAG_CUDA_CORE_IDCT", "FLAG_MULTI_SCAN", "scans", "idct_matrix", "idct_tables"]
+           "FLAG_KEEP_PLANES", "FLAG_HOST_SCAN", "FLAG_NO_SELFSYNC", "FLAG_FUSED_MCU", "FLAG_BMP_OUT", "FLAG_TENSOR_CORE_IDCT", "FLAG_CUDA_CORE_IDCT", "FLAG_MULTI_SCAN", "FLAG_SCALE_1_2",
+           "FLAG_SCALE_1_4", "FLAG_SCALE_1_8", "scans", "idct_matrix", "idct_tables"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HJD_LIB_PATH") or os.path.join(_HERE, "libhjd.so")   # override: tuning builds only
@@ -39,6 +40,9 @@ FLAG_BMP_OUT = 32
 FLAG_TENSOR_CORE_IDCT = 128  # always the fused kernel with the IDCT's fast tier as tcgen05.mma
 FLAG_CUDA_CORE_IDCT = 64     # always the fused kernel with the fast tier as FP32 FMA chains (default: chosen per chunk)
 FLAG_MULTI_SCAN = 256        # also decode progressive and non-interleaved files (each exactly like its baseline twin)
+FLAG_SCALE_1_2 = 1 << 9      # decode to ceil(W/2) x ceil(H/2) in the DCT domain (include/hjd.h; not with KEEP_PLANES,
+FLAG_SCALE_1_4 = 2 << 9      # BMP_OUT, TENSOR_CORE_IDCT or CUDA_CORE_IDCT)
+FLAG_SCALE_1_8 = 3 << 9      # 1/8: a block is its DC alone; with MULTI_SCAN the AC scans are not read
 
 IMG_WARN_BAD_CODE, IMG_WARN_COEF_RANGE, IMG_WARN_OVERRUN, IMG_WARN_RESTART = 1, 2, 4, 8
 
@@ -146,6 +150,7 @@ _SIGS = {
     "hjd_probe_jpeg_flags": (c_int, [c_void_p, c_int64, c_uint, POINTER(ImageInfo)]),
     "hjd_probe_jpeg_scans": (c_int, [c_void_p, c_int64, POINTER(ScanInfo), c_int]),
     "hjd_batch_num_scans": (c_int, [c_void_p, c_int]),
+    "hjd_batch_get_out_size": (c_int, [c_void_p, c_int, POINTER(c_uint32), POINTER(c_uint32)]),
     "hjd_huff_lookup_probe": (c_uint32, [c_void_p, c_void_p, c_int, c_int, c_uint32]),
 }
 
@@ -381,7 +386,8 @@ class BatchDecoder:
 
     @property
     def idct_variant(self) -> int:
-        """bit 0: chunks of the last decode went through the tensor-core fused kernel; bit 1: through the CUDA-core one"""
+        """bit 0: chunks of the last decode went through the tensor-core fused kernel; bit 1: through the CUDA-core one;
+        bit 2: through the scaled kernel (FLAG_SCALE_*)"""
         return lib().hjd_batch_idct_variant(self._h)
 
     @property
@@ -421,9 +427,16 @@ class BatchDecoder:
     def coef_bytes(self) -> int:
         return lib().hjd_batch_coef_bytes(self._h)
 
+    def out_size(self, i: int) -> tuple[int, int]:
+        """(width, height) of image i's decoded output: the source size, or ceil(W/d) x ceil(H/d) with FLAG_SCALE_1_d."""
+        w, h = c_uint32(), c_uint32()
+        _check(lib().hjd_batch_get_out_size(self._h, i, ctypes.byref(w), ctypes.byref(h)), "hjd_batch_get_out_size")
+        return w.value, h.value
+
     def rgb(self, i: int) -> np.ndarray:
-        inf = self.info(i)
-        out = np.zeros((inf.height, inf.width, 3), dtype=np.uint8)
+        """RGB of image i: uint8 [out_h, out_w, 3] (out_size)."""
+        w, h = self.out_size(i)
+        out = np.zeros((h, w, 3), dtype=np.uint8)
         _check(lib().hjd_batch_download_image(self._h, i, out.ctypes.data), "hjd_batch_download_image")
         return out
 

@@ -9,6 +9,7 @@
 #include "kernels.cuh"
 #include "selfsync.cuh"
 #include "multiscan.cuh"
+#include "scaled.cuh"
 
 #include <cuda_runtime.h>
 #include <math.h>
@@ -156,6 +157,7 @@ struct hjd_batch {
     std::vector<std::vector<uint8_t>> ms_tab_raw;
     std::vector<uint32_t> ms_items, n_scans;    // per image: work items (multi-scan images), scans (0: not decodable)
     std::vector<uint32_t> ms_w0;                // per image: its first work item (n + 1 entries)
+    std::vector<uint8_t> ms_image;              // per image: decoded by the multi-scan kernel (its blocks are zeroed first)
     std::unordered_multimap<uint64_t, uint32_t> tset_of, qset_of;   // content hash -> candidate sets (verified byte for byte)
     std::vector<HjdRawTables> tset_raw, qset_raw;                    // what each set was built from
     uint64_t total_blocks = 0, rgb_bytes = 0, plane_bytes = 0, scan_bytes = 0, pixels = 0, arena_bytes = 0;
@@ -166,6 +168,7 @@ struct hjd_batch {
     int launches = 0;
     int sm_count = 148;                         // multiprocessors of this device (work-list balancing)
     int tc_chunks = 0, cc_chunks = 0;           // chunks of the last decode whose MCUs went through the tensor-core / CUDA-core fused kernel
+    int sc_chunks = 0;                          // ... through the scaled kernel (HJD_FLAG_SCALE_*)
 
     DevBuf d_arena, d_imgs, d_tsets, d_qsets, d_work, d_segs, d_mcucta, d_slices, d_slicecnt, d_istart, d_coef, d_planes, d_rgb, d_status;
     DevBuf d_scans, d_mswork, d_msstarts, d_mstabs;
@@ -173,13 +176,31 @@ struct hjd_batch {
     PinBuf h_meta, h_out;                       // h_out: staging of the single-image calls
 };
 
-// Bytes of one image's region in the output slab: tightly packed RGB24, or (HJD_FLAG_BMP_OUT) the BMP file
-// WriteBMP24 would write, placed so that its pixel array starts 64 bytes into the region (the 54-byte
-// header at +10): rows padded to a multiple of 4 bytes, openjpg.cpp:534-535.
+// log2 of the scale denominator of HJD_FLAG_SCALE_* (0: full size), and the output size of a W x H image under it:
+// ceil(W / d) x ceil(H / d), libjpeg's jdiv_round_up.
+static int scale_shift(unsigned flags) { return (int)((flags & HJD_FLAG_SCALE_MASK) >> 9); }
+static uint32_t scaled_dim(unsigned flags, uint32_t v)
+{
+    const int s = scale_shift(flags);
+    return (uint32_t)(((uint64_t)v + (1u << s) - 1) >> s);
+}
+
+// Bytes of one image's region in the output slab: tightly packed RGB24 (of the scaled size with HJD_FLAG_SCALE_*), or
+// (HJD_FLAG_BMP_OUT) the BMP file WriteBMP24 would write, placed so that its pixel array starts 64 bytes into the
+// region (the 54-byte header at +10): rows padded to a multiple of 4 bytes, openjpg.cpp:534-535.
 static uint64_t image_out_bytes(unsigned flags, uint32_t w, uint32_t h)
 {
     if (flags & HJD_FLAG_BMP_OUT) return 64 + (uint64_t)((w * 3 + 3) & ~3u) * h;
-    return (uint64_t)w * h * 3;
+    return (uint64_t)scaled_dim(flags, w) * scaled_dim(flags, h) * 3;
+}
+
+// The reduced IDCT's cosine table for N samples per block side: the expression of compute_idct_constants with 16
+// replaced by 2N (host libm).
+static void compute_scaled_cos(int n, float* cos_n)
+{
+    const float PI = 3.14f;
+    for (int p = 0; p < n; p++)
+        for (int k = 0; k < n; k++) cos_n[p * n + k] = cosf(((2 * p + 1) * k * PI) / (float)(2 * n));
 }
 
 static void compute_idct_constants(float cos_tab[64], float* cc0, float* cc00)
@@ -224,6 +245,12 @@ extern "C" hjd_batch* hjd_batch_create(int device, unsigned flags)
     if (n <= 0) { fail(HJD_ERR_CUDA, "hjd_batch_create", "no CUDA device available (this library has no CPU fallback)"); return nullptr; }
     if (device < 0 || device >= n) { fail(HJD_ERR_ARG, "hjd_batch_create", "bad device index"); return nullptr; }
     if ((flags & HJD_FLAG_BMP_OUT) && (flags & HJD_FLAG_KEEP_PLANES)) { fail(HJD_ERR_ARG, "hjd_batch_create", "HJD_FLAG_BMP_OUT is an epilogue of the default (fused) kernels"); return nullptr; }
+    if ((flags & HJD_FLAG_SCALE_MASK) &&
+        (flags & (HJD_FLAG_KEEP_PLANES | HJD_FLAG_BMP_OUT | HJD_FLAG_TENSOR_CORE_IDCT | HJD_FLAG_CUDA_CORE_IDCT))) {
+        fail(HJD_ERR_ARG, "hjd_batch_create", "HJD_FLAG_SCALE_* has no planes, no BMP output and its own kernel: it combines with "
+                                              "none of HJD_FLAG_KEEP_PLANES, HJD_FLAG_BMP_OUT, HJD_FLAG_TENSOR_CORE_IDCT, HJD_FLAG_CUDA_CORE_IDCT");
+        return nullptr;
+    }
     if (cudaSetDevice(device) != cudaSuccess) { fail(HJD_ERR_CUDA, "cudaSetDevice"); return nullptr; }
     hjd_batch* b = new hjd_batch();
     b->device = device;
@@ -242,6 +269,16 @@ extern "C" hjd_batch* hjd_batch_create(int device, unsigned flags)
         float cos_tab[64], c0, c00;
         compute_idct_constants(cos_tab, &c0, &c00);
         e = hjd_set_idct_constants(cos_tab, c0, c00);
+        if (e == cudaSuccess) {
+            float cos4[16], cos2[4], cos1[1], cc[64], cc16[16];
+            compute_scaled_cos(4, cos4);
+            compute_scaled_cos(2, cos2);
+            compute_scaled_cos(1, cos1);
+            hjd_get_idct_tables(cos_tab, cc);
+            for (int u = 0; u < 4; u++)
+                for (int v = 0; v < 4; v++) cc16[u * 4 + v] = cc[u * 8 + v];
+            e = hjd_set_scaled_constants(cos4, cos2, cos1, cc16);
+        }
     }
     if (e != cudaSuccess) {
         fail(HJD_ERR_CUDA, "hjd_batch_create", cudaGetErrorString(e));
@@ -309,8 +346,12 @@ static int ms_table(hjd_batch* b, const HjdRawHuff& raw, int mode)
 static int ms_add_image(hjd_batch* b, int i, const HjdMultiParsed& mp, uint64_t dev_off)
 {
     const size_t scan0 = b->scans.size(), start0 = b->ms_starts.size(), work0 = b->mswork.size();
-    uint32_t items = 0;
+    uint32_t items = 0, n_scans = 0;
+    // At 1/8 a block is its DC coefficient alone: the AC scans (Ss > 0) are not read.
+    const bool dc_only = scale_shift(b->flags) == 3;
     for (const HjdScanParsed& p : mp.scans) {
+        if (dc_only && p.ss > 0) continue;
+        n_scans++;
         HjdScanDesc sd;
         memset(&sd, 0, sizeof sd);
         sd.image = (uint32_t)i;
@@ -345,7 +386,7 @@ static int ms_add_image(hjd_batch* b, int i, const HjdMultiParsed& mp, uint64_t 
         b->scans.push_back(sd);
     }
     b->ms_items[i] = items;
-    b->n_scans[i] = (uint32_t)mp.scans.size();
+    b->n_scans[i] = n_scans;
     return HJD_OK;
 }
 
@@ -365,7 +406,7 @@ static int upload_common(hjd_batch* b, bool chunked)
     b->host_restart_warn.assign(n, 0);
     b->ss.clear(); b->sswork.clear(); b->sssegs.clear();
     b->scans.clear(); b->mswork.clear(); b->ms_starts.clear(); b->ms_tabs.clear(); b->ms_tab_of.clear(); b->ms_tab_raw.clear();
-    b->ms_items.assign(n, 0); b->n_scans.assign(n, 0); b->ms_w0.assign((size_t)n + 1, 0);
+    b->ms_items.assign(n, 0); b->n_scans.assign(n, 0); b->ms_w0.assign((size_t)n + 1, 0); b->ms_image.assign(n, 0);
     b->ss_subs = b->ss_chunks = 0;
     b->ss_dst_bytes = 0;
     b->total_blocks = b->rgb_bytes = b->plane_bytes = b->scan_bytes = b->pixels = 0;
@@ -466,6 +507,7 @@ static int upload_common(hjd_batch* b, bool chunked)
         const HjdMultiParsed* mp = multi[(size_t)i].get();
         if (st == HJD_IMG_OK && mp) {
             st = ms_add_image(b, i, *mp, files[i].dev_off);
+            b->ms_image[i] = 1;
             full = mp->frame;
             hjd_raw_tables(full, &full_raw);
             have_full = true;
@@ -694,7 +736,7 @@ static int upload_common(hjd_batch* b, bool chunked)
                 k = e;
             }
             for (int i = c.img0; i < c.img1; i++) {
-                if (b->ms_w0[(size_t)i + 1] == b->ms_w0[(size_t)i] || b->parse_status[i] != HJD_IMG_OK) continue;
+                if (!b->ms_image[i] || b->parse_status[i] != HJD_IMG_OK) continue;
                 const HjdImageDesc& d = b->imgs[i];
                 if (!c.ms_zero.empty() && c.ms_zero.back().first + c.ms_zero.back().second == d.block_base)
                     c.ms_zero.back().second += d.n_blocks;
@@ -1052,7 +1094,17 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
         b->launches += 1;
     }
     if (ev) CU(cudaEventRecord(ev[2], st));
-    if (!(b->flags & HJD_FLAG_KEEP_PLANES)) {
+    if (scale_shift(b->flags)) {
+        // reduced-size decode: its own kernel in place of the fused one, counted in the same stage
+        if (c.blocks) {
+            b->sc_chunks++;
+            CU(hjd_launch_mcu_rgb_scaled((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
+                                         (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_mcucta.p + c.img0, n,
+                                         b->mcu_cta[c.img1] - b->mcu_cta[c.img0], c.max_mcus, scale_shift(b->flags), st));
+            b->launches += 1;
+        }
+        if (ev) CU(cudaEventRecord(ev[3], st));
+    } else if (!(b->flags & HJD_FLAG_KEEP_PLANES)) {
         // default: kernels 2+3 fused per MCU, planes never reach HBM
         if (c.blocks) {
             const uint32_t n_mcus_chunk = b->mcu_cta[c.img1] - b->mcu_cta[c.img0];
@@ -1085,7 +1137,7 @@ static int run_chunks(hjd_batch* b, bool h2d, uint8_t* rgb_host)
 {
     cudaStream_t main = b->stream;
     b->launches = 0;
-    b->tc_chunks = b->cc_chunks = 0;
+    b->tc_chunks = b->cc_chunks = b->sc_chunks = 0;
     b->ss_ran = false;
     if (b->any_parse_error && b->rgb_bytes) CU(cudaMemsetAsync(b->d_rgb.p, 0, b->rgb_bytes, main));
     CU(cudaEventRecord(b->ev[0], main));
@@ -1157,7 +1209,7 @@ extern "C" int hjd_batch_num_images(const hjd_batch* b) { return b ? (int)b->img
 extern "C" int hjd_batch_idct_variant(const hjd_batch* b)
 {
     if (!b || (b->flags & HJD_FLAG_KEEP_PLANES)) return 0;
-    return (b->tc_chunks ? 1 : 0) | (b->cc_chunks ? 2 : 0);
+    return (b->tc_chunks ? 1 : 0) | (b->cc_chunks ? 2 : 0) | (b->sc_chunks ? 4 : 0);
 }
 extern "C" int hjd_batch_selfsync_rounds(hjd_batch* b)
 {
@@ -1184,6 +1236,15 @@ extern "C" int hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* o)
     o->y_offset = d.y_off; o->cb_offset = d.cb_off; o->cr_offset = d.cr_off;
     o->y_pitch = d.y_pitch; o->c_pitch = d.c_pitch; o->status = b->parse_status[i];
     if (b->ms_items[i]) o->n_intervals = b->ms_items[i];
+    return HJD_OK;
+}
+
+extern "C" int hjd_batch_get_out_size(const hjd_batch* b, int i, uint32_t* w, uint32_t* h)
+{
+    if (!b || i < 0 || i >= (int)b->imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_get_out_size", "bad arguments");
+    const HjdImageDesc& d = b->imgs[i];
+    if (w) *w = scaled_dim(b->flags, d.width);
+    if (h) *h = scaled_dim(b->flags, d.height);
     return HJD_OK;
 }
 
@@ -1277,7 +1338,7 @@ extern "C" int hjd_batch_download_image(hjd_batch* b, int i, uint8_t* dst)
     if (!b || i < 0 || i >= (int)b->imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_download_image", "bad arguments");
     if (b->flags & HJD_FLAG_BMP_OUT) return fail(HJD_ERR_STATE, "hjd_batch_download_image", "this batch writes BMP files (HJD_FLAG_BMP_OUT): use hjd_batch_download_bmp");
     const HjdImageDesc& d = b->imgs[i];
-    return download(b, dst, (const uint8_t*)b->d_rgb.p + d.rgb_off, (uint64_t)d.width * d.height * 3,
+    return download(b, dst, (const uint8_t*)b->d_rgb.p + d.rgb_off, image_out_bytes(b->flags, d.width, d.height),
                     "hjd_batch_download_image");
 }
 
@@ -1547,6 +1608,7 @@ extern "C" int hjd_probe_jpeg_flags(const uint8_t* buf, int64_t size, unsigned f
         if (f.status == HJD_IMG_OK) {
             out->n_intervals = 0;
             for (const HjdScanParsed& s : mp->scans) {
+                if (scale_shift(flags) == 3 && s.ss > 0) continue;      // not read at 1/8 (see ms_add_image)
                 uint32_t mx, my;
                 hjd_scan_grid(f, s, &mx, &my);
                 const uint64_t want = s.restart_interval ? ((uint64_t)mx * my + s.restart_interval - 1) / s.restart_interval : 1;

@@ -79,6 +79,24 @@ extern "C" {
                                        its work items (restart intervals summed over the scans).  Single-scan baseline files take the
                                        default path unchanged.  At most HJD_MAX_SCANS_PER_IMAGE scans per file. */
 #define HJD_MAX_SCANS_PER_IMAGE 256
+/* Reduced-size decode in the DCT domain (a 2-bit field; 0 = full size).  With d = 2, 4 or 8 and N = 8/d samples per
+ * block side, a W x H image decodes to ceil(W/d) x ceil(H/d) RGB24 in the usual layout (top-down, stride 3 * out_w,
+ * R first, each image 256-byte aligned in the slab; hjd_batch_get_out_size).  Each block is de-quantised as the full
+ * decode does it (Cb with Cr's table) and its top-left N x N natural-order coefficients go through the reference's
+ * direct-form IDCT with N in place of 8: float sum over u < N (outer), v < N (inner) of
+ * cc[u][v] * arr[u][v] * cosN[x][u] * cosN[y][v], cosN[p][k] = cosf(((2p+1) * k * 3.14f) / (2N)), then (int16) of
+ * (int) of 0.25 * sum, + 128, clamp.  Per MCU the luma tile is (N hf) x (N vf) and the chroma tile N x N, upsampled by
+ * the reference's replication rule with 8 replaced by N; the colour conversion is the reference's.  N = 8 would be the
+ * full decode.  Every Huffman symbol of a sequential scan is still decoded (csrc/scaled.cu).
+ * With HJD_FLAG_MULTI_SCAN, scans are decoded as without a scale flag, except at 1/8, where an image's AC scans
+ * (Ss > 0) are not read at all: its coefficient slab holds only what its DC scans code, hjd_batch_num_scans and
+ * n_intervals count its DC scans only, and damage inside an AC scan is not reported.
+ * Not combinable (hjd_batch_create fails with HJD_ERR_ARG): HJD_FLAG_KEEP_PLANES (no scaled planes exist),
+ * HJD_FLAG_BMP_OUT, HJD_FLAG_TENSOR_CORE_IDCT and HJD_FLAG_CUDA_CORE_IDCT (they select full-size kernels). */
+#define HJD_FLAG_SCALE_1_2   (1u << 9)
+#define HJD_FLAG_SCALE_1_4   (2u << 9)
+#define HJD_FLAG_SCALE_1_8   (3u << 9)
+#define HJD_FLAG_SCALE_MASK  (3u << 9)
 
 typedef struct hjd_batch hjd_batch;
 
@@ -196,12 +214,17 @@ int  hjd_batch_selfsync_rounds(hjd_batch* b);                        /* syncs */
  * to 256 (testing / tuning; results do not depend on it).  Takes effect at the next upload. */
 int  hjd_batch_set_selfsync_range(hjd_batch* b, int range);
 /* Which fused kernel(s) the chunks of the last decode went through: bit 0 = tensor cores (csrc/mcu_tc.cuh), bit 1 = CUDA
- * cores; 0 = none (nothing decoded yet, or HJD_FLAG_KEEP_PLANES). */
+ * cores, bit 2 = the scaled kernel (HJD_FLAG_SCALE_*, csrc/scaled.cu); 0 = none (nothing decoded yet, or
+ * HJD_FLAG_KEEP_PLANES). */
 int  hjd_batch_idct_variant(const hjd_batch* b);
 int  hjd_batch_num_images(const hjd_batch* b);
-/* Scans image i of the last upload is decoded from (1: single-scan baseline; 0: not decodable). */
+/* Scans image i of the last upload is decoded from (1: single-scan baseline; 0: not decodable).  HJD_FLAG_SCALE_1_8
+ * with HJD_FLAG_MULTI_SCAN: its DC scans only. */
 int  hjd_batch_num_scans(const hjd_batch* b, int i);
+/* hjd_image_info describes the source image (width, height: its frame). */
 int  hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* out);
+/* Dimensions of image i's decoded output: width x height, or ceil(width/d) x ceil(height/d) with HJD_FLAG_SCALE_1_d. */
+int  hjd_batch_get_out_size(const hjd_batch* b, int i, uint32_t* w, uint32_t* h);
 int  hjd_batch_get_status(hjd_batch* b, int32_t* status /* n */);   /* syncs */
 int  hjd_batch_get_timings(hjd_batch* b, hjd_timings* out);          /* syncs */
 /* CUDA-event stopwatch on the batch stream: record event `slot` (0..HJD_MARK_SLOTS-1); milliseconds
@@ -214,7 +237,7 @@ uint64_t hjd_batch_rgb_bytes(const hjd_batch* b);     /* size of the RGB slab */
 uint64_t hjd_batch_coef_bytes(const hjd_batch* b);
 uint64_t hjd_batch_plane_bytes(const hjd_batch* b);
 uint64_t hjd_batch_scan_bytes(const hjd_batch* b);    /* sum of entropy-coded bytes */
-uint64_t hjd_batch_pixels(const hjd_batch* b);        /* sum of width*height */
+uint64_t hjd_batch_pixels(const hjd_batch* b);        /* sum of width*height (source pixels, also when scaled) */
 
 /* Device pointers of the result slabs (valid until the next upload / destroy). */
 void* hjd_batch_device_rgb(hjd_batch* b);
@@ -223,7 +246,7 @@ void* hjd_batch_device_planes(hjd_batch* b);
 
 /* Device -> host copies (synchronous with respect to the batch stream). */
 int  hjd_batch_download_rgb(hjd_batch* b, uint8_t* dst /* hjd_batch_rgb_bytes */);
-int  hjd_batch_download_image(hjd_batch* b, int i, uint8_t* dst /* w*h*3 */);
+int  hjd_batch_download_image(hjd_batch* b, int i, uint8_t* dst /* out_w*out_h*3, hjd_batch_get_out_size */);
 int  hjd_batch_download_coef(hjd_batch* b, int16_t* dst /* hjd_batch_coef_bytes */);
 uint64_t hjd_batch_bmp_bytes(const hjd_batch* b, int i);            /* HJD_FLAG_BMP_OUT: size of image i's BMP file (0: none) */
 int  hjd_batch_download_bmp(hjd_batch* b, int i, uint8_t* dst /* hjd_batch_bmp_bytes(i) */);
@@ -237,7 +260,7 @@ int  hjd_batch_decode_host(hjd_batch* b, const uint8_t* arena, const int64_t* of
                            int n, uint8_t* rgb_out, uint64_t rgb_capacity, uint64_t* rgb_offsets_out,
                            int32_t* status_out, int chunk_images);
 /* Bytes hjd_batch_decode_host needs in rgb_out for these files (header parse only); hjd_out_slab_bytes: the
- * same for a batch created with `flags` (HJD_FLAG_BMP_OUT changes the layout). */
+ * same for a batch created with `flags` (HJD_FLAG_BMP_OUT changes the layout, HJD_FLAG_SCALE_* the output size). */
 uint64_t hjd_rgb_slab_bytes(const uint8_t* arena, const int64_t* offsets, const int64_t* sizes, int n);
 uint64_t hjd_out_slab_bytes(const uint8_t* arena, const int64_t* offsets, const int64_t* sizes, int n, unsigned flags);
 
