@@ -340,6 +340,18 @@ static int ms_table(hjd_batch* b, const HjdRawHuff& raw, int mode)
     return (int)b->ms_tabs.size() - 1;
 }
 
+// Work items of one scan: the restart intervals its DRI implies (want_all) or, by default, no more than the file holds.
+static uint32_t ms_scan_items(const HjdParsed& frame, const HjdScanParsed& p, uint32_t* mcus_x, uint32_t* mcus_y,
+                              bool want_all = false)
+{
+    uint32_t mx, my;
+    hjd_scan_grid(frame, p, &mx, &my);
+    if (mcus_x) { *mcus_x = mx; *mcus_y = my; }
+    const uint64_t total = (uint64_t)mx * my;
+    const uint64_t want = p.restart_interval ? (total + p.restart_interval - 1) / p.restart_interval : 1;
+    return (uint32_t)(want_all || want < p.n_starts ? want : p.n_starts);
+}
+
 // Scan descriptors, tables, interval starts and work items of multi-scan image i (file at arena offset dev_off).
 // A scan with fewer RSTn markers than its DRI implies (a file cut inside it) gets the intervals it has: the last one
 // runs to the end of the data, and the image is flagged HJD_IMG_WARN_RESTART.  HJD_IMG_OK or HJD_IMG_ERR_BAD_TABLE.
@@ -360,11 +372,8 @@ static int ms_add_image(hjd_batch* b, int i, const HjdMultiParsed& mp, uint64_t 
         sd.ss = (uint8_t)p.ss; sd.se = (uint8_t)p.se; sd.ah = (uint8_t)p.ah; sd.al = (uint8_t)p.al;
         sd.kind = (uint8_t)p.kind; sd.level = (uint8_t)(p.level < 255 ? p.level : 255);
         sd.restart_interval = p.restart_interval;
-        hjd_scan_grid(mp.frame, p, &sd.mcus_x, &sd.mcus_y);
-        const uint64_t total = (uint64_t)sd.mcus_x * sd.mcus_y;
-        const uint64_t want = p.restart_interval ? (total + p.restart_interval - 1) / p.restart_interval : 1;
-        sd.n_intervals = (uint32_t)(want < p.n_starts ? want : p.n_starts);
-        if (p.restart_interval && p.n_starts != want) b->host_restart_warn[i] = 1;
+        sd.n_intervals = ms_scan_items(mp.frame, p, &sd.mcus_x, &sd.mcus_y);
+        if (p.restart_interval && p.n_starts != ms_scan_items(mp.frame, p, nullptr, nullptr, true)) b->host_restart_warn[i] = 1;
         sd.start_base = (uint32_t)b->ms_starts.size();
         sd.scan_len = (uint32_t)p.len;
         sd.scan_off = dev_off + p.off;
@@ -430,6 +439,7 @@ static int upload_common(hjd_batch* b, bool chunked)
         int ncomp, hf, vf;
         size_t scan_off, scan_len;
         uint64_t tk, qk;
+        uint64_t ms_items;         // multi-scan work items (what ms_add_image will add)
         int trep, qrep;            // image whose tables / quantisation tables these are byte-identical to (itself: a representative)
     };
     std::vector<Lite> lite((size_t)n);
@@ -453,6 +463,8 @@ static int upload_common(hjd_batch* b, bool chunked)
                 if (st == HJD_IMG_OK && mp->frame.scan_len > 0xFFFFFF00ull) st = HJD_IMG_ERR_UNSUPPORTED;
                 if (st == HJD_IMG_OK) {
                     p = mp->frame;
+                    for (const HjdScanParsed& sp : mp->scans)
+                        if (!(scale_shift(b->flags) == 3 && sp.ss > 0)) l.ms_items += ms_scan_items(mp->frame, sp, nullptr, nullptr);
                     multi[(size_t)i] = std::move(mp);
                 }
             }
@@ -488,6 +500,14 @@ static int upload_common(hjd_batch* b, bool chunked)
             }
             for (auto& th : pool) th.join();
         }
+    }
+
+    // Index limits a batch must stay inside (DESIGN §3), refused before anything is allocated or copied.  Multi-scan
+    // work items are numbered in int (hjd_k_multiscan's thread index), so a batch holds fewer than 2^31.
+    {
+        uint64_t items = 0;
+        for (const Lite& l : lite) items += l.ms_items;
+        if (items >= 0x80000000ull) return fail(HJD_ERR_ARG, "hjd_batch_upload", "batch exceeds 2^31 multi-scan work items");
     }
 
     HjdParsed full;                    // re-parse target for the representatives
@@ -609,6 +629,14 @@ static int upload_common(hjd_batch* b, bool chunked)
         }
     }
     if (b->total_blocks >= 0xFFFFFFFFull) return fail(HJD_ERR_ARG, "hjd_batch_upload", "batch exceeds 2^32 blocks");
+    {
+        // kernel 1b numbers the 16-byte chunks of the restart-free scans in uint32, with one gap per chunk of the plan and
+        // a sentinel: about 64 GiB of restart-free scan data
+        uint64_t ck = 0;
+        for (const HjdSsImage& si : b->ss) ck += si.n_chunks;
+        if (ck + (uint64_t)n + 2 > 0xFFFFFFFFull)
+            return fail(HJD_ERR_ARG, "hjd_batch_upload", "restart-free scans of the batch exceed 2^32 16-byte chunks (64 GiB)");
+    }
 
     // chunk plan: contiguous image ranges of roughly equal block counts
     {

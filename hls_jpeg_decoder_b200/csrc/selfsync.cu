@@ -858,7 +858,7 @@ hjd_k_ss_write(const HjdImageDesc* __restrict__ imgs, const HjdTableSet* __restr
                     const uint32_t src = warp_slots + ent.y * 128u + ((chunk ^ (ent.y & 7u)) << 4);
                     const uint4 w = hjd_lds_v4_sync(src);
                     hjd_sts_zero16_sync(src);
-                    ((uint4*)coef)[(size_t)(ent.x * 8u + chunk)] = w;
+                    ((uint4*)coef)[(size_t)ent.x * 8u + chunk] = w;      // 64-bit: ent.x * 8 wraps from block 2^29 on
                 }
             }
             __syncwarp();

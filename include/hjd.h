@@ -190,7 +190,10 @@ void       hjd_batch_destroy(hjd_batch* b);
 int  hjd_batch_set_stream(hjd_batch* b, void* cuda_stream);
 
 /* Parse headers, build Huffman/quant tables and descriptors, copy the files to HBM.
- * bufs[i]/sizes[i]: whole .jpg files in host memory (pinned memory makes the copy asynchronous). */
+ * bufs[i]/sizes[i]: whole .jpg files in host memory (pinned memory makes the copy asynchronous).
+ * Limits per batch (HJD_ERR_ARG, naming the limit, before anything is allocated or copied): fewer than 2^32 blocks;
+ * restart-free scans fitting in fewer than 2^32 16-byte chunks (about 64 GiB); with HJD_FLAG_MULTI_SCAN, fewer than
+ * 2^31 multi-scan work items (restart intervals of all scans).  DESIGN.md §3 "Index limits". */
 int  hjd_batch_upload(hjd_batch* b, const uint8_t* const* bufs, const int64_t* sizes, int n);
 /* Same, for files packed in one host arena: file i = arena[offsets[i] .. offsets[i]+sizes[i]).
  * One host->device copy of [offsets[0], offsets[n-1]+sizes[n-1]). */
