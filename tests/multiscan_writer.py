@@ -3,8 +3,12 @@ component) and progressive files (SOF2) from an explicit scan script.  The input
 ``oracle.port.decode(baseline, entropy_only=True)`` returns for a baseline template file, so every file written
 here carries exactly the template's quantised coefficients: the template is its baseline twin.
 
-Every scan gets its own Huffman tables (a flat code over the symbols it uses: up to 128 eight-bit codes, then
-nine-bit codes, never the all-ones code), written in a DHT just before its SOS; a DRI can change between scans.
+Every scan gets its own Huffman tables over the symbols it uses, written in a DHT just before its SOS; a DRI can
+change between scans.  The code of a scan is one of (never the all-ones code):
+  "flat"   up to 128 eight-bit codes, then nine-bit codes
+  "long"   every code 11 to 16 bits long, so that every lookup goes through a decoder's second-level table
+  "mixed"  random lengths 1 to 16, with one code of each length 11 to 16 whenever there are six or more symbols
+Optional 0xFF fill bytes (T.81 B.1.1.2) go before every RSTn and before the marker that follows each scan.
 
 TEST INFRASTRUCTURE ONLY.
 """
@@ -33,6 +37,39 @@ def flat_table(symbols) -> tuple[list, list]:
     bits[7] = min(len(vals), 128)
     bits[8] = len(vals) - bits[7]
     return bits, vals
+
+
+def long_table(symbols, rng) -> tuple[list, list]:
+    """(bits[16], vals): every symbol a code of 11 to 16 bits (at most 256 symbols: the Kraft sum stays below 1/8)."""
+    vals = sorted(set(symbols)) or [0]
+    return _table_of_lengths(vals, [int(x) for x in rng.integers(11, 17, len(vals))], rng)
+
+
+def mixed_table(symbols, rng) -> tuple[list, list]:
+    """(bits[16], vals): random code lengths 1..16 whose Kraft sum stays below 1 (so the all-ones code is never
+    assigned), one symbol at each length 11..16 when there are six or more symbols."""
+    vals = sorted(set(symbols)) or [0]
+    rng.shuffle(vals)
+    lengths = list(range(11, 17)) if len(vals) >= 6 else []
+    budget = (1 << 16) - 1 - sum(1 << (16 - L) for L in lengths)        # in units of 2^-16, one code kept free
+    for k in range(len(lengths), len(vals)):
+        spare = budget - (len(vals) - k - 1)                             # the rest need at least 16-bit codes
+        fits = [L for L in range(1, 17) if (1 << (16 - L)) <= spare]
+        L = fits[int(rng.integers(len(fits)))]
+        lengths.append(L)
+        budget -= 1 << (16 - L)
+    return _table_of_lengths(vals, lengths, rng)
+
+
+def _table_of_lengths(vals, lengths, rng):
+    order = sorted(range(len(vals)), key=lambda k: (lengths[k], rng.random()))
+    bits = [0] * 16
+    for L in lengths:
+        bits[L - 1] += 1
+    return bits, [vals[k] for k in order]
+
+
+TABLES = {"flat": lambda symbols, rng: flat_table(symbols), "long": long_table, "mixed": mixed_table}
 
 
 def _codes(bits, vals):
@@ -93,9 +130,9 @@ class _Scan:
         if n:
             self.ops.append(("bits", v, n))
 
-    def emit(self):
-        dc = flat_table([o[1] for o in self.ops if o[0] == "dc"])
-        ac = flat_table([o[1] for o in self.ops if o[0] == "ac"])
+    def emit(self, table="flat", rng=None, fill=0):
+        dc = TABLES[table]([o[1] for o in self.ops if o[0] == "dc"], rng)
+        ac = TABLES[table]([o[1] for o in self.ops if o[0] == "ac"], rng)
         cd, ca = _codes(*dc), _codes(*ac)
         out, bw, rst = bytearray(), BitWriter(), 0
         for o in self.ops:
@@ -107,13 +144,13 @@ class _Scan:
                 bw.put(o[1], o[2])
             else:
                 bw.flush()
-                out += bw.out + bytes([0xFF, 0xD0 + (rst & 7)])
+                out += bw.out + b"\xff" * fill + bytes([0xFF, 0xD0 + (rst & 7)])
                 bw, rst = BitWriter(), rst + 1
         bw.flush()
-        return bytes(out + bw.out), dc, ac
+        return bytes(out + bw.out + b"\xff" * fill), dc, ac
 
 
-def _encode_scan(coef, geo: _Geom, comps, ss, se, ah, al, restart):
+def _encode_scan(coef, geo: _Geom, comps, ss, se, ah, al, restart, table="flat", rng=None, fill=0):
     sc = _Scan()
     c64 = np.asarray(coef, dtype=np.int64)
     pred = {c: 0 for c in comps}
@@ -161,6 +198,11 @@ def _encode_scan(coef, geo: _Geom, comps, ss, se, ah, al, restart):
             elif ss == 0:                                       # DC refine
                 sc.bits((int(blk[0]) >> al) & 1, 1)
             elif ah == 0:                                       # AC first
+                if not (np.abs(blk[ss:se + 1]) >> al).any():    # an empty band: only the EOB run grows
+                    st["eobrun"] += 1
+                    if st["eobrun"] == 0x7FFF:
+                        flush_eob()
+                    continue
                 r = 0
                 for k in range(ss, se + 1):
                     v = int(blk[k])
@@ -179,6 +221,11 @@ def _encode_scan(coef, geo: _Geom, comps, ss, se, ah, al, restart):
                     if st["eobrun"] == 0x7FFF:
                         flush_eob()
             else:                                               # AC refine (T.81 G.1.2.3, as libjpeg's encoder)
+                if not (np.abs(blk[ss:se + 1]) >> al).any():    # an empty band: only the EOB run grows
+                    st["eobrun"] += 1
+                    if st["eobrun"] == 0x7FFF:
+                        flush_eob()
+                    continue
                 absv = [abs(int(blk[k])) >> al for k in range(64)]
                 eob = max([k for k in range(ss, se + 1) if absv[k] == 1], default=0)
                 r, br = 0, []
@@ -207,15 +254,17 @@ def _encode_scan(coef, geo: _Geom, comps, ss, se, ah, al, restart):
                     if st["eobrun"] == 0x7FFF or len(st["be"]) > 937:
                         flush_eob()
     flush_eob()
-    return sc.emit()
+    return sc.emit(table, rng, fill)
 
 
 def write_multiscan(template: bytes, coef: np.ndarray, geometry: dict, script, progressive: bool = True,
-                    restarts=None, truncate_after: int | None = None) -> bytes:
+                    restarts=None, truncate_after: int | None = None, tables="flat", fill: int = 0,
+                    seed: int = 0) -> bytes:
     """A multi-scan file with the coefficients `coef` ([blocks, 64] zig-zag, absolute DC, MCU order, as
     port.decode(template, entropy_only=True)["coef"]).  script: [(components, Ss, Se, Ah, Al)], frame component
     indices; restarts: per scan the DRI in that scan's MCUs (0 / None: none); truncate_after: stop (EOI) after
-    that many scans."""
+    that many scans; tables: "flat", "long" or "mixed" (see above), for every scan or a list with one per scan;
+    fill: 0xFF fill bytes before every RSTn and before the marker after each scan; seed: of the random tables."""
     segs, _ = segments(template)
     geo = _Geom(geometry)
     sof = [p for m, p in segs if m in (0xC0, 0xC1)][0]
@@ -232,7 +281,9 @@ def write_multiscan(template: bytes, coef: np.ndarray, geometry: dict, script, p
         if truncate_after is not None and n >= truncate_after:
             break
         ri = (restarts[n] if restarts else 0) or 0
-        data, dc, ac = _encode_scan(coef, geo, list(comps), ss, se, ah, al, ri)
+        table = tables if isinstance(tables, str) else tables[n]
+        data, dc, ac = _encode_scan(coef, geo, list(comps), ss, se, ah, al, ri, table,
+                                    np.random.default_rng([seed, n]), fill)
         # tables for this scan: DC in slot n % 2, AC in slot (n + 1) % 4, so the selectors change between scans
         tdc, tac = n % 2, (n + 1) % 4
         payload = b""
@@ -258,17 +309,44 @@ def write_non_interleaved(template: bytes, coef: np.ndarray, geometry: dict, res
                            restarts=[restart_blocks] * ncomp)
 
 
+def coded_mask(geometry: dict) -> np.ndarray:
+    """Blocks that hold pixels of the image (the MCU-padding luma blocks of a colour image lie outside luma's own
+    block grid: a scan of luma alone does not code them)."""
+    ncomp, hf, vf = geometry["ncomp"], geometry["hf"], geometry["vf"]
+    ny = hf * vf if ncomp == 3 else 1
+    bpm = ny + 2 if ncomp == 3 else 1
+    bw, bh = -(-geometry["width"] // 8), -(-geometry["height"] // 8)
+    m = np.ones(geometry["mcus_x"] * geometry["mcus_y"] * bpm, dtype=bool)
+    if ncomp == 3:
+        for mcu in range(geometry["mcus_x"] * geometry["mcus_y"]):
+            my, mx = divmod(mcu, geometry["mcus_x"])
+            for s in range(ny):
+                by, bx = my * vf + s // hf, mx * hf + s % hf
+                m[mcu * bpm + s] = by < bh and bx < bw
+    return m
+
+
 def expected_after(coef: np.ndarray, ncomp: int, geometry: dict, script, k: int) -> np.ndarray:
     """The coefficients the first k scans of `script` define (numpy; for files cut after scan k): sign-magnitude
-    |v| >> Al for AC first passes, an arithmetic shift for DC, refinement bits added back."""
+    |v| >> Al for AC first passes, an arithmetic shift for DC, refinement bits added back, whole blocks for sequential
+    scans (Ss 0, Se 63).  Positions no scan codes
+    are 0, among them the MCU-padding luma blocks of scans over luma alone; a refinement band need not be a band of
+    the first passes."""
     c = np.asarray(coef, dtype=np.int32)
     out = np.zeros_like(c)
     ny = geometry["hf"] * geometry["vf"] if ncomp == 3 else 1
     bpm = ny + 2 if ncomp == 3 else 1
     comp_of = np.array([0 if b < ny else b - ny + 1 for b in range(bpm)] * (c.shape[0] // bpm))
+    inside = coded_mask(geometry)
     for comps, ss, se, ah, al in script[:k]:
         rows = np.isin(comp_of, comps)
-        if ss == 0:
+        if len(comps) == 1:
+            rows &= inside
+        if ss == 0 and se == 63:                        # sequential: the whole block
+            out[rows] = c[rows]
+        elif ss == 0 and ah:
+            out[rows, 0] |= ((c[rows, 0] >> al) & 1) << al
+        elif ss == 0:
             out[rows, 0] = (c[rows, 0] >> al) << al
         else:
             band = c[rows][:, ss:se + 1]

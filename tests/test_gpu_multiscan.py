@@ -12,6 +12,7 @@ from PIL import Image
 
 from tests import multiscan_writer as mw
 from tests.cases import cmyk_jpeg, small_cases
+from tests.multiscan_writer import coded_mask
 from tests.test_multiscan_host import CUSTOM_SCRIPT, PAIRS, pil_pair, writer_files
 from tools.gen_jpegs import synth_rgb
 
@@ -42,22 +43,6 @@ def decode(hjd, files, flags=0):
                 if r is not None:
                     r["planes"] = dec.planes(i, slab)
         return st, out
-
-
-def coded_mask(geometry):
-    """Blocks that hold pixels of the image (MCU-padding luma blocks of a non-interleaved DC scan stay 0)."""
-    ncomp, hf, vf = geometry["ncomp"], geometry["hf"], geometry["vf"]
-    ny = hf * vf if ncomp == 3 else 1
-    bpm = ny + 2 if ncomp == 3 else 1
-    bw, bh = -(-geometry["width"] // 8), -(-geometry["height"] // 8)
-    m = np.ones(geometry["mcus_x"] * geometry["mcus_y"] * bpm, dtype=bool)
-    if ncomp == 3:
-        for mcu in range(geometry["mcus_x"] * geometry["mcus_y"]):
-            my, mx = divmod(mcu, geometry["mcus_x"])
-            for s in range(ny):
-                by, bx = my * vf + s // hf, mx * hf + s % hf
-                m[mcu * bpm + s] = by < bh and bx < bw
-    return m
 
 
 def check_twin(port, got, twin, mask=None):
