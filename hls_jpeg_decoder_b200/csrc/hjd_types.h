@@ -97,6 +97,13 @@ struct HjdEntropySeg {
     uint32_t n;                  // intervals in this segment
 };
 
+#ifndef HJD_ENT_THREADS
+#define HJD_ENT_THREADS   256   // entropy kernel: one restart interval per thread
+#endif
+#ifndef HJD_ENT_MINBLOCKS
+#define HJD_ENT_MINBLOCKS 4     // CTAs per SM the entropy kernel is compiled for (register cap)
+#endif
+
 // Marker scan of long scans: slices of HJD_SCAN_SLICE_BYTES (a multiple of the 16 KB a CTA scans per step).
 #define HJD_SCAN_SLICE_MIN   (1u << 20)     // scans longer than this are sliced
 #define HJD_SCAN_SLICE_BYTES (1u << 16)

@@ -4,12 +4,6 @@
 #include <stdint.h>
 #include "hjd_types.h"
 
-#ifndef HJD_ENT_THREADS
-#define HJD_ENT_THREADS   256   // entropy kernel: one restart interval per thread
-#endif
-#ifndef HJD_ENT_MINBLOCKS
-#define HJD_ENT_MINBLOCKS 4     // CTAs per SM the entropy kernel is compiled for (register cap)
-#endif
 #define HJD_IDCT_THREADS  128   // unfused IDCT kernel: one 8x8 block per thread
 #define HJD_COLOR_THREADS 128   // unfused colour kernel: 16 pixels of one row per thread
 #define HJD_MCU_THREADS   128   // per-MCU fused kernel: one MCU (all its blocks -> RGB) per thread
