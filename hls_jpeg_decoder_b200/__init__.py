@@ -26,7 +26,7 @@ import numpy as np
 __all__ = ["probe", "MultiDecoder", "shard_range_c", "ConvertJpgFile", "ConvertJpgFiles", "DecodeJpgFileData", "JpegGetImageSize", "WriteBMP24", "encode_bmp24",
            "BatchDecoder", "HjdError", "lib", "build", "LIB_PATH",
            "FLAG_KEEP_PLANES", "FLAG_HOST_SCAN", "FLAG_NO_SELFSYNC", "FLAG_FUSED_MCU", "FLAG_BMP_OUT", "FLAG_TENSOR_CORE_IDCT", "FLAG_CUDA_CORE_IDCT", "FLAG_MULTI_SCAN", "FLAG_SCALE_1_2",
-           "FLAG_SCALE_1_4", "FLAG_SCALE_1_8", "scans", "idct_matrix", "idct_tables"]
+           "FLAG_SCALE_1_4", "FLAG_SCALE_1_8", "FLAG_GRAY_OUT", "scans", "idct_matrix", "idct_tables"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HJD_LIB_PATH") or os.path.join(_HERE, "libhjd.so")   # override: tuning builds only
@@ -43,6 +43,8 @@ FLAG_MULTI_SCAN = 256        # also decode progressive and non-interleaved files
 FLAG_SCALE_1_2 = 1 << 9      # decode to ceil(W/2) x ceil(H/2) in the DCT domain (include/hjd.h; not with KEEP_PLANES,
 FLAG_SCALE_1_4 = 2 << 9      # BMP_OUT, TENSOR_CORE_IDCT or CUDA_CORE_IDCT)
 FLAG_SCALE_1_8 = 3 << 9      # 1/8: a block is its DC alone; with MULTI_SCAN the AC scans are not read
+FLAG_GRAY_OUT = 1 << 11      # one byte per pixel: the decoded Y component (BatchDecoder.gray; include/hjd.h; not with
+                             # KEEP_PLANES, BMP_OUT, TENSOR_CORE_IDCT or CUDA_CORE_IDCT)
 
 IMG_WARN_BAD_CODE, IMG_WARN_COEF_RANGE, IMG_WARN_OVERRUN, IMG_WARN_RESTART = 1, 2, 4, 8
 
@@ -312,6 +314,7 @@ class BatchDecoder:
         if not self._h:
             raise HjdError(f"hjd_batch_create failed: {_err()}")
         self.device = device
+        self.flags = flags
         self._keep = None
 
     def close(self):
@@ -387,7 +390,7 @@ class BatchDecoder:
     @property
     def idct_variant(self) -> int:
         """bit 0: chunks of the last decode went through the tensor-core fused kernel; bit 1: through the CUDA-core one;
-        bit 2: through the scaled kernel (FLAG_SCALE_*)"""
+        bit 2: through the scaled kernel (FLAG_SCALE_*); bit 3: through a luma-only kernel (FLAG_GRAY_OUT)"""
         return lib().hjd_batch_idct_variant(self._h)
 
     @property
@@ -435,8 +438,19 @@ class BatchDecoder:
 
     def rgb(self, i: int) -> np.ndarray:
         """RGB of image i: uint8 [out_h, out_w, 3] (out_size)."""
+        if self.flags & FLAG_GRAY_OUT:
+            raise HjdError("rgb(): this batch decodes one byte per pixel (FLAG_GRAY_OUT): use gray()")
         w, h = self.out_size(i)
         out = np.zeros((h, w, 3), dtype=np.uint8)
+        _check(lib().hjd_batch_download_image(self._h, i, out.ctypes.data), "hjd_batch_download_image")
+        return out
+
+    def gray(self, i: int) -> np.ndarray:
+        """Luma of image i (batch created with FLAG_GRAY_OUT): uint8 [out_h, out_w] (out_size), the decoded Y samples."""
+        if not self.flags & FLAG_GRAY_OUT:
+            raise HjdError("gray(): this batch was not created with FLAG_GRAY_OUT")
+        w, h = self.out_size(i)
+        out = np.zeros((h, w), dtype=np.uint8)
         _check(lib().hjd_batch_download_image(self._h, i, out.ctypes.data), "hjd_batch_download_image")
         return out
 

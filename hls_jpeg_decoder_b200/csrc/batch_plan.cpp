@@ -332,6 +332,13 @@ static int layout_images(const std::vector<FileRef>& files, const PlanConfig& cf
     p->mcu_cta.assign((size_t)n + 1, 0);
     for (int i = 0; i < n; i++)
         p->mcu_cta[i + 1] = p->mcu_cta[i] + (p->imgs[i].blocks_per_mcu ? p->imgs[i].n_mcus : 0);
+    if (cfg.flags & HJD_FLAG_GRAY_OUT) {
+        // fewer luma blocks than blocks (< 2^32, checked above), so the prefix fits in uint32
+        p->luma_cta.assign((size_t)n + 1, 0);
+        for (int i = 0; i < n; i++)
+            p->luma_cta[i + 1] = p->luma_cta[i] +
+                                 (p->imgs[i].blocks_per_mcu ? (uint32_t)luma_blocks(p->imgs[i].width, p->imgs[i].height) : 0);
+    }
     return HJD_OK;
 }
 
@@ -415,6 +422,7 @@ static void chunk_extents(const std::vector<FileRef>& files, BatchPlan* p, Chunk
         }
         if (d.n_blocks > c.max_blocks) c.max_blocks = (uint32_t)d.n_blocks;
         if (d.n_mcus > c.max_mcus) c.max_mcus = d.n_mcus;
+        if (d.blocks_per_mcu && luma_blocks(d.width, d.height) > c.max_luma) c.max_luma = (uint32_t)luma_blocks(d.width, d.height);
         if (d.width > c.max_w) c.max_w = d.width;
         if (d.height > c.max_h) c.max_h = d.height;
     }

@@ -24,18 +24,29 @@ static inline uint32_t scaled_dim(unsigned flags, uint32_t v)
     return (uint32_t)(((uint64_t)v + (1u << s) - 1) >> s);
 }
 
-// Bytes of one image's region in the output slab: tightly packed RGB24 (of the scaled size with HJD_FLAG_SCALE_*), or
-// (HJD_FLAG_BMP_OUT) the BMP file WriteBMP24 would write, placed so that its pixel array starts 64 bytes into the
-// region (the 54-byte header at +10): rows padded to a multiple of 4 bytes, openjpg.cpp:534-535.
+// Bytes of one image's region in the output slab: tightly packed RGB24 (of the scaled size with HJD_FLAG_SCALE_*), one
+// byte per pixel (HJD_FLAG_GRAY_OUT), or (HJD_FLAG_BMP_OUT) the BMP file WriteBMP24 would write, placed so that its
+// pixel array starts 64 bytes into the region (the 54-byte header at +10): rows padded to a multiple of 4 bytes,
+// openjpg.cpp:534-535.
 static inline uint64_t image_out_bytes(unsigned flags, uint32_t w, uint32_t h)
 {
     if (flags & HJD_FLAG_BMP_OUT) return 64 + (uint64_t)((w * 3 + 3) & ~3u) * h;
-    return (uint64_t)scaled_dim(flags, w) * scaled_dim(flags, h) * 3;
+    return (uint64_t)scaled_dim(flags, w) * scaled_dim(flags, h) * ((flags & HJD_FLAG_GRAY_OUT) ? 1 : 3);
 }
 
 // Whether a multi-scan batch created with `flags` reads scan `s`: at 1/8 a block is its DC coefficient alone, so the AC
-// scans (Ss > 0) are not.
-static inline bool scan_is_read(unsigned flags, const HjdScanParsed& s) { return !(scale_shift(flags) == 3 && s.ss > 0); }
+// scans (Ss > 0) are not; a luma-only decode (HJD_FLAG_GRAY_OUT) does not read the scans without the frame's first
+// component.
+static inline bool scan_is_read(unsigned flags, const HjdScanParsed& s)
+{
+    if (scale_shift(flags) == 3 && s.ss > 0) return false;
+    if (flags & HJD_FLAG_GRAY_OUT) {
+        for (int k = 0; k < s.ncomp; k++)
+            if (s.comp[k] == 0) return true;
+        return false;
+    }
+    return true;
+}
 
 // Work items of one scan: the restart intervals its DRI implies (want_all) or, by default, no more than the file holds.
 uint32_t ms_scan_items(const HjdParsed& frame, const HjdScanParsed& p, uint32_t* mcus_x, uint32_t* mcus_y,
@@ -44,6 +55,9 @@ uint32_t ms_scan_items(const HjdParsed& frame, const HjdScanParsed& p, uint32_t*
 // MCU geometry of a frame (loadjpg.cpp:1170-1174) and the restart intervals of its one interleaved scan.
 struct FrameGeometry { uint32_t blocks_per_mcu, mcus_x, mcus_y, n_mcus, n_intervals; };
 FrameGeometry frame_geometry(uint32_t width, uint32_t height, int ncomp, int hf, int vf, uint32_t restart_interval);
+
+// Luma blocks that hold at least one pixel of a W x H image: ceil(W/8) x ceil(H/8) (the full-size luma kernel's threads).
+static inline uint64_t luma_blocks(uint32_t w, uint32_t h) { return (uint64_t)((w + 7) / 8) * ((h + 7) / 8); }
 
 struct FileRef { const uint8_t* ptr; int64_t size; uint64_t dev_off; };
 
@@ -58,6 +72,7 @@ struct Chunk {
     uint64_t arena_lo = 0, arena_hi = 0;      // device arena byte range holding these files
     uint64_t rgb_lo = 0, rgb_hi = 0;
     uint32_t max_blocks = 0, max_w = 0, max_h = 0, max_mcus = 0;
+    uint32_t max_luma = 0;                    // most luma blocks inside W x H of one image (HJD_FLAG_GRAY_OUT kernel grid)
     uint64_t blocks = 0;
     // kernel 1b (restart-free images of this chunk): ranges in the batch-wide index spaces, each with a gap of
     // one entry behind it so that the chunks' prefix sums (which append a sentinel) can run side by side
@@ -93,6 +108,7 @@ struct BatchPlan {
     std::vector<HjdEntropySeg> segs;
     std::vector<HjdScanSlice> slices;    // marker-scan slices of long restart-marker scans
     std::vector<uint32_t> mcu_cta;       // exclusive prefix of the per-image MCU counts (n + 1), for the flat grid of the per-MCU kernel
+    std::vector<uint32_t> luma_cta;      // HJD_FLAG_GRAY_OUT: the same for the luma blocks inside W x H (luma_blocks), per-block kernel
     std::vector<uint32_t> host_istart;   // HJD_FLAG_HOST_SCAN only
     std::vector<uint8_t> host_restart_warn;     // HJD_FLAG_HOST_SCAN only (and multi-scan images)
     // kernel 1b

@@ -117,8 +117,9 @@ struct hjd_batch {
     int launches = 0;
     int tc_chunks = 0, cc_chunks = 0;           // chunks whose MCUs went through the tensor-core / CUDA-core fused kernel
     int sc_chunks = 0;                          // ... through the scaled kernel (HJD_FLAG_SCALE_*)
+    int gy_chunks = 0;                          // ... through a luma-only kernel (HJD_FLAG_GRAY_OUT)
 
-    DevBuf d_arena, d_imgs, d_tsets, d_qsets, d_work, d_segs, d_mcucta, d_slices, d_slicecnt, d_istart, d_coef, d_planes, d_rgb, d_status;
+    DevBuf d_arena, d_imgs, d_tsets, d_qsets, d_work, d_segs, d_mcucta, d_lumacta, d_slices, d_slicecnt, d_istart, d_coef, d_planes, d_rgb, d_status;
     DevBuf d_scans, d_mswork, d_msstarts, d_mstabs;
     DevBuf d_ss, d_sswork, d_sssegs, d_destuff, d_dlen, d_counts, d_scantmp, d_ssE0, d_ssX, d_ssnb, d_flag;
     PinBuf h_meta, h_out;                       // h_out: staging of the single-image calls
@@ -177,6 +178,13 @@ extern "C" hjd_batch* hjd_batch_create(int device, unsigned flags)
         (flags & (HJD_FLAG_KEEP_PLANES | HJD_FLAG_BMP_OUT | HJD_FLAG_TENSOR_CORE_IDCT | HJD_FLAG_CUDA_CORE_IDCT))) {
         fail(HJD_ERR_ARG, "hjd_batch_create", "HJD_FLAG_SCALE_* has no planes, no BMP output and its own kernel: it combines with "
                                               "none of HJD_FLAG_KEEP_PLANES, HJD_FLAG_BMP_OUT, HJD_FLAG_TENSOR_CORE_IDCT, HJD_FLAG_CUDA_CORE_IDCT");
+        return nullptr;
+    }
+    if ((flags & HJD_FLAG_GRAY_OUT) &&
+        (flags & (HJD_FLAG_KEEP_PLANES | HJD_FLAG_BMP_OUT | HJD_FLAG_TENSOR_CORE_IDCT | HJD_FLAG_CUDA_CORE_IDCT))) {
+        fail(HJD_ERR_ARG, "hjd_batch_create", "HJD_FLAG_GRAY_OUT writes Y alone with its own kernel: it combines with none of "
+                                              "HJD_FLAG_KEEP_PLANES (the planes already hold Y), HJD_FLAG_BMP_OUT (no 8-bit BMP), "
+                                              "HJD_FLAG_TENSOR_CORE_IDCT, HJD_FLAG_CUDA_CORE_IDCT (RGB kernels)");
         return nullptr;
     }
     if (cudaSetDevice(device) != cudaSuccess) { fail(HJD_ERR_CUDA, "cudaSetDevice"); return nullptr; }
@@ -254,6 +262,7 @@ static int ensure_slabs(hjd_batch* b)
     CU(b->d_slices.ensure(sizeof(HjdScanSlice) * (p.slices.size() + 1)));
     CU(b->d_slicecnt.ensure(sizeof(uint32_t) * (p.slices.size() + 1)));
     CU(b->d_mcucta.ensure(sizeof(uint32_t) * (n + 2)));
+    if (b->flags & HJD_FLAG_GRAY_OUT) CU(b->d_lumacta.ensure(sizeof(uint32_t) * (n + 2)));
     CU(b->d_istart.ensure(sizeof(uint32_t) * ((size_t)p.total_intervals + 2)));
     CU(b->d_coef.ensure(p.total_blocks * 128 + 256));
     CU(b->d_rgb.ensure(p.rgb_bytes + 256));
@@ -298,6 +307,7 @@ static int stage_plan(hjd_batch* b)
         {&b->d_segs, p.segs.data(), sizeof(HjdEntropySeg) * p.segs.size()},
         {&b->d_sssegs, p.sssegs.data(), sizeof(HjdSsSeg) * p.sssegs.size()},
         {&b->d_mcucta, p.mcu_cta.data(), sizeof(uint32_t) * p.mcu_cta.size()},
+        {&b->d_lumacta, p.luma_cta.data(), sizeof(uint32_t) * p.luma_cta.size()},
         {&b->d_slices, p.slices.data(), sizeof(HjdScanSlice) * p.slices.size()},
         {&b->d_scans, p.scans.data(), sizeof(HjdScanDesc) * p.scans.size()},
         {&b->d_mswork, p.mswork.data(), sizeof(HjdMsWork) * p.mswork.size()},
@@ -513,7 +523,25 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
         b->launches += 1;
     }
     if (ev) CU(cudaEventRecord(ev[2], st));
-    if (scale_shift(b->flags)) {
+    if (b->flags & HJD_FLAG_GRAY_OUT) {
+        // luma-only decode (full size or scaled): its own kernel in place of the fused one, counted in the same stage
+        if (c.blocks) {
+            b->gy_chunks++;
+            if (scale_shift(b->flags)) {
+                b->sc_chunks++;
+                CU(hjd_launch_luma_scaled((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
+                                          (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_mcucta.p + c.img0, n,
+                                          b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0], c.max_mcus, scale_shift(b->flags), st));
+                b->launches += 1;
+            } else {
+                CU(hjd_launch_luma((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
+                                   (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_lumacta.p + c.img0, n,
+                                   b->plan.luma_cta[c.img1] - b->plan.luma_cta[c.img0], c.max_luma, st));
+                b->launches += 1;
+            }
+        }
+        if (ev) CU(cudaEventRecord(ev[3], st));
+    } else if (scale_shift(b->flags)) {
         // reduced-size decode: its own kernel in place of the fused one, counted in the same stage
         if (c.blocks) {
             b->sc_chunks++;
@@ -556,7 +584,7 @@ static int run_chunks(hjd_batch* b, bool h2d, uint8_t* rgb_host)
 {
     cudaStream_t main = b->stream;
     b->launches = 0;
-    b->tc_chunks = b->cc_chunks = b->sc_chunks = 0;
+    b->tc_chunks = b->cc_chunks = b->sc_chunks = b->gy_chunks = 0;
     b->ss_ran = false;
     if (b->plan.any_parse_error && b->plan.rgb_bytes) CU(cudaMemsetAsync(b->d_rgb.p, 0, b->plan.rgb_bytes, main));
     CU(cudaEventRecord(b->ev[0], main));
@@ -628,7 +656,7 @@ extern "C" int hjd_batch_num_images(const hjd_batch* b) { return b ? (int)b->pla
 extern "C" int hjd_batch_idct_variant(const hjd_batch* b)
 {
     if (!b || (b->flags & HJD_FLAG_KEEP_PLANES)) return 0;
-    return (b->tc_chunks ? 1 : 0) | (b->cc_chunks ? 2 : 0) | (b->sc_chunks ? 4 : 0);
+    return (b->tc_chunks ? 1 : 0) | (b->cc_chunks ? 2 : 0) | (b->sc_chunks ? 4 : 0) | (b->gy_chunks ? 8 : 0);
 }
 // Kernel 1b's round words of the last decode (run_selfsync), read once the stream is idle: the most rounds any chunk
 // ran (working rounds + the one that confirmed), and whether a chunk hit the round limit.

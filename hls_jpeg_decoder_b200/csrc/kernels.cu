@@ -1113,6 +1113,89 @@ hjd_k_mcu_rgb(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// luma only (HJD_FLAG_GRAY_OUT): one thread decodes one luma block to its W x H crop of the Y plane
+// ------------------------------------------------------------------------------------------
+// The threads of an image take its luma blocks that hold a pixel, row-major over ceil(W/8) x ceil(H/8), so the
+// lanes of a warp own horizontally adjacent blocks and each of the eight row stores of a warp covers up to 256
+// contiguous bytes.  Chroma blocks and MCU-padding blocks are not read.  hjd_idct_block, unchanged, writes the
+// block into a thread-private shared-memory tile interleaved by thread (as hjd_k_mcu_rgb does), where the exact
+// re-evaluation patches its bytes; then the rows go out clipped at W and H, 8 bytes at once where aligned.
+// Grids as hjd_k_mcu_rgb (FLAT: a 1-D grid over all luma blocks of the batch, the image found by binary search).
+template <bool FLAT>
+__global__ void __launch_bounds__(HJD_LUMA_THREADS, HJD_MCU_MINBLOCKS)
+hjd_k_luma(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ imgs,
+           const HjdQuantSet* __restrict__ qsets, uint8_t* __restrict__ out,
+           const uint32_t* __restrict__ luma_prefix, int n_images, int img_base)
+{
+    __shared__ float s_cos[64];
+    __shared__ uint2 s_tile[8 * HJD_LUMA_THREADS];               // 8 rows x T threads x 8 bytes
+    const uint32_t t = threadIdx.x;
+    if (t < 64) s_cos[t] = c_cos[t];
+    __syncthreads();
+
+    const HjdImageDesc* d;
+    uint32_t k;
+    if (FLAT) {
+        const uint32_t key = blockIdx.x * HJD_LUMA_THREADS + t + luma_prefix[0];
+        if (key >= luma_prefix[n_images]) return;
+        int lo = 0, hi = n_images - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (luma_prefix[mid] <= key) lo = mid; else hi = mid - 1;
+        }
+        d = imgs + lo;
+        k = key - luma_prefix[lo];
+    } else {
+        d = imgs + (blockIdx.y + img_base);
+        k = blockIdx.x * HJD_LUMA_THREADS + t;
+    }
+    const uint32_t W = d->width, H = d->height;
+    const uint32_t bw = (W + 7) >> 3;
+    if (d->blocks_per_mcu == 0 || k >= bw * ((H + 7) >> 3)) return;
+    const uint32_t by = k / bw, bx = k - by * bw;                 // block column / row in the Y plane
+    const uint32_t hf = d->hf, vf = d->vf;                        // 1 or 2 (1 for one-component files)
+    const uint32_t mx = bx / hf, my = by / vf;
+    const uint32_t bi = (by - my * vf) * hf + (bx - mx * hf);     // Y blocks row-major inside the MCU (loadjpg.cpp:949-959)
+    const uint64_t blk = d->block_base + (uint64_t)(my * d->mcus_x + mx) * d->blocks_per_mcu + bi;
+    constexpr uint32_t kPitch = HJD_LUMA_THREADS * 8;
+    uint8_t* tile = (uint8_t*)&s_tile[t];
+    hjd_idct_block((const uint4*)(coef + blk * 64), (const uint4*)qsets[d->quant_set].qp[0], s_cos, tile, kPitch);
+
+    const uint32_t x0 = bx * 8, y0 = by * 8;
+    const uint32_t nx = min(8u, W - x0), nr = min(8u, H - y0);
+    uint8_t* dst = out + d->rgb_off + (uint64_t)y0 * W + x0;
+#pragma unroll 1
+    for (uint32_t r = 0; r < nr; r++) {
+        const uint2 v = *(const uint2*)(tile + r * kPitch);
+        uint8_t* row = dst + (uint64_t)r * W;
+        if (nx == 8 && (((uintptr_t)row) & 7) == 0) {
+            *(uint2*)row = v;
+        } else {
+#pragma unroll
+            for (uint32_t i = 0; i < 8; i++)
+                if (i < nx) row[i] = (uint8_t)((i < 4 ? v.x : v.y) >> (8 * (i & 3)));
+        }
+    }
+}
+
+cudaError_t hjd_launch_luma(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
+                            const uint32_t* luma_prefix, int n_images, uint32_t n_luma, uint32_t max_luma, cudaStream_t st)
+{
+    if (n_images <= 0 || n_luma == 0 || max_luma == 0) return cudaSuccess;
+    const unsigned gx = (max_luma + HJD_LUMA_THREADS - 1) / HJD_LUMA_THREADS;
+    if ((uint64_t)gx * HJD_LUMA_THREADS * (uint64_t)n_images <= (uint64_t)n_luma * 4) {   // the rule of hjd_launch_mcu_rgb
+        for (int base = 0; base < n_images; base += 65535) {
+            const int n = min(65535, n_images - base);
+            hjd_k_luma<false><<<dim3(gx, n), HJD_LUMA_THREADS, 0, st>>>(coef, imgs, qsets, out, nullptr, n_images, base);
+        }
+    } else {
+        const unsigned g = (unsigned)(((uint64_t)n_luma + HJD_LUMA_THREADS - 1) / HJD_LUMA_THREADS);
+        hjd_k_luma<true><<<g, HJD_LUMA_THREADS, 0, st>>>(coef, imgs, qsets, out, luma_prefix, n_images, 0);
+    }
+    return cudaGetLastError();
+}
+
 #include "mcu_tc.cuh"
 
 // The IDCT matrix of the tensor-core kernel (see mcu_tc.cuh): M[k][8y+x] = 0.25 * C(u)C(v) * cos[x][u] * cos[y][v], the

@@ -50,3 +50,12 @@ cudaError_t hjd_launch_color(const uint8_t* planes, const HjdImageDesc* imgs, ui
 cudaError_t hjd_launch_mcu_rgb(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets,
                                uint8_t* rgb, const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus,
                                uint32_t max_mcus, bool bmp, int variant, cudaStream_t st);
+
+// Luma-only decode at full size (HJD_FLAG_GRAY_OUT): one thread = one luma block that holds a pixel of its image
+// (ceil(W/8) x ceil(H/8) of them, row-major), the IDCT of the fused kernel, rows clipped at W and H; image i is
+// written at imgs[i].rgb_off as W x H bytes, stride W.  Chroma blocks are not read.  luma_prefix[i] = those blocks
+// of images 0..i-1 (any common offset; n_images + 1 entries); n_luma = luma_prefix[n_images] - luma_prefix[0];
+// max_luma = blocks of the largest image.  The grid choice of hjd_launch_mcu_rgb, over blocks instead of MCUs.
+#define HJD_LUMA_THREADS 128
+cudaError_t hjd_launch_luma(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
+                            const uint32_t* luma_prefix, int n_images, uint32_t n_luma, uint32_t max_luma, cudaStream_t st);

@@ -213,6 +213,95 @@ hjd_k_mcu_rgb_scaled(const int16_t* __restrict__ coef, const HjdImageDesc* __res
     }
 }
 
+// Luma-only sibling of hjd_k_mcu_rgb_scaled (HJD_FLAG_GRAY_OUT with a scale flag): the same threads, grids and luma
+// IDCTs, no chroma IDCT and no colour conversion; the N x N luma samples of each block are stored as they are, one byte
+// per pixel, stride ow.
+template <int N, bool FLAT>
+__global__ void __launch_bounds__(HJD_MCU_THREADS)
+hjd_k_luma_scaled(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ imgs,
+                  const HjdQuantSet* __restrict__ qsets, uint8_t* __restrict__ out,
+                  const uint32_t* __restrict__ mcu_prefix, int n_images, int img_base)
+{
+    constexpr uint32_t D = 8 / N;
+    const uint32_t t = threadIdx.x;
+    const HjdImageDesc* d;
+    uint32_t m;
+    if (FLAT) {
+        const uint32_t key = blockIdx.x * HJD_MCU_THREADS + t + mcu_prefix[0];
+        if (key >= mcu_prefix[n_images]) return;
+        int lo = 0, hi = n_images - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (mcu_prefix[mid] <= key) lo = mid; else hi = mid - 1;
+        }
+        d = imgs + lo;
+        m = key - mcu_prefix[lo];
+    } else {
+        d = imgs + (blockIdx.y + img_base);
+        m = blockIdx.x * HJD_MCU_THREADS + t;
+    }
+    if (m >= d->n_mcus || d->blocks_per_mcu == 0) return;
+    const uint32_t hf = d->hf, vf = d->vf, bpm = d->blocks_per_mcu;
+    const uint32_t ny = d->ncomp == 1 ? 1u : hf * vf;
+    const uint32_t my = m / d->mcus_x, mx = m - my * d->mcus_x;
+    const HjdQuantSet* qs = qsets + d->quant_set;
+    const int16_t* cp = coef + (d->block_base + (uint64_t)m * bpm) * 64;
+    const uint32_t ow = (d->width + D - 1) / D, oh = (d->height + D - 1) / D;   // jdiv_round_up(W, d)
+    uint8_t* img_out = out + d->rgb_off;
+#pragma unroll 1
+    for (uint32_t bi = 0; bi < ny; bi++) {
+        const uint32_t bx = bi % hf, by = bi / hf;
+        const uint32_t x0 = (mx * hf + bx) * N, y0 = (my * vf + by) * N;
+        if (x0 >= ow || y0 >= oh) continue;             // pixels at or beyond the output size are not written
+        int v[N * N];
+        sc_idct<N>(cp + bi * 64, qs->q[0], v);
+        const uint32_t npix = min((uint32_t)N, ow - x0);
+#pragma unroll
+        for (int y = 0; y < N; y++) {
+            if (y0 + y >= oh) break;
+            uint8_t* dst = img_out + (uint64_t)(y0 + y) * ow + x0;
+            if (N == 4 && npix == 4 && (((uintptr_t)dst) & 3) == 0) {
+                *(uint32_t*)dst = (uint32_t)v[y * N] | (uint32_t)v[y * N + 1] << 8 | (uint32_t)v[y * N + 2] << 16 |
+                                  (uint32_t)v[y * N + 3] << 24;
+            } else {
+#pragma unroll
+                for (int x = 0; x < N; x++)
+                    if ((uint32_t)x < npix) dst[x] = (uint8_t)v[y * N + x];
+            }
+        }
+    }
+}
+
+template <int N>
+static void launch_luma_n(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
+                          const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus, uint32_t max_mcus, cudaStream_t st)
+{
+    const unsigned gx = (max_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS;
+    if ((uint64_t)gx * HJD_MCU_THREADS * (uint64_t)n_images <= (uint64_t)n_mcus * 4) {   // the grid choice of launch_n
+        for (int base = 0; base < n_images; base += 65535) {
+            const int n = min(65535, n_images - base);
+            hjd_k_luma_scaled<N, false><<<dim3(gx, n), HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, out, nullptr, n_images, base);
+        }
+    } else {
+        const unsigned g = (unsigned)(((uint64_t)n_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS);
+        hjd_k_luma_scaled<N, true><<<g, HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, out, mcu_prefix, n_images, 0);
+    }
+}
+
+cudaError_t hjd_launch_luma_scaled(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets,
+                                   uint8_t* out, const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus,
+                                   uint32_t max_mcus, int shift, cudaStream_t st)
+{
+    if (n_images <= 0 || n_mcus == 0 || max_mcus == 0) return cudaSuccess;
+    switch (shift) {
+        case 1: launch_luma_n<4>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
+        case 2: launch_luma_n<2>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
+        case 3: launch_luma_n<1>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
 template <int N>
 static void launch_n(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* rgb,
                      const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus, uint32_t max_mcus, cudaStream_t st)

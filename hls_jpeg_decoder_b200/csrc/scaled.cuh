@@ -14,3 +14,8 @@ cudaError_t hjd_set_scaled_constants(const float cos4[16], const float cos2[4], 
 cudaError_t hjd_launch_mcu_rgb_scaled(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets,
                                       uint8_t* rgb, const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus,
                                       uint32_t max_mcus, int shift, cudaStream_t st);
+// The same for HJD_FLAG_GRAY_OUT: the luma samples only (no chroma IDCT, no colour conversion), written at imgs[i].rgb_off
+// as ceil(W >> shift) x ceil(H >> shift) bytes, stride that width.
+cudaError_t hjd_launch_luma_scaled(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets,
+                                   uint8_t* out, const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus,
+                                   uint32_t max_mcus, int shift, cudaStream_t st);

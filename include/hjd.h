@@ -97,6 +97,22 @@ extern "C" {
 #define HJD_FLAG_SCALE_1_4   (2u << 9)
 #define HJD_FLAG_SCALE_1_8   (3u << 9)
 #define HJD_FLAG_SCALE_MASK  (3u << 9)
+/* Single-channel luma output (the grayscale read mode of libjpeg's JCS_GRAYSCALE, nvJPEG's NVJPEG_OUTPUT_Y): a W x H
+ * image decodes to W x H bytes (with HJD_FLAG_SCALE_1_d: ceil(W/d) x ceil(H/d)), top-down rows, stride = output width,
+ * each image 256-byte aligned in the slab at rgb_offset.  Pixel (x, y) is the Y sample (x, y) the full decode computes
+ * before colour conversion: the reference's IDCT of the luma blocks with the luma table, +128, clamp -- exactly the Y
+ * plane of HJD_FLAG_KEEP_PLANES, cropped from the MCU-padded plane to W x H.  A one-component file outputs its only
+ * component (= each channel of its RGB decode).  With a scale flag: the luma samples of the scaled decode.  Not a
+ * weighted sum of R, G and B.
+ * With HJD_FLAG_MULTI_SCAN, a scan none of whose components is the frame's first is not read: it gets no work items, is
+ * not counted by hjd_batch_num_scans or n_intervals, damage inside it is not reported, and the coefficients only it
+ * codes stay 0.  Interleaved scans (sequential ones, a DC scan of Y, Cb and Cr) are read whole.  With
+ * HJD_FLAG_SCALE_1_8 both rules apply.
+ * Combines with HJD_FLAG_MULTI_SCAN, HJD_FLAG_SCALE_*, HJD_FLAG_HOST_SCAN and HJD_FLAG_NO_SELFSYNC.  Not combinable
+ * (hjd_batch_create fails with HJD_ERR_ARG): HJD_FLAG_BMP_OUT (an 8-bit palettised BMP is not WriteBMP24's format),
+ * HJD_FLAG_KEEP_PLANES (the planes already hold Y), HJD_FLAG_TENSOR_CORE_IDCT and HJD_FLAG_CUDA_CORE_IDCT (they select
+ * RGB kernels). */
+#define HJD_FLAG_GRAY_OUT    (1u << 11)
 
 typedef struct hjd_batch hjd_batch;
 
@@ -217,16 +233,17 @@ int  hjd_batch_selfsync_rounds(hjd_batch* b);                        /* syncs */
  * to 256 (testing / tuning; results do not depend on it).  Takes effect at the next upload. */
 int  hjd_batch_set_selfsync_range(hjd_batch* b, int range);
 /* Which fused kernel(s) the chunks of the last decode went through: bit 0 = tensor cores (csrc/mcu_tc.cuh), bit 1 = CUDA
- * cores, bit 2 = the scaled kernel (HJD_FLAG_SCALE_*, csrc/scaled.cu); 0 = none (nothing decoded yet, or
- * HJD_FLAG_KEEP_PLANES). */
+ * cores, bit 2 = the scaled kernel (HJD_FLAG_SCALE_*, csrc/scaled.cu), bit 3 = a luma-only kernel (HJD_FLAG_GRAY_OUT;
+ * with a scale flag set together with bit 2); 0 = none (nothing decoded yet, or HJD_FLAG_KEEP_PLANES). */
 int  hjd_batch_idct_variant(const hjd_batch* b);
 int  hjd_batch_num_images(const hjd_batch* b);
 /* Scans image i of the last upload is decoded from (1: single-scan baseline; 0: not decodable).  HJD_FLAG_SCALE_1_8
- * with HJD_FLAG_MULTI_SCAN: its DC scans only. */
+ * with HJD_FLAG_MULTI_SCAN: its DC scans only; HJD_FLAG_GRAY_OUT with HJD_FLAG_MULTI_SCAN: the scans that contain luma. */
 int  hjd_batch_num_scans(const hjd_batch* b, int i);
 /* hjd_image_info describes the source image (width, height: its frame). */
 int  hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* out);
-/* Dimensions of image i's decoded output: width x height, or ceil(width/d) x ceil(height/d) with HJD_FLAG_SCALE_1_d. */
+/* Dimensions of image i's decoded output: width x height, or ceil(width/d) x ceil(height/d) with HJD_FLAG_SCALE_1_d
+ * (the same with HJD_FLAG_GRAY_OUT). */
 int  hjd_batch_get_out_size(const hjd_batch* b, int i, uint32_t* w, uint32_t* h);
 int  hjd_batch_get_status(hjd_batch* b, int32_t* status /* n */);   /* syncs */
 int  hjd_batch_get_timings(hjd_batch* b, hjd_timings* out);          /* syncs */
@@ -236,7 +253,7 @@ int  hjd_batch_get_timings(hjd_batch* b, hjd_timings* out);          /* syncs */
 #define HJD_MARK_SLOTS 130
 int   hjd_batch_mark(hjd_batch* b, int slot);
 float hjd_batch_elapsed_ms(hjd_batch* b, int slot_a, int slot_b);
-uint64_t hjd_batch_rgb_bytes(const hjd_batch* b);     /* size of the RGB slab */
+uint64_t hjd_batch_rgb_bytes(const hjd_batch* b);     /* size of the RGB slab (the output slab: 1 byte per pixel with HJD_FLAG_GRAY_OUT) */
 uint64_t hjd_batch_coef_bytes(const hjd_batch* b);
 uint64_t hjd_batch_plane_bytes(const hjd_batch* b);
 uint64_t hjd_batch_scan_bytes(const hjd_batch* b);    /* sum of entropy-coded bytes */
@@ -249,7 +266,8 @@ void* hjd_batch_device_planes(hjd_batch* b);
 
 /* Device -> host copies (synchronous with respect to the batch stream). */
 int  hjd_batch_download_rgb(hjd_batch* b, uint8_t* dst /* hjd_batch_rgb_bytes */);
-int  hjd_batch_download_image(hjd_batch* b, int i, uint8_t* dst /* out_w*out_h*3, hjd_batch_get_out_size */);
+int  hjd_batch_download_image(hjd_batch* b, int i, uint8_t* dst /* out_w*out_h*3 (HJD_FLAG_GRAY_OUT: out_w*out_h),
+                                                                    hjd_batch_get_out_size */);
 int  hjd_batch_download_coef(hjd_batch* b, int16_t* dst /* hjd_batch_coef_bytes */);
 uint64_t hjd_batch_bmp_bytes(const hjd_batch* b, int i);            /* HJD_FLAG_BMP_OUT: size of image i's BMP file (0: none) */
 int  hjd_batch_download_bmp(hjd_batch* b, int i, uint8_t* dst /* hjd_batch_bmp_bytes(i) */);
@@ -263,7 +281,9 @@ int  hjd_batch_decode_host(hjd_batch* b, const uint8_t* arena, const int64_t* of
                            int n, uint8_t* rgb_out, uint64_t rgb_capacity, uint64_t* rgb_offsets_out,
                            int32_t* status_out, int chunk_images);
 /* Bytes hjd_batch_decode_host needs in rgb_out for these files (header parse only); hjd_out_slab_bytes: the
- * same for a batch created with `flags` (HJD_FLAG_BMP_OUT changes the layout, HJD_FLAG_SCALE_* the output size). */
+ * same for a batch created with `flags` (HJD_FLAG_BMP_OUT changes the layout, HJD_FLAG_SCALE_* the output size,
+ * HJD_FLAG_GRAY_OUT the bytes per pixel: align_up(out_w * out_h, 256) per image).  The hjd_multi_* calls follow the
+ * flags of their handle in the same way. */
 uint64_t hjd_rgb_slab_bytes(const uint8_t* arena, const int64_t* offsets, const int64_t* sizes, int n);
 uint64_t hjd_out_slab_bytes(const uint8_t* arena, const int64_t* offsets, const int64_t* sizes, int n, unsigned flags);
 
