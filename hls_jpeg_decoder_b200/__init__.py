@@ -26,7 +26,7 @@ import numpy as np
 __all__ = ["probe", "MultiDecoder", "shard_range_c", "ConvertJpgFile", "ConvertJpgFiles", "DecodeJpgFileData", "JpegGetImageSize", "WriteBMP24", "encode_bmp24",
            "BatchDecoder", "HjdError", "lib", "build", "LIB_PATH",
            "FLAG_KEEP_PLANES", "FLAG_HOST_SCAN", "FLAG_NO_SELFSYNC", "FLAG_FUSED_MCU", "FLAG_BMP_OUT", "FLAG_TENSOR_CORE_IDCT", "FLAG_CUDA_CORE_IDCT", "FLAG_MULTI_SCAN", "FLAG_SCALE_1_2",
-           "FLAG_SCALE_1_4", "FLAG_SCALE_1_8", "FLAG_GRAY_OUT", "scans", "idct_matrix", "idct_tables"]
+           "FLAG_SCALE_1_4", "FLAG_SCALE_1_8", "FLAG_GRAY_OUT", "FLAG_EXIF_ORIENT", "scans", "orientation", "idct_matrix", "idct_tables"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("HJD_LIB_PATH") or os.path.join(_HERE, "libhjd.so")   # override: tuning builds only
@@ -45,6 +45,8 @@ FLAG_SCALE_1_4 = 2 << 9      # BMP_OUT, TENSOR_CORE_IDCT or CUDA_CORE_IDCT)
 FLAG_SCALE_1_8 = 3 << 9      # 1/8: a block is its DC alone; with MULTI_SCAN the AC scans are not read
 FLAG_GRAY_OUT = 1 << 11      # one byte per pixel: the decoded Y component (BatchDecoder.gray; include/hjd.h; not with
                              # KEEP_PLANES, BMP_OUT, TENSOR_CORE_IDCT or CUDA_CORE_IDCT)
+FLAG_EXIF_ORIENT = 1 << 12   # apply each file's EXIF orientation to its output (out_size swaps for 5-8; include/hjd.h; not
+                             # with BMP_OUT)
 
 IMG_WARN_BAD_CODE, IMG_WARN_COEF_RANGE, IMG_WARN_OVERRUN, IMG_WARN_RESTART = 1, 2, 4, 8
 
@@ -153,6 +155,8 @@ _SIGS = {
     "hjd_probe_jpeg_scans": (c_int, [c_void_p, c_int64, POINTER(ScanInfo), c_int]),
     "hjd_batch_num_scans": (c_int, [c_void_p, c_int]),
     "hjd_batch_get_out_size": (c_int, [c_void_p, c_int, POINTER(c_uint32), POINTER(c_uint32)]),
+    "hjd_batch_get_orientation": (c_int, [c_void_p, c_int]),
+    "hjd_probe_jpeg_orientation": (c_int, [c_void_p, c_int64]),
     "hjd_huff_lookup_probe": (c_uint32, [c_void_p, c_void_p, c_int, c_int, c_uint32]),
 }
 
@@ -249,6 +253,16 @@ def scans(buf: bytes) -> list[dict]:
     lib().hjd_probe_jpeg_scans(ptr, data.size, out, n)
     return [dict(ncomp=s.ncomp, comp=list(s.comp[:s.ncomp]), ss=s.ss, se=s.se, ah=s.ah, al=s.al, level=s.level,
                  restart_interval=s.restart_interval, bytes=s.bytes) for s in out[:n]]
+
+
+def orientation(buf: bytes) -> int:
+    """The EXIF orientation (1..8) the file states, as FLAG_EXIF_ORIENT applies it (header parse only, no GPU); 1 when
+    the file has none or a malformed one.  Raises HjdError when the buffer does not start with SOI."""
+    data = np.frombuffer(buf, dtype=np.uint8)
+    o = lib().hjd_probe_jpeg_orientation(data.ctypes.data if data.size else None, data.size)
+    if o < 1:
+        raise HjdError(f"not a JPEG (status {o})")
+    return int(o)
 
 
 def WriteBMP24(szBmpFileName: str, Width: int, Height: int, RGB) -> None:
@@ -431,10 +445,18 @@ class BatchDecoder:
         return lib().hjd_batch_coef_bytes(self._h)
 
     def out_size(self, i: int) -> tuple[int, int]:
-        """(width, height) of image i's decoded output: the source size, or ceil(W/d) x ceil(H/d) with FLAG_SCALE_1_d."""
+        """(width, height) of image i's decoded output: the source size, or ceil(W/d) x ceil(H/d) with FLAG_SCALE_1_d;
+        swapped with FLAG_EXIF_ORIENT for orientations 5-8."""
         w, h = c_uint32(), c_uint32()
         _check(lib().hjd_batch_get_out_size(self._h, i, ctypes.byref(w), ctypes.byref(h)), "hjd_batch_get_out_size")
         return w.value, h.value
+
+    def orientation(self, i: int) -> int:
+        """The EXIF orientation (1..8) image i's file states; applied to the output only with FLAG_EXIF_ORIENT."""
+        o = lib().hjd_batch_get_orientation(self._h, i)
+        if o < 1:
+            raise HjdError(f"hjd_batch_get_orientation failed: {_err()}")
+        return int(o)
 
     def rgb(self, i: int) -> np.ndarray:
         """RGB of image i: uint8 [out_h, out_w, 3] (out_size)."""

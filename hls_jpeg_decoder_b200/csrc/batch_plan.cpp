@@ -104,6 +104,7 @@ struct Lite {
     uint64_t tk, qk;
     uint64_t ms_items;         // multi-scan work items (what ms_add_image will add)
     int trep, qrep;            // image whose tables / quantisation tables these are byte-identical to (itself: a representative)
+    int orientation;           // EXIF orientation the file states (1..8)
 };
 typedef std::vector<std::unique_ptr<HjdMultiParsed>> MultiList;
 
@@ -145,6 +146,7 @@ static int parse_files(const std::vector<FileRef>& files, unsigned flags, std::v
                 }
             }
             l.status = st;
+            l.orientation = (files[i].ptr && files[i].size > 0) ? p.orientation : 1;
             if (st != HJD_IMG_OK) continue;
             l.width = p.width; l.height = p.height; l.restart_interval = p.restart_interval;
             l.ncomp = p.ncomp; l.hf = p.hf; l.vf = p.vf;
@@ -265,6 +267,7 @@ static int layout_images(const std::vector<FileRef>& files, const PlanConfig& cf
         d.rgb_off = p->rgb_bytes;
         d.y_off = d.cb_off = d.cr_off = p->plane_bytes;
         const Lite& ps = lite[(size_t)i];
+        p->orientation[i] = (uint8_t)ps.orientation;
         const HjdMultiParsed* mp = multi[(size_t)i].get();
         int st = ps.status;
         uint32_t tset = 0, qset = 0;
@@ -342,6 +345,44 @@ static int layout_images(const std::vector<FileRef>& files, const PlanConfig& cf
     return HJD_OK;
 }
 
+// HJD_FLAG_EXIF_ORIENT: every decodable image whose file states an orientation other than 1 is decoded into a private
+// staging region behind rgb_bytes (its descriptor's rgb_off, which the decode kernels write to) and turned into its place
+// in the slab (out_off) by the orientation pass.  Private regions: chunks in flight together never share one.
+static void plan_staging(const PlanConfig& cfg, BatchPlan* p)
+{
+    const int n = (int)p->imgs.size();
+    p->out_off.resize((size_t)n);
+    for (int i = 0; i < n; i++) {
+        HjdImageDesc& d = p->imgs[i];
+        p->out_off[i] = d.rgb_off;
+        if (!(cfg.flags & HJD_FLAG_EXIF_ORIENT) || p->orientation[i] == 1 || !d.blocks_per_mcu) continue;
+        d.rgb_off = p->rgb_bytes + p->stage_bytes;
+        p->stage_bytes += align_up(image_out_bytes(cfg.flags, d.width, d.height), 256);
+    }
+}
+
+// The orientation jobs of a chunk's images, and the exclusive prefix of their tiles (one batch-wide list).  The tile
+// count fits in uint32: every tile covers at least one luma block of its image, and a batch has fewer than 2^32 blocks.
+static void chunk_orient(const PlanConfig& cfg, BatchPlan* p, Chunk& c)
+{
+    if (p->orient_tiles.empty()) p->orient_tiles.push_back(0);
+    c.oj0 = (uint32_t)p->orient_jobs.size();
+    for (int i = c.img0; i < c.img1; i++) {
+        const HjdImageDesc& d = p->imgs[i];
+        if (d.rgb_off == p->out_off[i]) continue;
+        HjdOrientJob j;
+        memset(&j, 0, sizeof j);
+        j.src_off = d.rgb_off;
+        j.dst_off = p->out_off[i];
+        j.w = scaled_dim(cfg.flags, d.width);
+        j.h = scaled_dim(cfg.flags, d.height);
+        j.o = p->orientation[i];
+        p->orient_jobs.push_back(j);
+        p->orient_tiles.push_back(p->orient_tiles.back() + orient_tiles(j.w, j.h));
+    }
+    c.oj1 = (uint32_t)p->orient_jobs.size();
+}
+
 // Stage 3: contiguous image ranges of roughly equal block counts.
 static void plan_chunks(const PlanConfig& cfg, BatchPlan* p)
 {
@@ -412,8 +453,8 @@ static void chunk_extents(const std::vector<FileRef>& files, BatchPlan* p, Chunk
 {
     const int n = (int)p->imgs.size();
     c.arena_lo = ~0ull; c.arena_hi = 0;
-    c.rgb_lo = p->imgs[c.img0].rgb_off;
-    c.rgb_hi = (c.img1 < n) ? p->imgs[c.img1].rgb_off : p->rgb_bytes;
+    c.rgb_lo = p->out_off[c.img0];
+    c.rgb_hi = (c.img1 < n) ? p->out_off[c.img1] : p->rgb_bytes;
     for (int i = c.img0; i < c.img1; i++) {
         const HjdImageDesc& d = p->imgs[i];
         if (files[i].ptr && files[i].size > 0) {
@@ -573,6 +614,7 @@ int hjd_plan_batch(const std::vector<FileRef>& files, const PlanConfig& cfg, Bat
     p->parse_status.assign(n, 0);
     p->host_restart_warn.assign(n, 0);
     p->ms_items.assign(n, 0); p->n_scans.assign(n, 0); p->ms_image.assign(n, 0);
+    p->orientation.assign(n, 1);
     std::vector<Lite> lite(n);
     MultiList multi(n);
     int rc = parse_files(files, cfg.flags, lite, multi, err);
@@ -580,9 +622,11 @@ int hjd_plan_batch(const std::vector<FileRef>& files, const PlanConfig& cfg, Bat
     std::vector<uint32_t> ms_w0(n + 1, 0);
     rc = layout_images(files, cfg, lite, multi, p, ms_w0, err);
     if (rc != HJD_OK) return rc;
+    plan_staging(cfg, p);
     plan_chunks(cfg, p);
     for (Chunk& c : p->chunks) {
         chunk_extents(files, p, c);
+        chunk_orient(cfg, p, c);
         chunk_entropy_work(cfg, p, c);
         chunk_multiscan(p, c, ms_w0[(size_t)c.img0], ms_w0[(size_t)c.img1]);
     }

@@ -56,6 +56,21 @@ uint32_t ms_scan_items(const HjdParsed& frame, const HjdScanParsed& p, uint32_t*
 struct FrameGeometry { uint32_t blocks_per_mcu, mcus_x, mcus_y, n_mcus, n_intervals; };
 FrameGeometry frame_geometry(uint32_t width, uint32_t height, int ncomp, int hf, int vf, uint32_t restart_interval);
 
+// Size of an image's decoded output (hjd_batch_get_out_size): the scaled size of its w x h frame, with width and height
+// swapped when HJD_FLAG_EXIF_ORIENT applies an orientation 5..8 (o: what its file states).
+static inline void out_size(unsigned flags, uint32_t w, uint32_t h, int o, uint32_t* out_w, uint32_t* out_h)
+{
+    const bool swap = (flags & HJD_FLAG_EXIF_ORIENT) && o >= 5;
+    *out_w = scaled_dim(flags, swap ? h : w);
+    *out_h = scaled_dim(flags, swap ? w : h);
+}
+
+// Output tiles of the orientation pass (csrc/orient.cu) of an out_w x out_h image.
+static inline uint32_t orient_tiles(uint32_t out_w, uint32_t out_h)
+{
+    return ((out_w + HJD_ORIENT_TILE - 1) / HJD_ORIENT_TILE) * ((out_h + HJD_ORIENT_TILE - 1) / HJD_ORIENT_TILE);
+}
+
 // Luma blocks that hold at least one pixel of a W x H image: ceil(W/8) x ceil(H/8) (the full-size luma kernel's threads).
 static inline uint64_t luma_blocks(uint32_t w, uint32_t h) { return (uint64_t)((w + 7) / 8) * ((h + 7) / 8); }
 
@@ -84,6 +99,7 @@ struct Chunk {
     // multi-scan images of this chunk: their slab blocks (zeroed before the first level), their work items per level
     std::vector<std::pair<uint64_t, uint64_t>> ms_zero;     // (first block, blocks)
     std::vector<std::pair<uint32_t, uint32_t>> ms_levels;   // work item range of each level present, in level order
+    uint32_t oj0 = 0, oj1 = 0;                // HJD_FLAG_EXIF_ORIENT: this chunk's entries of BatchPlan::orient_jobs
 };
 
 // What the planner is asked for.
@@ -127,6 +143,16 @@ struct BatchPlan {
     std::vector<std::vector<uint8_t>> ms_tab_raw;
     std::vector<uint32_t> ms_items, n_scans;    // work items (multi-scan images), scans (0: not decodable)
     std::vector<uint8_t> ms_image;              // decoded by the multi-scan kernel (its blocks are zeroed first)
+    // EXIF orientation.  orientation: what each file states (1..8), with or without the flag.  out_off: where each
+    // image's output ends up in the slab, the offset every host consumer uses; it equals imgs[i].rgb_off unless the
+    // image is oriented (HJD_FLAG_EXIF_ORIENT, orientation != 1), when imgs[i].rgb_off -- where the decode kernels write
+    // -- is a private staging region of image_out_bytes behind rgb_bytes.  orient_jobs: one per oriented image, in
+    // image order; orient_tiles: the exclusive prefix of their output tiles (n + 1).
+    std::vector<uint8_t> orientation;
+    std::vector<uint64_t> out_off;
+    std::vector<HjdOrientJob> orient_jobs;
+    std::vector<uint32_t> orient_tiles;
+    uint64_t stage_bytes = 0;                   // staging regions, behind rgb_bytes in the same device allocation
     std::vector<Chunk> chunks;
     uint64_t total_blocks = 0, rgb_bytes = 0, plane_bytes = 0, scan_bytes = 0, pixels = 0;
     uint32_t total_intervals = 0;

@@ -13,6 +13,7 @@
 #include "selfsync.cuh"
 #include "multiscan.cuh"
 #include "scaled.cuh"
+#include "orient.cuh"
 
 #include <cuda_runtime.h>
 #include <math.h>
@@ -121,6 +122,7 @@ struct hjd_batch {
 
     DevBuf d_arena, d_imgs, d_tsets, d_qsets, d_work, d_segs, d_mcucta, d_lumacta, d_slices, d_slicecnt, d_istart, d_coef, d_planes, d_rgb, d_status;
     DevBuf d_scans, d_mswork, d_msstarts, d_mstabs;
+    DevBuf d_ojobs, d_otiles;                   // HJD_FLAG_EXIF_ORIENT
     DevBuf d_ss, d_sswork, d_sssegs, d_destuff, d_dlen, d_counts, d_scantmp, d_ssE0, d_ssX, d_ssnb, d_flag;
     PinBuf h_meta, h_out;                       // h_out: staging of the single-image calls
 };
@@ -170,6 +172,11 @@ extern "C" int hjd_device_count(void)
 
 extern "C" hjd_batch* hjd_batch_create(int device, unsigned flags)
 {
+    if ((flags & HJD_FLAG_EXIF_ORIENT) && (flags & HJD_FLAG_BMP_OUT)) {
+        fail(HJD_ERR_ARG, "hjd_batch_create", "HJD_FLAG_EXIF_ORIENT does not combine with HJD_FLAG_BMP_OUT (the BMP layout is "
+                                              "bottom-up with padded rows; the orientation pass writes top-down RGB24 or luma)");
+        return nullptr;                  // checked first: it does not depend on the device
+    }
     int n = hjd_device_count();
     if (n <= 0) { fail(HJD_ERR_CUDA, "hjd_batch_create", "no CUDA device available (this library has no CPU fallback)"); return nullptr; }
     if (device < 0 || device >= n) { fail(HJD_ERR_ARG, "hjd_batch_create", "bad device index"); return nullptr; }
@@ -265,7 +272,7 @@ static int ensure_slabs(hjd_batch* b)
     if (b->flags & HJD_FLAG_GRAY_OUT) CU(b->d_lumacta.ensure(sizeof(uint32_t) * (n + 2)));
     CU(b->d_istart.ensure(sizeof(uint32_t) * ((size_t)p.total_intervals + 2)));
     CU(b->d_coef.ensure(p.total_blocks * 128 + 256));
-    CU(b->d_rgb.ensure(p.rgb_bytes + 256));
+    CU(b->d_rgb.ensure(p.rgb_bytes + p.stage_bytes + 256));      // staging regions of oriented images behind the slab
     CU(b->d_status.ensure(sizeof(int32_t) * (n + 1)));
     if (b->flags & HJD_FLAG_KEEP_PLANES) CU(b->d_planes.ensure(p.plane_bytes + 256));
     if (!p.ss.empty()) {
@@ -286,6 +293,10 @@ static int ensure_slabs(hjd_batch* b)
         CU(b->d_mswork.ensure(sizeof(HjdMsWork) * p.mswork.size() + 16));
         CU(b->d_msstarts.ensure(sizeof(uint32_t) * p.ms_starts.size() + 16));
         CU(b->d_mstabs.ensure(sizeof(HjdHuffTable) * p.ms_tabs.size() + 16));
+    }
+    if (!p.orient_jobs.empty()) {
+        CU(b->d_ojobs.ensure(sizeof(HjdOrientJob) * p.orient_jobs.size()));
+        CU(b->d_otiles.ensure(sizeof(uint32_t) * p.orient_tiles.size()));
     }
     return HJD_OK;
 }
@@ -313,6 +324,8 @@ static int stage_plan(hjd_batch* b)
         {&b->d_mswork, p.mswork.data(), sizeof(HjdMsWork) * p.mswork.size()},
         {&b->d_msstarts, p.ms_starts.data(), sizeof(uint32_t) * p.ms_starts.size()},
         {&b->d_mstabs, p.ms_tabs.data(), sizeof(HjdHuffTable) * p.ms_tabs.size()},
+        {&b->d_ojobs, p.orient_jobs.data(), sizeof(HjdOrientJob) * p.orient_jobs.size()},
+        {&b->d_otiles, p.orient_tiles.data(), p.orient_jobs.empty() ? 0 : sizeof(uint32_t) * p.orient_tiles.size()},
     };
     size_t total = 0;
     for (const Stage& s : stages) total = align_up(total, 256) + s.bytes;
@@ -488,6 +501,18 @@ static int mcu_variant(unsigned flags, uint64_t blocks, uint32_t n_mcus, uint32_
     return (blocks >= 3ull * n_mcus && (uint64_t)n_mcus >= 1024ull * n_images && n_mcus >= 148u * 4u * 128u) ? HJD_MCU_TENSOR_CORE : HJD_MCU_CUDA_CORE;
 }
 
+// HJD_FLAG_EXIF_ORIENT: the orientation pass over the chunk's oriented images, from their staging regions to their
+// places in the slab, right after the kernel that wrote them (counted in that kernel's stage).
+static int launch_orient(hjd_batch* b, const Chunk& c, cudaStream_t st)
+{
+    if (c.oj1 <= c.oj0) return HJD_OK;
+    const std::vector<uint32_t>& tiles = b->plan.orient_tiles;
+    CU(hjd_launch_orient((uint8_t*)b->d_rgb.p, (const HjdOrientJob*)b->d_ojobs.p + c.oj0, (const uint32_t*)b->d_otiles.p + c.oj0,
+                         (int)(c.oj1 - c.oj0), tiles[c.oj1] - tiles[c.oj0], (b->flags & HJD_FLAG_GRAY_OUT) ? 1 : 3, st));
+    b->launches += 1;
+    return HJD_OK;
+}
+
 // Kernels of one chunk on one stream.  ev != nullptr: record stage boundaries (serial mode only).
 static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaStream_t st, cudaEvent_t* ev)
 {
@@ -540,6 +565,7 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
                 b->launches += 1;
             }
         }
+        if (int rc = launch_orient(b, c, st)) return rc;
         if (ev) CU(cudaEventRecord(ev[3], st));
     } else if (scale_shift(b->flags)) {
         // reduced-size decode: its own kernel in place of the fused one, counted in the same stage
@@ -550,6 +576,7 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
                                          b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0], c.max_mcus, scale_shift(b->flags), st));
             b->launches += 1;
         }
+        if (int rc = launch_orient(b, c, st)) return rc;
         if (ev) CU(cudaEventRecord(ev[3], st));
     } else if (!(b->flags & HJD_FLAG_KEEP_PLANES)) {
         // default: kernels 2+3 fused per MCU, planes never reach HBM
@@ -563,6 +590,7 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
                                   variant, st));
             b->launches += 1;
         }
+        if (int rc = launch_orient(b, c, st)) return rc;
         if (ev) CU(cudaEventRecord(ev[3], st));
     } else {
         if (c.blocks) {
@@ -575,6 +603,7 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
             CU(hjd_launch_color((const uint8_t*)b->d_planes.p, imgs + c.img0, (uint8_t*)b->d_rgb.p, n, c.max_w, c.max_h, st));
             b->launches += (n + 65534) / 65535;
         }
+        if (int rc = launch_orient(b, c, st)) return rc;       // the colour kernel writes the output here
     }
     return HJD_OK;
 }
@@ -694,7 +723,7 @@ extern "C" int hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* o)
     o->width = d.width; o->height = d.height; o->ncomp = d.ncomp; o->hf = d.hf; o->vf = d.vf;
     o->blocks_per_mcu = d.blocks_per_mcu; o->mcus_x = d.mcus_x; o->mcus_y = d.mcus_y;
     o->restart_interval = d.restart_interval; o->n_intervals = d.n_intervals; o->scan_bytes = d.scan_len;
-    o->block_base = d.block_base; o->n_blocks = d.n_blocks; o->rgb_offset = d.rgb_off;
+    o->block_base = d.block_base; o->n_blocks = d.n_blocks; o->rgb_offset = b->plan.out_off[i];
     o->y_offset = d.y_off; o->cb_offset = d.cb_off; o->cr_offset = d.cr_off;
     o->y_pitch = d.y_pitch; o->c_pitch = d.c_pitch; o->status = b->plan.parse_status[i];
     if (b->plan.ms_items[i]) o->n_intervals = b->plan.ms_items[i];
@@ -705,9 +734,17 @@ extern "C" int hjd_batch_get_out_size(const hjd_batch* b, int i, uint32_t* w, ui
 {
     if (!b || i < 0 || i >= (int)b->plan.imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_get_out_size", "bad arguments");
     const HjdImageDesc& d = b->plan.imgs[i];
-    if (w) *w = scaled_dim(b->flags, d.width);
-    if (h) *h = scaled_dim(b->flags, d.height);
+    uint32_t ow, oh;
+    out_size(b->flags, d.width, d.height, b->plan.orientation[i], &ow, &oh);
+    if (w) *w = ow;
+    if (h) *h = oh;
     return HJD_OK;
+}
+
+extern "C" int hjd_batch_get_orientation(const hjd_batch* b, int i)
+{
+    if (!b || i < 0 || i >= (int)b->plan.imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_get_orientation", "bad arguments");
+    return b->plan.orientation[i];
 }
 
 extern "C" int hjd_batch_num_scans(const hjd_batch* b, int i)
@@ -799,7 +836,7 @@ extern "C" int hjd_batch_download_image(hjd_batch* b, int i, uint8_t* dst)
     if (!b || i < 0 || i >= (int)b->plan.imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_download_image", "bad arguments");
     if (b->flags & HJD_FLAG_BMP_OUT) return fail(HJD_ERR_STATE, "hjd_batch_download_image", "this batch writes BMP files (HJD_FLAG_BMP_OUT): use hjd_batch_download_bmp");
     const HjdImageDesc& d = b->plan.imgs[i];
-    return download(b, dst, (const uint8_t*)b->d_rgb.p + d.rgb_off, image_out_bytes(b->flags, d.width, d.height),
+    return download(b, dst, (const uint8_t*)b->d_rgb.p + b->plan.out_off[i], image_out_bytes(b->flags, d.width, d.height),
                     "hjd_batch_download_image");
 }
 
@@ -814,8 +851,7 @@ extern "C" int hjd_batch_download_bmp(hjd_batch* b, int i, uint8_t* dst)
 {
     if (!b || i < 0 || i >= (int)b->plan.imgs.size()) return fail(HJD_ERR_ARG, "hjd_batch_download_bmp", "bad arguments");
     if (!(b->flags & HJD_FLAG_BMP_OUT)) return fail(HJD_ERR_STATE, "hjd_batch_download_bmp", "batch was not created with HJD_FLAG_BMP_OUT");
-    const HjdImageDesc& d = b->plan.imgs[i];
-    return download(b, dst, (const uint8_t*)b->d_rgb.p + d.rgb_off + 10, hjd_batch_bmp_bytes(b, i), "hjd_batch_download_bmp");
+    return download(b, dst, (const uint8_t*)b->d_rgb.p + b->plan.out_off[i] + 10, hjd_batch_bmp_bytes(b, i), "hjd_batch_download_bmp");
 }
 
 extern "C" int hjd_batch_download_coef(hjd_batch* b, int16_t* dst)
@@ -873,7 +909,7 @@ extern "C" int hjd_batch_decode_host(hjd_batch* b, const uint8_t* arena, const i
     if (rc) return rc;
     b->decoded = true;
     if (rgb_offsets_out)
-        for (int i = 0; i < n; i++) rgb_offsets_out[i] = b->plan.imgs[i].rgb_off;
+        for (int i = 0; i < n; i++) rgb_offsets_out[i] = b->plan.out_off[i];
     if (status_out) { rc = hjd_batch_get_status(b, status_out); if (rc) return rc; }
     CU(cudaStreamSynchronize(b->stream));
     return HJD_OK;
@@ -1073,6 +1109,17 @@ extern "C" int hjd_probe_jpeg_flags(const uint8_t* buf, int64_t size, unsigned f
     return f.status;
 }
 
+extern "C" int hjd_probe_jpeg_orientation(const uint8_t* buf, int64_t size)
+{
+    if (!buf || size < 2 || buf[0] != 0xFF || buf[1] != 0xD8) return HJD_IMG_ERR_NOT_JPEG;
+    HjdParsed ps;
+    if (hjd_parse_jpeg(buf, (size_t)size, &ps) != HJD_IMG_ERR_UNSUPPORTED) return ps.orientation;
+    // e.g. a progressive file: the multi-scan walk, which does not stop at its SOF2, reads the Exif APP1 wherever it is
+    std::unique_ptr<HjdMultiParsed> mp(new HjdMultiParsed());
+    hjd_parse_jpeg_multi(buf, (size_t)size, mp.get());
+    return mp->frame.orientation;
+}
+
 extern "C" int hjd_probe_jpeg_scans(const uint8_t* buf, int64_t size, hjd_scan_info* out, int max)
 {
     if (max < 0 || (max > 0 && !out)) return fail(HJD_ERR_ARG, "hjd_probe_jpeg_scans", "bad arguments");
@@ -1145,7 +1192,7 @@ static int decode_one(bool bmp, const uint8_t* buf, int size, void* (*alloc)(siz
     const HjdImageDesc& d = b->plan.imgs[0];
     const size_t bytes = bmp ? (size_t)hjd_batch_bmp_bytes(b, 0) : (size_t)d.width * d.height * 3;
     if (cudaSetDevice(b->device) != cudaSuccess || b->h_out.ensure(bytes + 16) != cudaSuccess) { cudaGetLastError(); fail(HJD_ERR_NOMEM, who, "pinned staging buffer"); return 0; }
-    if (cudaMemcpyAsync(b->h_out.p, (const uint8_t*)b->d_rgb.p + d.rgb_off + (bmp ? 10 : 0), bytes, cudaMemcpyDeviceToHost, b->stream) != cudaSuccess ||
+    if (cudaMemcpyAsync(b->h_out.p, (const uint8_t*)b->d_rgb.p + b->plan.out_off[0] + (bmp ? 10 : 0), bytes, cudaMemcpyDeviceToHost, b->stream) != cudaSuccess ||
         cudaStreamSynchronize(b->stream) != cudaSuccess) { fail(HJD_ERR_CUDA, who, cudaGetErrorString(cudaGetLastError())); return 0; }
     uint8_t* out = (uint8_t*)alloc(bytes ? bytes : 1);
     if (!out) { fail(HJD_ERR_NOMEM, who, "allocation failed"); return 0; }

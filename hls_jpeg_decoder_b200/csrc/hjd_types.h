@@ -188,6 +188,17 @@ struct HjdMsWork {
     uint32_t interval;
 };
 
+// ---- EXIF orientation (HJD_FLAG_EXIF_ORIENT, csrc/orient.cu) -----------------------------------
+// One oriented image: the output kernel wrote its decoded w x h pixels at src_off (a private staging region of the
+// output slab); the orientation pass writes them turned by EXIF orientation o (2..8) at dst_off, the image's place in
+// the output slab.  Offsets in bytes of the output slab.
+struct HjdOrientJob {
+    uint64_t src_off, dst_off;
+    uint32_t w, h;               // decoded size (scaled with HJD_FLAG_SCALE_*), before orientation
+    uint32_t o, pad;
+};
+#define HJD_ORIENT_TILE 64       // the orientation pass writes output tiles of HJD_ORIENT_TILE^2 pixels, one per CTA
+
 // Per-image status bits written by kernels (mirrors HJD_IMG_WARN_* in include/hjd.h).
 #define HJD_ST_BAD_CODE     1
 #define HJD_ST_COEF_RANGE   2

@@ -59,6 +59,32 @@ int parse_dht(Reader& r, size_t end, HjdParsed* o)
 
 } // namespace
 
+int hjd_exif_orientation(const uint8_t* p, size_t len)
+{
+    if (len < 6 || memcmp(p, "Exif\0\0", 6) != 0) return 0;
+    const uint8_t* t = p + 6;                      // TIFF header; its offsets are relative to here
+    const uint64_t n = len - 6;
+    if (n < 8) return 1;
+    bool le;
+    if (t[0] == 'I' && t[1] == 'I' && t[2] == 0x2A && t[3] == 0) le = true;
+    else if (t[0] == 'M' && t[1] == 'M' && t[2] == 0 && t[3] == 0x2A) le = false;
+    else return 1;
+    auto u16 = [&](uint64_t at) { return (uint32_t)(le ? t[at] | t[at + 1] << 8 : t[at] << 8 | t[at + 1]); };
+    auto u32 = [&](uint64_t at) { return le ? u16(at) | u16(at + 2) << 16 : u16(at) << 16 | u16(at + 2); };
+    const uint64_t ifd = u32(4);
+    if (ifd + 2 > n) return 1;
+    const uint64_t count = u16(ifd);
+    if (ifd + 2 + 12 * count > n) return 1;        // 64-bit: no overflow
+    for (uint64_t k = 0; k < count; k++) {
+        const uint64_t e = ifd + 2 + 12 * k;
+        if (u16(e) != 0x0112) continue;
+        if (u16(e + 2) != 3 || u32(e + 4) != 1) return 1;    // SHORT, count 1: the value sits in the first two bytes
+        const uint32_t v = u16(e + 8);
+        return v >= 1 && v <= 8 ? (int)v : 1;
+    }
+    return 1;
+}
+
 size_t hjd_scan_length(const uint8_t* scan, size_t avail)
 {
     // Large file that ends with EOI: taken as "nothing follows the scan" without walking it (a memchr walk
@@ -86,9 +112,10 @@ int hjd_parse_jpeg(const uint8_t* buf, size_t size, HjdParsed* o)
 {
     memset(o, 0, sizeof *o);
     o->status = HJD_IMG_ERR_NOT_JPEG;
+    o->orientation = 1;
     if (!buf || size < 4 || buf[0] != 0xFF || buf[1] != 0xD8) return o->status;   // openjpg.cpp:481
     Reader r{buf, size, 2};
-    bool have_frame = false;
+    bool have_frame = false, have_exif = false;
     int cid[3] = {0, 0, 0};
     int chf[3] = {1, 1, 1}, cvf[3] = {1, 1, 1};
 
@@ -159,6 +186,9 @@ int hjd_parse_jpeg(const uint8_t* buf, size_t size, HjdParsed* o)
             o->scan_off = end;
             o->scan_len = hjd_scan_length(buf + end, size - end);
             break;
+        } else if (m == 0xE1 && !have_exif) {
+            const int v = hjd_exif_orientation(buf + r.i, end - r.i);
+            if (v) { o->orientation = v; have_exif = true; }
         }
         // APPn, COM and anything else with a length: skipped (openjpg.cpp:448-461)
         r.i = end;
@@ -207,9 +237,10 @@ int hjd_parse_jpeg_multi(const uint8_t* buf, size_t size, HjdMultiParsed* mp)
     mp->scans.clear();
     mp->starts.clear();
     o->status = HJD_IMG_ERR_NOT_JPEG;
+    o->orientation = 1;
     if (!buf || size < 4 || buf[0] != 0xFF || buf[1] != 0xD8) return o->status;
     Reader r{buf, size, 2};
-    bool have_frame = false, progressive = false;
+    bool have_frame = false, progressive = false, have_exif = false;
     int cid[3] = {0, 0, 0};
     int chf[3] = {1, 1, 1}, cvf[3] = {1, 1, 1};
     uint32_t dri = 0;
@@ -342,6 +373,9 @@ int hjd_parse_jpeg_multi(const uint8_t* buf, size_t size, HjdMultiParsed* mp)
             mp->scans.push_back(s);
             r.i = end + s.len;
             continue;
+        } else if (m == 0xE1 && !have_exif && mp->scans.empty()) {
+            const int v = hjd_exif_orientation(buf + r.i, end - r.i);
+            if (v) { o->orientation = v; have_exif = true; }
         }
         r.i = end;
     }

@@ -30,10 +30,17 @@ struct HjdParsed {
     uint32_t restart_interval;
     size_t   scan_off;           // offset of the first entropy-coded byte in the file
     size_t   scan_len;
+    int      orientation;        // EXIF orientation 1..8 (1: none, or malformed; see hjd_exif_orientation)
 };
 
 // Header parse only (no table building).  Returns HJD_IMG_OK or a negative HJD_IMG_ERR_*.
 int hjd_parse_jpeg(const uint8_t* buf, size_t size, HjdParsed* out);
+
+// EXIF orientation of one APP1 payload (the bytes after the segment's length field, `len` of them): 0 when the payload
+// does not start with "Exif\0\0" (not an Exif segment), else the value of IFD0's tag 0x0112 (type SHORT, count 1) in
+// 1..8, or 1 when the TIFF structure is malformed, reaches past the payload, or has no such entry in IFD0.  Every read
+// is bounded by `len`; no other IFD is followed.  Both marker walks take the first Exif APP1 before the first SOS.
+int hjd_exif_orientation(const uint8_t* payload, size_t len);
 
 // ---- multi-scan files (HJD_FLAG_MULTI_SCAN): progressive SOF2 and sequential files with several scans ----
 struct HjdScanParsed {

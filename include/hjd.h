@@ -113,6 +113,26 @@ extern "C" {
  * HJD_FLAG_KEEP_PLANES (the planes already hold Y), HJD_FLAG_TENSOR_CORE_IDCT and HJD_FLAG_CUDA_CORE_IDCT (they select
  * RGB kernels). */
 #define HJD_FLAG_GRAY_OUT    (1u << 11)
+/* Apply each image's EXIF orientation to its decoded output (torchvision's apply_exif_orientation, PIL.ImageOps.
+ * exif_transpose).  The orientation o is read from the first APP1 segment before the first SOS whose payload starts
+ * with "Exif\0\0": the TIFF header after those 6 bytes ("II*\0" or "MM\0*", then the 32-bit offset of IFD0, relative
+ * to the header), and in IFD0 (16-bit entry count, 12-byte entries tag, type, count, value) the entry with tag 0x0112,
+ * type SHORT (3) and count 1: the first two bytes of its value field, in the file's byte order.  In every other case
+ * o = 1: no Exif APP1 before the first SOS; an offset, count or entry reaching past the segment; another type or
+ * count; a value outside 1..8; the tag only in another IFD (ExifIFD, IFD1).  A malformed tag is never an error.
+ * With the decoded output W' x H' (the source size, or ceil(W/d) x ceil(H/d) with HJD_FLAG_SCALE_1_d) and bpp bytes
+ * per pixel (3, or 1 with HJD_FLAG_GRAY_OUT), output pixel out(x, y) is, by o (EXIF 2.3 / TIFF 6.0):
+ *   1 as stored             W' x H'  in(x, y)              5 transpose          H' x W'  in(y, x)
+ *   2 mirror horizontally   W' x H'  in(W'-1-x, y)         6 rotate 90 cw       H' x W'  in(y, H'-1-x)
+ *   3 rotate 180            W' x H'  in(W'-1-x, H'-1-y)    7 transverse         H' x W'  in(W'-1-y, H'-1-x)
+ *   4 mirror vertically     W' x H'  in(x, H'-1-y)         8 rotate 90 ccw      H' x W'  in(W'-1-y, x)
+ * Each image keeps its region of the slab (same rgb_offset, 256-byte alignment, hjd_batch_rgb_bytes and
+ * hjd_out_slab_bytes); its rows are top-down with stride out_w * bpp, and hjd_batch_get_out_size returns the oriented
+ * size.  hjd_image_info and hjd_batch_pixels keep describing the source.  Without the flag nothing changes, also for
+ * files that carry a tag.  Combines with every flag but HJD_FLAG_BMP_OUT (hjd_batch_create fails with HJD_ERR_ARG);
+ * with HJD_FLAG_KEEP_PLANES the planes stay as stored and only the RGB slab is oriented.  hjd_batch_decode_host and
+ * the hjd_multi_* calls follow the handle's flags.  The single-image calls and the file converter do not orient. */
+#define HJD_FLAG_EXIF_ORIENT (1u << 12)
 
 typedef struct hjd_batch hjd_batch;
 
@@ -184,6 +204,9 @@ typedef struct hjd_scan_info {
     uint32_t restart_interval, bytes;
 } hjd_scan_info;
 int  hjd_probe_jpeg_scans(const uint8_t* buf, int64_t size, hjd_scan_info* out, int max);
+/* The EXIF orientation (1..8) the file states, by the rule of HJD_FLAG_EXIF_ORIENT (header parse only, no GPU);
+ * HJD_IMG_ERR_NOT_JPEG when the buffer does not start with SOI. */
+int  hjd_probe_jpeg_orientation(const uint8_t* buf, int64_t size);
 /* openjpg.cpp:504 WriteBMP24. */
 int  hjd_write_bmp24(const char* path, unsigned width, unsigned height, const uint8_t* rgb);
 /* Same bytes as hjd_write_bmp24 into memory; returns the BMP size (call with out = NULL to size it). */
@@ -243,8 +266,11 @@ int  hjd_batch_num_scans(const hjd_batch* b, int i);
 /* hjd_image_info describes the source image (width, height: its frame). */
 int  hjd_batch_get_info(const hjd_batch* b, int i, hjd_image_info* out);
 /* Dimensions of image i's decoded output: width x height, or ceil(width/d) x ceil(height/d) with HJD_FLAG_SCALE_1_d
- * (the same with HJD_FLAG_GRAY_OUT). */
+ * (the same with HJD_FLAG_GRAY_OUT); with HJD_FLAG_EXIF_ORIENT and orientation 5..8, width and height swapped. */
 int  hjd_batch_get_out_size(const hjd_batch* b, int i, uint32_t* w, uint32_t* h);
+/* The EXIF orientation (1..8) image i's file states, with or without HJD_FLAG_EXIF_ORIENT (which decides only whether
+ * it is applied); negative (HJD_ERR_ARG) for a bad index. */
+int  hjd_batch_get_orientation(const hjd_batch* b, int i);
 int  hjd_batch_get_status(hjd_batch* b, int32_t* status /* n */);   /* syncs */
 int  hjd_batch_get_timings(hjd_batch* b, hjd_timings* out);          /* syncs */
 /* CUDA-event stopwatch on the batch stream: record event `slot` (0..HJD_MARK_SLOTS-1); milliseconds
