@@ -548,47 +548,31 @@ static int launch_chunk(hjd_batch* b, const Chunk& c, size_t chunk_index, cudaSt
         b->launches += 1;
     }
     if (ev) CU(cudaEventRecord(ev[2], st));
-    if (b->flags & HJD_FLAG_GRAY_OUT) {
-        // luma-only decode (full size or scaled): its own kernel in place of the fused one, counted in the same stage
+    if (!(b->flags & HJD_FLAG_KEEP_PLANES)) {
+        // one output kernel in place of kernels 2+3, planes never reach HBM: luma-only (HJD_FLAG_GRAY_OUT) and reduced-size
+        // (HJD_FLAG_SCALE_*) decodes have their own, the default is the fused kernel on the CUDA or the tensor cores
         if (c.blocks) {
-            b->gy_chunks++;
-            if (scale_shift(b->flags)) {
+            const int16_t* coef = (const int16_t*)b->d_coef.p;
+            const HjdQuantSet* qsets = (const HjdQuantSet*)b->d_qsets.p;
+            uint8_t* out = (uint8_t*)b->d_rgb.p;
+            const uint32_t* mcu_prefix = (const uint32_t*)b->d_mcucta.p + c.img0;
+            const uint32_t n_mcus = b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0];
+            const bool gray = (b->flags & HJD_FLAG_GRAY_OUT) != 0;
+            const int shift = scale_shift(b->flags);
+            if (gray) b->gy_chunks++;
+            if (shift) {
                 b->sc_chunks++;
-                CU(hjd_launch_luma_scaled((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
-                                          (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_mcucta.p + c.img0, n,
-                                          b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0], c.max_mcus, scale_shift(b->flags), st));
-                b->launches += 1;
-            } else {
-                CU(hjd_launch_luma((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
-                                   (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_lumacta.p + c.img0, n,
+                CU(hjd_launch_scaled(coef, imgs + c.img0, qsets, out, mcu_prefix, n, n_mcus, c.max_mcus, shift, gray, st));
+            } else if (gray) {
+                CU(hjd_launch_luma(coef, imgs + c.img0, qsets, out, (const uint32_t*)b->d_lumacta.p + c.img0, n,
                                    b->plan.luma_cta[c.img1] - b->plan.luma_cta[c.img0], c.max_luma, st));
-                b->launches += 1;
+            } else {
+                const int variant = mcu_variant(b->flags, c.blocks, n_mcus, (uint32_t)n);
+                if (variant == HJD_MCU_TENSOR_CORE) b->tc_chunks++; else b->cc_chunks++;
+                CU(hjd_launch_mcu_rgb(coef, imgs + c.img0, qsets, out, mcu_prefix, n, n_mcus, c.max_mcus,
+                                      (b->flags & HJD_FLAG_BMP_OUT) != 0, variant, st));
             }
-        }
-        if (int rc = launch_orient(b, c, st)) return rc;
-        if (ev) CU(cudaEventRecord(ev[3], st));
-    } else if (scale_shift(b->flags)) {
-        // reduced-size decode: its own kernel in place of the fused one, counted in the same stage
-        if (c.blocks) {
-            b->sc_chunks++;
-            CU(hjd_launch_mcu_rgb_scaled((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
-                                         (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_mcucta.p + c.img0, n,
-                                         b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0], c.max_mcus, scale_shift(b->flags), st));
-            b->launches += 1;
-        }
-        if (int rc = launch_orient(b, c, st)) return rc;
-        if (ev) CU(cudaEventRecord(ev[3], st));
-    } else if (!(b->flags & HJD_FLAG_KEEP_PLANES)) {
-        // default: kernels 2+3 fused per MCU, planes never reach HBM
-        if (c.blocks) {
-            const uint32_t n_mcus_chunk = b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0];
-            const int variant = mcu_variant(b->flags, c.blocks, n_mcus_chunk, (uint32_t)n);
-            if (variant == HJD_MCU_TENSOR_CORE) b->tc_chunks++; else b->cc_chunks++;
-            CU(hjd_launch_mcu_rgb((const int16_t*)b->d_coef.p, imgs + c.img0, (const HjdQuantSet*)b->d_qsets.p,
-                                  (uint8_t*)b->d_rgb.p, (const uint32_t*)b->d_mcucta.p + c.img0, n,
-                                  b->plan.mcu_cta[c.img1] - b->plan.mcu_cta[c.img0], c.max_mcus, (b->flags & HJD_FLAG_BMP_OUT) != 0,
-                                  variant, st));
-            b->launches += 1;
+            b->launches += 1;       // one even where the (image, CTA) grid takes several launches of 65,535 images
         }
         if (int rc = launch_orient(b, c, st)) return rc;
         if (ev) CU(cudaEventRecord(ev[3], st));

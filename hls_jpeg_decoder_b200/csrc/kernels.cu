@@ -992,29 +992,11 @@ hjd_k_mcu_rgb(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__
     if (t < 64) s_cos[t] = c_cos[t];
     __syncthreads();
 
-    // Two grid shapes (two instantiations: the kernel sits at the 128-register cap, and a run-time switch
-    // cost 2 %).  Images of similar size: blockIdx.y = image, blockIdx.x = its CTA (no look-up).
-    // Mixed or tiny sizes (FLAT): a 1-D grid over ALL MCUs of the batch, the image of each thread found by
-    // binary search in mcu_prefix[i] = MCUs of the images before i.  The 2-D grid is sized for the largest
-    // image and launched 2 M empty CTAs for one 4096x4096 image among 4096 thumbnails (2.2 ms instead of
-    // 0.6), and gives a 16x16 image a CTA with one active thread; the search costs similar-sized batches
-    // 4 % (a chain of dependent loads in front of every CTA), an empty CTA next to nothing.
+    // Two grid shapes (device_common.cuh), two instantiations: the kernel sits at the 128-register cap, and a
+    // run-time switch cost 2 %.
     const HjdImageDesc* d;
     uint32_t m;
-    if (FLAT) {
-        const uint32_t key = blockIdx.x * HJD_MCU_THREADS + t + mcu_prefix[0];
-        if (key >= mcu_prefix[n_images]) return;
-        int lo = 0, hi = n_images - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (mcu_prefix[mid] <= key) lo = mid; else hi = mid - 1;
-        }
-        d = imgs + lo;
-        m = key - mcu_prefix[lo];
-    } else {
-        d = imgs + (blockIdx.y + img_base);
-        m = blockIdx.x * HJD_MCU_THREADS + t;
-    }
+    if (!hjd_locate<FLAT, HJD_MCU_THREADS>(imgs, mcu_prefix, n_images, img_base, d, m)) return;
     if (m >= d->n_mcus || d->blocks_per_mcu == 0) return;
     const uint32_t hf = d->hf, vf = d->vf, bpm = d->blocks_per_mcu;
     const bool gray = d->ncomp == 1;
@@ -1121,7 +1103,7 @@ hjd_k_mcu_rgb(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__
 // contiguous bytes.  Chroma blocks and MCU-padding blocks are not read.  hjd_idct_block, unchanged, writes the
 // block into a thread-private shared-memory tile interleaved by thread (as hjd_k_mcu_rgb does), where the exact
 // re-evaluation patches its bytes; then the rows go out clipped at W and H, 8 bytes at once where aligned.
-// Grids as hjd_k_mcu_rgb (FLAT: a 1-D grid over all luma blocks of the batch, the image found by binary search).
+// Grids as hjd_k_mcu_rgb, over luma blocks instead of MCUs.
 template <bool FLAT>
 __global__ void __launch_bounds__(HJD_LUMA_THREADS, HJD_MCU_MINBLOCKS)
 hjd_k_luma(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ imgs,
@@ -1136,20 +1118,7 @@ hjd_k_luma(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ im
 
     const HjdImageDesc* d;
     uint32_t k;
-    if (FLAT) {
-        const uint32_t key = blockIdx.x * HJD_LUMA_THREADS + t + luma_prefix[0];
-        if (key >= luma_prefix[n_images]) return;
-        int lo = 0, hi = n_images - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (luma_prefix[mid] <= key) lo = mid; else hi = mid - 1;
-        }
-        d = imgs + lo;
-        k = key - luma_prefix[lo];
-    } else {
-        d = imgs + (blockIdx.y + img_base);
-        k = blockIdx.x * HJD_LUMA_THREADS + t;
-    }
+    if (!hjd_locate<FLAT, HJD_LUMA_THREADS>(imgs, luma_prefix, n_images, img_base, d, k)) return;
     const uint32_t W = d->width, H = d->height;
     const uint32_t bw = (W + 7) >> 3;
     if (d->blocks_per_mcu == 0 || k >= bw * ((H + 7) >> 3)) return;
@@ -1183,16 +1152,8 @@ cudaError_t hjd_launch_luma(const int16_t* coef, const HjdImageDesc* imgs, const
                             const uint32_t* luma_prefix, int n_images, uint32_t n_luma, uint32_t max_luma, cudaStream_t st)
 {
     if (n_images <= 0 || n_luma == 0 || max_luma == 0) return cudaSuccess;
-    const unsigned gx = (max_luma + HJD_LUMA_THREADS - 1) / HJD_LUMA_THREADS;
-    if ((uint64_t)gx * HJD_LUMA_THREADS * (uint64_t)n_images <= (uint64_t)n_luma * 4) {   // the rule of hjd_launch_mcu_rgb
-        for (int base = 0; base < n_images; base += 65535) {
-            const int n = min(65535, n_images - base);
-            hjd_k_luma<false><<<dim3(gx, n), HJD_LUMA_THREADS, 0, st>>>(coef, imgs, qsets, out, nullptr, n_images, base);
-        }
-    } else {
-        const unsigned g = (unsigned)(((uint64_t)n_luma + HJD_LUMA_THREADS - 1) / HJD_LUMA_THREADS);
-        hjd_k_luma<true><<<g, HJD_LUMA_THREADS, 0, st>>>(coef, imgs, qsets, out, luma_prefix, n_images, 0);
-    }
+    hjd_launch_per_image(hjd_k_luma<false>, hjd_k_luma<true>, HJD_LUMA_THREADS, luma_prefix, n_images, n_luma, max_luma, st,
+                         coef, imgs, qsets, out);
     return cudaGetLastError();
 }
 
@@ -1240,10 +1201,10 @@ cudaError_t hjd_launch_mcu_rgb(const int16_t* coef, const HjdImageDesc* imgs, co
     if (variant == HJD_MCU_TENSOR_CORE) {
         // units of 128 MCUs, walked by the groups of one resident CTA per SM.  Images of similar size: unit = (image, 128 MCUs of it),
         // no look-up; clearly skewed or tiny-image batches: units over all MCUs of the batch, the image found by binary search
-        // (an idle thread slot is cheap, a search in front of every unit is not: the same rule as for the CUDA-core kernel below).
+        // (an idle thread slot is cheap, a search in front of every unit is not: the rule of the CUDA-core kernel, over units).
         uint32_t units_x = (max_mcus + 127u) / 128u;
         uint64_t n_units = (uint64_t)units_x * (uint64_t)n_images;
-        if (n_units * 128u > (uint64_t)n_mcus * 4 || n_units > 0xFFFFFFFFull) { units_x = 0; n_units = ((uint64_t)n_mcus + 127u) / 128u; }
+        if (!hjd_grid_per_image(max_mcus, n_images, n_mcus, 128u) || n_units > 0xFFFFFFFFull) { units_x = 0; n_units = ((uint64_t)n_mcus + 127u) / 128u; }
         int dev = 0;
         cudaError_t e = cudaGetDevice(&dev);
         if (e != cudaSuccess) return e;
@@ -1253,20 +1214,12 @@ cudaError_t hjd_launch_mcu_rgb(const int16_t* coef, const HjdImageDesc* imgs, co
         else hjd_k_mcu_rgb_tc<false><<<g, HJD_TC_THREADS, HJD_TC_SMEM_BYTES, st>>>(coef, imgs, qsets, rgb, mcu_prefix, n_images, (uint32_t)n_units, units_x);
         return cudaGetLastError();
     }
-    const unsigned gx = (max_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS;
-    // thread slots of the 2-D grid against MCUs there are: an idle slot is cheap (config 5 runs at 1.6 x:
-    // 1.02 ms against 1.11 ms with the search), so only clearly skewed or tiny-image batches go flat
-    if ((uint64_t)gx * HJD_MCU_THREADS * (uint64_t)n_images <= (uint64_t)n_mcus * 4) {
-        for (int base = 0; base < n_images; base += 65535) {
-            const int n = min(65535, n_images - base);
-            if (bmp) hjd_k_mcu_rgb<false, true><<<dim3(gx, n), HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, rgb, nullptr, n_images, base);
-            else hjd_k_mcu_rgb<false, false><<<dim3(gx, n), HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, rgb, nullptr, n_images, base);
-        }
-    } else {
-        const unsigned g = (unsigned)(((uint64_t)n_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS);
-        if (bmp) hjd_k_mcu_rgb<true, true><<<g, HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, rgb, mcu_prefix, n_images, 0);
-        else hjd_k_mcu_rgb<true, false><<<g, HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, rgb, mcu_prefix, n_images, 0);
-    }
+    if (bmp)
+        hjd_launch_per_image(hjd_k_mcu_rgb<false, true>, hjd_k_mcu_rgb<true, true>, HJD_MCU_THREADS, mcu_prefix, n_images,
+                             n_mcus, max_mcus, st, coef, imgs, qsets, rgb);
+    else
+        hjd_launch_per_image(hjd_k_mcu_rgb<false, false>, hjd_k_mcu_rgb<true, false>, HJD_MCU_THREADS, mcu_prefix, n_images,
+                             n_mcus, max_mcus, st, coef, imgs, qsets, rgb);
     return cudaGetLastError();
 }
 

@@ -39,10 +39,16 @@ cudaError_t hjd_launch_idct_planes(const int16_t* coef, const HjdImageDesc* imgs
 cudaError_t hjd_launch_color(const uint8_t* planes, const HjdImageDesc* imgs, uint8_t* rgb, int n_images,
                              uint32_t max_width, uint32_t max_height, cudaStream_t st);
 
+// Per-image output kernels (hjd_launch_mcu_rgb, hjd_launch_luma, hjd_launch_scaled in scaled.cuh): one thread per item of
+// an image (an MCU or a luma block), taking the items through three arguments:
+//   prefix[i] = items of images 0..i-1 (any common offset; n_images + 1 entries);
+//   n_items   = prefix[n_images] - prefix[0];
+//   max_items = items of the largest image.
+// Batches of similar-sized images get an (image, CTA) grid, mixed or tiny sizes a flat grid over all items
+// (device_common.cuh).
+
 // Kernels 2+3 fused per MCU (default path): one thread = one MCU, coefficients -> RGB, no plane traffic, no barriers.
-// mcu_prefix[i] = MCUs of images 0..i-1 (any common offset; n_images + 1 entries);
-// n_mcus = mcu_prefix[n_images] - mcu_prefix[0]; max_mcus = MCUs of the largest image.  Batches of
-// similar-sized images get an (image, CTA) grid, mixed or tiny sizes a flat grid over all MCUs (see the kernel).
+// A per-image output kernel over MCUs (mcu_prefix, n_mcus, max_mcus).
 // bmp: write the reference's BMP file layout (header at rgb_off + 10, bottom-up B G R rows from rgb_off + 64).
 // variant: where the IDCT's fast tier runs and who re-evaluates the flagged samples; same bytes out.
 #define HJD_MCU_CUDA_CORE    0   // FP32 FMA chains on the CUDA cores, every thread re-evaluates its own flagged samples (default)
@@ -53,9 +59,8 @@ cudaError_t hjd_launch_mcu_rgb(const int16_t* coef, const HjdImageDesc* imgs, co
 
 // Luma-only decode at full size (HJD_FLAG_GRAY_OUT): one thread = one luma block that holds a pixel of its image
 // (ceil(W/8) x ceil(H/8) of them, row-major), the IDCT of the fused kernel, rows clipped at W and H; image i is
-// written at imgs[i].rgb_off as W x H bytes, stride W.  Chroma blocks are not read.  luma_prefix[i] = those blocks
-// of images 0..i-1 (any common offset; n_images + 1 entries); n_luma = luma_prefix[n_images] - luma_prefix[0];
-// max_luma = blocks of the largest image.  The grid choice of hjd_launch_mcu_rgb, over blocks instead of MCUs.
+// written at imgs[i].rgb_off as W x H bytes, stride W.  Chroma blocks are not read.  A per-image output kernel over
+// those luma blocks (luma_prefix, n_luma, max_luma).
 #define HJD_LUMA_THREADS 128
 cudaError_t hjd_launch_luma(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
                             const uint32_t* luma_prefix, int n_images, uint32_t n_luma, uint32_t max_luma, cudaStream_t st);

@@ -251,13 +251,9 @@ hjd_k_mcu_rgb_tc(const int16_t* __restrict__ coef, const HjdImageDesc* __restric
             const uint32_t key = unit * 128u + tg + mcu_prefix[0];
             if (key >= mcu_prefix[n_images]) valid = false;
             else {
-                int lo = 0, hi = n_images - 1;
-                while (lo < hi) {
-                    const int mid = (lo + hi + 1) >> 1;
-                    if (mcu_prefix[mid] <= key) lo = mid; else hi = mid - 1;
-                }
-                d = imgs + lo;
-                m = key - mcu_prefix[lo];
+                const int i = hjd_image_of(mcu_prefix, n_images, key);
+                d = imgs + i;
+                m = key - mcu_prefix[i];
             }
         } else {
             const uint32_t img = unit / units_x;

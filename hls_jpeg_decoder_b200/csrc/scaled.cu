@@ -8,6 +8,7 @@
 // so the bytes are exactly those the definition in include/hjd.h gives.
 #include "scaled.cuh"
 #include "kernels.cuh"
+#include "device_common.cuh"
 #include <cuda_runtime.h>
 
 static __constant__ float c_sc_cos4[16];   // cos4[p * 4 + k] = cosf(((2p+1) * k * 3.14f) / 8)
@@ -122,131 +123,49 @@ __device__ __forceinline__ void sc_ycc(int y, int cb, int cr, int* o)
     o[2] = min(max(b, 0), 255);
 }
 
-// One thread = one MCU, as hjd_k_mcu_rgb (kernels.cu), with its two grid shapes (FLAT: a 1-D grid over all MCUs of the
-// batch, the image found by binary search in mcu_prefix).  Consecutive threads take consecutive MCUs of a row, so the
-// row segments a warp stores are adjacent.  The chroma tiles (N x N each) go to a thread-private shared-memory region
-// (an odd number of words per thread: no bank conflicts); each luma block is converted and stored as soon as its
-// IDCT is done.
-template <int N, bool FLAT>
+// One thread = one MCU, as hjd_k_mcu_rgb (kernels.cu), with its two grid shapes (device_common.cuh).  Consecutive
+// threads take consecutive MCUs of a row, so the row segments a warp stores are adjacent.  Each luma block is stored as
+// soon as its IDCT is done.  RGB: the chroma tiles (N x N each) go to a thread-private shared-memory region (an odd
+// number of words per thread: no bank conflicts), and the luma samples are converted with them.  GRAY
+// (HJD_FLAG_GRAY_OUT): no chroma IDCT, no colour conversion and no shared memory; the luma samples are stored as they
+// are, one byte per pixel.
+template <int N, bool GRAY, bool FLAT>
 __global__ void __launch_bounds__(HJD_MCU_THREADS)
-hjd_k_mcu_rgb_scaled(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ imgs,
-                     const HjdQuantSet* __restrict__ qsets, uint8_t* __restrict__ rgb,
-                     const uint32_t* __restrict__ mcu_prefix, int n_images, int img_base)
+hjd_k_mcu_scaled(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ imgs,
+                 const HjdQuantSet* __restrict__ qsets, uint8_t* __restrict__ out,
+                 const uint32_t* __restrict__ mcu_prefix, int n_images, int img_base)
 {
     constexpr uint32_t D = 8 / N;                       // scale denominator
-    constexpr int CW = (N * N + 3) / 4;                 // words of one chroma tile
-    constexpr int S = (2 * CW) | 1;                     // words per thread
-    __shared__ uint32_t s_c[S * HJD_MCU_THREADS];
-    const uint32_t t = threadIdx.x;
+    constexpr int C = GRAY ? 1 : 3;                     // bytes per output pixel
     const HjdImageDesc* d;
     uint32_t m;
-    if (FLAT) {
-        const uint32_t key = blockIdx.x * HJD_MCU_THREADS + t + mcu_prefix[0];
-        if (key >= mcu_prefix[n_images]) return;
-        int lo = 0, hi = n_images - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (mcu_prefix[mid] <= key) lo = mid; else hi = mid - 1;
-        }
-        d = imgs + lo;
-        m = key - mcu_prefix[lo];
-    } else {
-        d = imgs + (blockIdx.y + img_base);
-        m = blockIdx.x * HJD_MCU_THREADS + t;
-    }
+    if (!hjd_locate<FLAT, HJD_MCU_THREADS>(imgs, mcu_prefix, n_images, img_base, d, m)) return;
     if (m >= d->n_mcus || d->blocks_per_mcu == 0) return;
     const uint32_t hf = d->hf, vf = d->vf, bpm = d->blocks_per_mcu;
-    const bool gray = d->ncomp == 1;
-    const uint32_t ny = gray ? 1u : hf * vf;
+    const bool mono = d->ncomp == 1;                    // one-component file
+    const uint32_t ny = mono ? 1u : hf * vf;
     const uint32_t my = m / d->mcus_x, mx = m - my * d->mcus_x;
     const int hs = (int)hf - 1, vs = (int)vf - 1;
     const HjdQuantSet* qs = qsets + d->quant_set;
     const int16_t* cp = coef + (d->block_base + (uint64_t)m * bpm) * 64;
     const uint32_t ow = (d->width + D - 1) / D, oh = (d->height + D - 1) / D;   // jdiv_round_up(W, d)
-    uint8_t* tcb = (uint8_t*)(s_c + t * S);
-    uint8_t* tcr = tcb + 4 * CW;
-    if (!gray) {
-        int v[N * N];
-        sc_idct<N>(cp + ny * 64, qs->q[1], v);          // q[1]: Cr's table (loadjpg.cpp:984)
+    uint8_t *tcb = nullptr, *tcr = nullptr;
+    if constexpr (!GRAY) {
+        constexpr int CW = (N * N + 3) / 4;             // words of one chroma tile
+        constexpr int S = (2 * CW) | 1;                 // words per thread
+        __shared__ uint32_t s_c[S * HJD_MCU_THREADS];
+        tcb = (uint8_t*)(s_c + threadIdx.x * S);
+        tcr = tcb + 4 * CW;
+        if (!mono) {
+            int v[N * N];
+            sc_idct<N>(cp + ny * 64, qs->q[1], v);      // q[1]: Cr's table (loadjpg.cpp:984)
 #pragma unroll
-        for (int i = 0; i < N * N; i++) tcb[i] = (uint8_t)v[i];
-        sc_idct<N>(cp + (ny + 1) * 64, qs->q[2], v);
+            for (int i = 0; i < N * N; i++) tcb[i] = (uint8_t)v[i];
+            sc_idct<N>(cp + (ny + 1) * 64, qs->q[2], v);
 #pragma unroll
-        for (int i = 0; i < N * N; i++) tcr[i] = (uint8_t)v[i];
-    }
-    uint8_t* img_rgb = rgb + d->rgb_off;
-#pragma unroll 1
-    for (uint32_t bi = 0; bi < ny; bi++) {
-        const uint32_t bx = bi % hf, by = bi / hf;
-        const uint32_t x0 = (mx * hf + bx) * N, y0 = (my * vf + by) * N;
-        if (x0 >= ow || y0 >= oh) continue;             // pixels at or beyond the output size are not written
-        int v[N * N];
-        sc_idct<N>(cp + bi * 64, qs->q[0], v);
-        const uint32_t npix = min((uint32_t)N, ow - x0);
-#pragma unroll
-        for (int y = 0; y < N; y++) {
-            if (y0 + y >= oh) break;
-            int ch[3 * N];
-#pragma unroll
-            for (int x = 0; x < N; x++) {
-                int cb = 128, cr = 128;
-                if (!gray) {
-                    const uint32_t coff = ((bx * N + x) >> hs) + ((by * N + y) >> vs) * N;
-                    cb = tcb[coff];
-                    cr = tcr[coff];
-                }
-                sc_ycc(v[y * N + x], cb, cr, ch + 3 * x);
-            }
-            uint8_t* dst = img_rgb + ((uint64_t)(y0 + y) * ow + x0) * 3;
-            if (N == 4 && npix == 4 && (((uintptr_t)dst) & 3) == 0) {
-                uint32_t* o = (uint32_t*)dst;
-#pragma unroll
-                for (int w = 0; w < 3 * N / 4; w++)
-                    o[w] = (uint32_t)ch[4 * w] | (uint32_t)ch[4 * w + 1] << 8 | (uint32_t)ch[4 * w + 2] << 16 |
-                           (uint32_t)ch[4 * w + 3] << 24;
-            } else {
-#pragma unroll
-                for (int i = 0; i < 3 * N; i++)
-                    if ((uint32_t)i < npix * 3) dst[i] = (uint8_t)ch[i];
-            }
+            for (int i = 0; i < N * N; i++) tcr[i] = (uint8_t)v[i];
         }
     }
-}
-
-// Luma-only sibling of hjd_k_mcu_rgb_scaled (HJD_FLAG_GRAY_OUT with a scale flag): the same threads, grids and luma
-// IDCTs, no chroma IDCT and no colour conversion; the N x N luma samples of each block are stored as they are, one byte
-// per pixel, stride ow.
-template <int N, bool FLAT>
-__global__ void __launch_bounds__(HJD_MCU_THREADS)
-hjd_k_luma_scaled(const int16_t* __restrict__ coef, const HjdImageDesc* __restrict__ imgs,
-                  const HjdQuantSet* __restrict__ qsets, uint8_t* __restrict__ out,
-                  const uint32_t* __restrict__ mcu_prefix, int n_images, int img_base)
-{
-    constexpr uint32_t D = 8 / N;
-    const uint32_t t = threadIdx.x;
-    const HjdImageDesc* d;
-    uint32_t m;
-    if (FLAT) {
-        const uint32_t key = blockIdx.x * HJD_MCU_THREADS + t + mcu_prefix[0];
-        if (key >= mcu_prefix[n_images]) return;
-        int lo = 0, hi = n_images - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (mcu_prefix[mid] <= key) lo = mid; else hi = mid - 1;
-        }
-        d = imgs + lo;
-        m = key - mcu_prefix[lo];
-    } else {
-        d = imgs + (blockIdx.y + img_base);
-        m = blockIdx.x * HJD_MCU_THREADS + t;
-    }
-    if (m >= d->n_mcus || d->blocks_per_mcu == 0) return;
-    const uint32_t hf = d->hf, vf = d->vf, bpm = d->blocks_per_mcu;
-    const uint32_t ny = d->ncomp == 1 ? 1u : hf * vf;
-    const uint32_t my = m / d->mcus_x, mx = m - my * d->mcus_x;
-    const HjdQuantSet* qs = qsets + d->quant_set;
-    const int16_t* cp = coef + (d->block_base + (uint64_t)m * bpm) * 64;
-    const uint32_t ow = (d->width + D - 1) / D, oh = (d->height + D - 1) / D;   // jdiv_round_up(W, d)
     uint8_t* img_out = out + d->rgb_off;
 #pragma unroll 1
     for (uint32_t bi = 0; bi < ny; bi++) {
@@ -259,75 +178,58 @@ hjd_k_luma_scaled(const int16_t* __restrict__ coef, const HjdImageDesc* __restri
 #pragma unroll
         for (int y = 0; y < N; y++) {
             if (y0 + y >= oh) break;
-            uint8_t* dst = img_out + (uint64_t)(y0 + y) * ow + x0;
+            int ch[C * N];                              // the row's output bytes
+#pragma unroll
+            for (int x = 0; x < N; x++) {
+                if constexpr (GRAY) {
+                    ch[x] = v[y * N + x];
+                } else {
+                    int cb = 128, cr = 128;
+                    if (!mono) {
+                        const uint32_t coff = ((bx * N + x) >> hs) + ((by * N + y) >> vs) * N;
+                        cb = tcb[coff];
+                        cr = tcr[coff];
+                    }
+                    sc_ycc(v[y * N + x], cb, cr, ch + 3 * x);
+                }
+            }
+            uint8_t* dst = img_out + ((uint64_t)(y0 + y) * ow + x0) * C;
             if (N == 4 && npix == 4 && (((uintptr_t)dst) & 3) == 0) {
-                *(uint32_t*)dst = (uint32_t)v[y * N] | (uint32_t)v[y * N + 1] << 8 | (uint32_t)v[y * N + 2] << 16 |
-                                  (uint32_t)v[y * N + 3] << 24;
+                uint32_t* o = (uint32_t*)dst;
+#pragma unroll
+                for (int w = 0; w < C * N / 4; w++)
+                    o[w] = (uint32_t)ch[4 * w] | (uint32_t)ch[4 * w + 1] << 8 | (uint32_t)ch[4 * w + 2] << 16 |
+                           (uint32_t)ch[4 * w + 3] << 24;
             } else {
 #pragma unroll
-                for (int x = 0; x < N; x++)
-                    if ((uint32_t)x < npix) dst[x] = (uint8_t)v[y * N + x];
+                for (int i = 0; i < C * N; i++)
+                    if ((uint32_t)i < npix * C) dst[i] = (uint8_t)ch[i];
             }
         }
     }
 }
 
 template <int N>
-static void launch_luma_n(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
-                          const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus, uint32_t max_mcus, cudaStream_t st)
+static void launch_n(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
+                     const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus, uint32_t max_mcus, bool gray, cudaStream_t st)
 {
-    const unsigned gx = (max_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS;
-    if ((uint64_t)gx * HJD_MCU_THREADS * (uint64_t)n_images <= (uint64_t)n_mcus * 4) {   // the grid choice of launch_n
-        for (int base = 0; base < n_images; base += 65535) {
-            const int n = min(65535, n_images - base);
-            hjd_k_luma_scaled<N, false><<<dim3(gx, n), HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, out, nullptr, n_images, base);
-        }
-    } else {
-        const unsigned g = (unsigned)(((uint64_t)n_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS);
-        hjd_k_luma_scaled<N, true><<<g, HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, out, mcu_prefix, n_images, 0);
-    }
+    if (gray)
+        hjd_launch_per_image(hjd_k_mcu_scaled<N, true, false>, hjd_k_mcu_scaled<N, true, true>, HJD_MCU_THREADS, mcu_prefix,
+                             n_images, n_mcus, max_mcus, st, coef, imgs, qsets, out);
+    else
+        hjd_launch_per_image(hjd_k_mcu_scaled<N, false, false>, hjd_k_mcu_scaled<N, false, true>, HJD_MCU_THREADS, mcu_prefix,
+                             n_images, n_mcus, max_mcus, st, coef, imgs, qsets, out);
 }
 
-cudaError_t hjd_launch_luma_scaled(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets,
-                                   uint8_t* out, const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus,
-                                   uint32_t max_mcus, int shift, cudaStream_t st)
+cudaError_t hjd_launch_scaled(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* out,
+                              const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus, uint32_t max_mcus, int shift,
+                              bool gray, cudaStream_t st)
 {
     if (n_images <= 0 || n_mcus == 0 || max_mcus == 0) return cudaSuccess;
     switch (shift) {
-        case 1: launch_luma_n<4>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
-        case 2: launch_luma_n<2>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
-        case 3: launch_luma_n<1>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
-}
-
-template <int N>
-static void launch_n(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets, uint8_t* rgb,
-                     const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus, uint32_t max_mcus, cudaStream_t st)
-{
-    const unsigned gx = (max_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS;
-    // the grid choice of hjd_launch_mcu_rgb: an (image, CTA) grid unless it would be mostly idle thread slots
-    if ((uint64_t)gx * HJD_MCU_THREADS * (uint64_t)n_images <= (uint64_t)n_mcus * 4) {
-        for (int base = 0; base < n_images; base += 65535) {
-            const int n = min(65535, n_images - base);
-            hjd_k_mcu_rgb_scaled<N, false><<<dim3(gx, n), HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, rgb, nullptr, n_images, base);
-        }
-    } else {
-        const unsigned g = (unsigned)(((uint64_t)n_mcus + HJD_MCU_THREADS - 1) / HJD_MCU_THREADS);
-        hjd_k_mcu_rgb_scaled<N, true><<<g, HJD_MCU_THREADS, 0, st>>>(coef, imgs, qsets, rgb, mcu_prefix, n_images, 0);
-    }
-}
-
-cudaError_t hjd_launch_mcu_rgb_scaled(const int16_t* coef, const HjdImageDesc* imgs, const HjdQuantSet* qsets,
-                                      uint8_t* rgb, const uint32_t* mcu_prefix, int n_images, uint32_t n_mcus,
-                                      uint32_t max_mcus, int shift, cudaStream_t st)
-{
-    if (n_images <= 0 || n_mcus == 0 || max_mcus == 0) return cudaSuccess;
-    switch (shift) {
-        case 1: launch_n<4>(coef, imgs, qsets, rgb, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
-        case 2: launch_n<2>(coef, imgs, qsets, rgb, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
-        case 3: launch_n<1>(coef, imgs, qsets, rgb, mcu_prefix, n_images, n_mcus, max_mcus, st); break;
+        case 1: launch_n<4>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, gray, st); break;
+        case 2: launch_n<2>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, gray, st); break;
+        case 3: launch_n<1>(coef, imgs, qsets, out, mcu_prefix, n_images, n_mcus, max_mcus, gray, st); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

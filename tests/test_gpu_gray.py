@@ -1,4 +1,4 @@
-"""Luma-only decode on the GPU (FLAG_GRAY_OUT: hjd_k_luma in csrc/kernels.cu, hjd_k_luma_scaled in csrc/scaled.cu), byte
+"""Luma-only decode on the GPU (FLAG_GRAY_OUT: hjd_k_luma in csrc/kernels.cu, hjd_k_mcu_scaled in csrc/scaled.cu), byte
 for byte against the oracle's Y plane cropped to W x H, a KEEP_PLANES batch's Y plane, the reference's own plane tap where
 it is built, and the luma of the scaled decode; through every sampling, entropy path, grid shape and host path, and with
 FLAG_MULTI_SCAN (scans without luma are not read)."""
