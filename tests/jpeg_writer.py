@@ -98,11 +98,22 @@ def _dqt_payload(tid: int, q) -> bytes:
 
 def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = None, restart_interval: int = 0,
             sof_precision: int | None = None, sos_override: bytes | None = None, trailer: bytes = b"\xff\xd9",
-            quant: dict | None = None, tq: list | None = None) -> bytes:
+            quant: dict | None = None, tq: list | None = None, selectors: list | None = None, fill: int = 0,
+            dc_mod16: bool = False, decoy: dict | None = None, dht_order: list | None = None,
+            sof_marker: int | None = None, dri_segment: bool = False, zrl_tail=()) -> bytes:
     """Re-emit `jpg` (baseline, decoded to `coef` [blocks, 64] zig-zag with absolute DC, scan order) with the
     Huffman tables of `tables` ({(class, id): (bits, vals)} overriding the file's own), a new restart interval,
     and optional header oddities.  `quant` ({table id: 64 values, zig-zag order}) replaces the file's DQT segments;
-    `tq` sets each component's quantisation table selector in the SOF."""
+    `tq` sets each component's quantisation table selector in the SOF.
+    selectors: per component (DC id, AC id), written to the SOS (default: the file's own SOS).
+    fill: that many 0xFF fill bytes (T.81 B.1.1.2) before every RSTn and before the trailer.
+    dc_mod16: DC differences taken modulo 2^16 (in [-32768, 32767]), so that an absolute DC sequence may wrap the
+    int16 range of `coef` as a decoder that keeps its predictor in int16 does.
+    decoy: {(class, id): (bits, vals)} written in a DHT before the real tables, which redefine every such id.
+    dht_order: the (class, id) keys in the order their DHT segments are written (default: sorted).
+    sof_marker: 0xC0 / 0xC1 for the frame header (default: the file's).  dri_segment: write a DRI segment even for
+    restart_interval 0.  zrl_tail: blocks whose trailing zeros are coded as ZRLs before the EOB (as far as the
+    ZRLs stay inside the block; T.81 allows it, libjpeg never writes it)."""
     segs, _ = segments(jpg)
     tabs = dht_tables(segs)
     if tables:
@@ -111,10 +122,14 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
     sos = [p for m, p in segs if m == 0xDA][0]
     ncomp = sof[5]
     comp_ids = [sof[6 + 3 * c] for c in range(ncomp)]
+    if selectors is not None:
+        sos = bytes([ncomp]) + b"".join(bytes([comp_ids[c], (selectors[c][0] << 4) | selectors[c][1]])
+                                         for c in range(ncomp)) + sos[1 + 2 * sos[0]:]
     sel = {}
     for k in range(sos[0]):
         cs, t = sos[1 + 2 * k], sos[2 + 2 * k]
         sel[comp_ids.index(cs)] = (t >> 4, t & 15)
+    zrl_tail = set(int(b) for b in zrl_tail)
     codes = {key: canonical_codes(*tabs[key]) for key in tabs}
 
     hf, vf = geometry["hf"], geometry["vf"]
@@ -130,7 +145,7 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
     for mcu in range(n_mcus):
         if restart_interval and mcu and mcu % restart_interval == 0:
             bw.flush()
-            scan += bw.out + bytes([0xFF, 0xD0 + (rst & 7)])
+            scan += bw.out + b"\xff" * fill + bytes([0xFF, 0xD0 + (rst & 7)])
             bw = BitWriter()
             pred = [0, 0, 0]
             rst += 1
@@ -139,6 +154,8 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
             dc_codes, ac_codes = codes[(0, sel[comp][0])], codes[(1, sel[comp][1])]
             blk = coef[mcu * bpm + bi].astype(np.int64)
             diff = int(blk[0]) - pred[comp]
+            if dc_mod16:
+                diff = ((diff + 0x8000) & 0xFFFF) - 0x8000
             pred[comp] = int(blk[0])
             cat = abs(diff).bit_length()
             if cat not in dc_codes:
@@ -162,11 +179,15 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
                 bw.put(c, length)
                 bw.put(v if v >= 0 else v + (1 << size) - 1, size)
                 run = 0
+            if mcu * bpm + bi in zrl_tail:
+                for _ in range((62 - last) // 16):
+                    c, length = ac_codes[0xF0]
+                    bw.put(c, length)
             if last < 63:
                 c, length = ac_codes[0x00]
                 bw.put(c, length)
     bw.flush()
-    scan += bw.out
+    scan += bw.out + b"\xff" * fill
 
     out = bytearray(b"\xff\xd8")
     dqt_done = False
@@ -186,10 +207,14 @@ def rewrite(jpg: bytes, coef: np.ndarray, geometry: dict, tables: dict | None = 
             for c in range(ncomp):
                 p[6 + 3 * c + 2] = tq[c]
             p = bytes(p)
+        if m in (0xC0, 0xC1) and sof_marker is not None:
+            m = sof_marker
         out += _seg(m, p)
-    for (tc, th), (bits, vals) in sorted(tabs.items()):
-        out += _seg(0xC4, _dht_payload(tc, th, bits, vals))
-    if restart_interval:
+    if decoy:
+        out += _seg(0xC4, b"".join(_dht_payload(tc, th, *decoy[(tc, th)]) for tc, th in sorted(decoy)))
+    for tc, th in (sorted(tabs) if dht_order is None else dht_order):
+        out += _seg(0xC4, _dht_payload(tc, th, *tabs[(tc, th)]))
+    if restart_interval or dri_segment:
         out += _seg(0xDD, struct.pack(">H", restart_interval))
     out += _seg(0xDA, sos_override if sos_override is not None else sos)
     out += scan + trailer
@@ -206,17 +231,17 @@ def block_index(geometry: dict, ncomp: int, mcu: int, comp: int, sub: int = 0) -
 
 
 def blocks_to_jpeg(template: bytes, blocks: np.ndarray, geometry: dict, quant: dict, tq: list | None = None,
-                   tables: dict | None = None, restart_interval: int = 0) -> bytes:
+                   tables: dict | None = None, restart_interval: int = 0, **kw) -> bytes:
     """A baseline file that holds exactly `blocks` ([blocks, 64] int, zig-zag order, absolute DC, MCU / scan order).
     `template` gives size, sampling and Huffman tables: a file written by PIL with its standard tables, which code
     every DC category 0-11 and every AC run/size; `geometry` is its port.decode(..., entropy_only=True)["geometry"].
     `quant` ({id: 64 values, zig-zag}) and `tq` (table id per component, default 0, 1, 1 / 0) are the
-    quantisation tables written."""
+    quantisation tables written.  Further keyword arguments go to rewrite()."""
     ncomp = geometry["ncomp"]
     if tq is None:
         tq = [0, 1, 1][:ncomp]
     return rewrite(template, np.asarray(blocks), geometry, tables=tables, restart_interval=restart_interval,
-                   quant=quant, tq=tq)
+                   quant=quant, tq=tq, **kw)
 
 
 def replace_tables(jpg: bytes, tables: dict, sof_precision: int | None = None, sos_override: bytes | None = None) -> bytes:
