@@ -125,3 +125,49 @@ int hjdo_decode_scaled(const uint8_t* jpg, size_t size, int shift, uint8_t* rgb,
     free(f);
     return err;
 }
+
+/* ------------------------------------------------------------------ loops for tests/colour_cube.py ----------- */
+
+/* The colour step on every (Y, Cb, Cr) byte triple: rgb[((Y << 16) | (Cb << 8) | Cr) * 3 + channel], 48 MB.
+   fma = 0: hjdo_ycc_to_rgb itself.  fma = 1: the same expressions with every product contracted into an FMA (what a
+   compiler allowed to contract would make of them), so that the tests can count where contraction changes a byte. */
+void hjdo_ycc_cube(int fma, uint8_t* rgb)
+{
+    int yc, cb, cr;
+    for (yc = 0; yc < 256; yc++)
+        for (cb = 0; cb < 256; cb++)
+            for (cr = 0; cr < 256; cr++) {
+                uint8_t* o = rgb + (((size_t)yc << 16) | ((size_t)cb << 8) | (size_t)cr) * 3;
+                if (!fma) {
+                    hjdo_ycc_to_rgb(yc, cb, cr, o);
+                } else {
+                    const float fy = (float)yc, fcb = (float)(cb - 128), fcr = (float)(cr - 128);
+                    o[0] = clamp_u8((int)fmaf(1.402f, fcr, fy));
+                    o[1] = clamp_u8((int)fmaf(-0.71414f, fcr, fmaf(-0.34414f, fcb, fy)));
+                    o[2] = clamp_u8((int)fmaf(1.772f, fcb, fy));
+                }
+            }
+}
+
+/* The decoded sample of DC-only blocks (quantised DC c0[i], table entry q0[i] at the DC, every AC zero) through
+   hjdo_decode_single_block (n = 8) or hjdo_scaled_block (n = 4, 2, 1): out[i].  Returns the number of samples that differ
+   from the first sample of their block (a DC-only block decodes flat, so 0). */
+long hjdo_dc_only(const int32_t* c0, const int32_t* q0, long count, int n, uint8_t* out)
+{
+    int16_t coef[64];
+    float q[64];
+    uint8_t blk[64];
+    long i, uneven = 0;
+    int k;
+    memset(coef, 0, sizeof coef);
+    for (k = 0; k < 64; k++) q[k] = 1.0f;
+    for (i = 0; i < count; i++) {
+        coef[0] = (int16_t)c0[i];
+        q[0] = (float)q0[i];
+        if (n == 8) hjdo_decode_single_block(coef, q, blk, 8);
+        else hjdo_scaled_block(coef, q, n, blk, n);
+        for (k = 1; k < n * n; k++) uneven += blk[k] != blk[0];
+        out[i] = blk[0];
+    }
+    return uneven;
+}

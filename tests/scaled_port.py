@@ -45,6 +45,10 @@ def lib() -> ctypes.CDLL:
         L.hjdo_decode_scaled.restype = ctypes.c_int
         L.hjdo_decode_scaled.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_void_p,
                                          ctypes.POINTER(ctypes.c_uint), ctypes.POINTER(ctypes.c_uint)]
+        L.hjdo_ycc_cube.restype = None
+        L.hjdo_ycc_cube.argtypes = [ctypes.c_int, ctypes.c_void_p]
+        L.hjdo_dc_only.restype = ctypes.c_long
+        L.hjdo_dc_only.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_long, ctypes.c_int, ctypes.c_void_p]
         _lib = L
     return _lib
 
@@ -55,6 +59,25 @@ def scaled_block(coef64: np.ndarray, q64: np.ndarray, n: int) -> np.ndarray:
     q64 = np.ascontiguousarray(q64, dtype=np.float32)
     out = np.zeros((n, n), dtype=np.uint8)
     lib().hjdo_scaled_block(coef64.ctypes.data, q64.ctypes.data, n, out.ctypes.data, n)
+    return out
+
+
+def ycc_cube(fma: bool = False) -> np.ndarray:
+    """hjdo_ycc_to_rgb on every byte triple: uint8 [Y, Cb, Cr, channel] (256, 256, 256, 3).  fma: every product
+    contracted into an FMA instead."""
+    out = np.empty((256, 256, 256, 3), dtype=np.uint8)
+    lib().hjdo_ycc_cube(int(fma), out.ctypes.data)
+    return out
+
+
+def dc_only(c0, q0, n: int) -> np.ndarray:
+    """The sample of each DC-only block (quantised DC c0[i], DC table entry q0[i]) through the single-block decode
+    (n = 8) or the reduced IDCT (n = 4, 2, 1): uint8 [len(c0)].  Asserts that every block decodes flat."""
+    c0 = np.ascontiguousarray(c0, dtype=np.int32)
+    q0 = np.ascontiguousarray(np.broadcast_to(q0, c0.shape), dtype=np.int32)
+    out = np.empty(c0.shape, dtype=np.uint8)
+    uneven = lib().hjdo_dc_only(c0.ctypes.data, q0.ctypes.data, c0.size, n, out.ctypes.data)
+    assert uneven == 0, f"{uneven} samples of DC-only blocks differ from their block's first sample"
     return out
 
 

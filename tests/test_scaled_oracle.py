@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 
 from tests import jpeg_writer as jw
+from tests.colour_cube import ycc_to_rgb
 from tests import scaled_port as sp
 from tests.cases import small_cases
 from tools.gen_jpegs import encode_jpeg, synth_rgb
@@ -68,16 +69,6 @@ def model_blocks(coef, q, n, raw=None):
             val = (val.astype(np.int32) + 128).astype(np.int16)
             out[:, y, x] = np.clip(val, 0, 255)
     return out
-
-
-def ycc_to_rgb(yc, cb, cr):
-    """hjdo_ycc_to_rgb in float32, one rounding per operation."""
-    f32 = np.float32
-    yf, cbf, crf = yc.astype(np.float32), (cb.astype(np.int32) - 128).astype(np.float32), (cr.astype(np.int32) - 128).astype(np.float32)
-    r = yf + f32(1.402) * crf
-    g = (yf - f32(0.34414) * cbf) - f32(0.71414) * crf
-    b = yf + f32(1.772) * cbf
-    return np.stack([np.clip(np.trunc(ch).astype(np.int64), 0, 255) for ch in (r, g, b)], axis=-1).astype(np.uint8)
 
 
 def quant_tables(jpg):
