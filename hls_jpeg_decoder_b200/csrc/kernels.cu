@@ -397,8 +397,13 @@ hjd_k_entropy_restart(const uint8_t* __restrict__ arena, const HjdImageDesc* __r
 #pragma unroll
             for (int rep = 0; rep < HJD_ENT_SYMS; rep++) {
                 if (!done_block) {
-                    if (br.nbits < 32) {                 // rare: several very long symbols in a row
-                        br_refill<false>(br); br_refill<false>(br); br_refill<false>(br); br_refill<false>(br);
+                    if (br.nbits < 32) {                 // several long symbols since the round's top-up
+                        // Refill until a refill would change nothing (the window is full, or no padding is due), at
+                        // most four times: four leave at least 32 bits (each adds a byte or more), and stopping at the
+                        // first idle one gives the window all four would; the warp runs as many as its neediest lane.
+#pragma unroll 1
+                        for (int i = 0; i < 4 && (br.pos != br.end ? br.nbits <= 56 : br.nbits <= 32); i++)
+                            br_refill<false>(br);
                     }
                     const bool is_ac = k != 0;
                     const uint32_t t = sh_tab + (is_ac ? (t0 >> 16) : (t0 & 0xFFFFu));
